@@ -2,7 +2,7 @@
 """bench.py -- MH chain-steps/s of the B200 engine (and of the reference on the host cores).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload dgauss|rosen2d|rosen16|gmix64]
-                  [--remote-mode reference|summix] [--pool M] [--lag 0|1]
+                  [--remote-mode reference|summix] [--pool M] [--lag 0|1] [--dump-outputs DIR]
   python bench.py --impl reference ...        # the reference's own CPU loop (oracle/_ref)
 
 A "step" is one exchange window of the hot path: `sync` (=10) Metropolis-Hastings steps of every chain
@@ -39,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # a benchmark run leaves the tree as it found it (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -394,7 +395,30 @@ def timed_windows(ctx, job, K, flush):
     return ms, per_rank, delta
 
 
-def measure(ctx, Cg, rmode, M, K, advance, warmup, flush, lag=None, ranks=None, clocks=None):
+DUMP_BYTES = 60 * 1000 * 1000       # --dump-outputs: array bytes over every rank (under 64 MB with the .npy headers)
+DUMP_SEED = 20260101
+
+
+def dump_outputs(job, path):
+    """Write what the timed path hands its caller after its last window -- the chains' state (p, ly) and running moments
+    (mu, sig, psum2), and the newest kept history row (rows: parameters + logL, the MCout element) -- as float64 .npy files.
+    Over the byte budget, a fixed seeded sample of chains (the same chains in every run of the same arguments) is kept."""
+    import numpy as np
+    st = job.e.state()
+    kept = job.e.stats()["history_rows"] // job.Cg
+    if kept > 0:
+        st["rows"] = job.e.history(first=kept - 1, count=1)[0]
+    per_chain = sum(a[0].nbytes for a in st.values())
+    n = min(job.Cg, DUMP_BYTES // job.world // per_chain)
+    idx = slice(None) if n == job.Cg else np.sort(np.random.default_rng(DUMP_SEED).choice(job.Cg, n, replace=False))
+    os.makedirs(path, exist_ok=True)
+    tag = "" if job.world == 1 else "rank%d_" % job.rank
+    for name, a in st.items():
+        np.save(os.path.join(path, tag + name + ".npy"), np.ascontiguousarray(a[idx], dtype=np.float64))
+    return n
+
+
+def measure(ctx, Cg, rmode, M, K, advance, warmup, flush, lag=None, ranks=None, clocks=None, dump=None):
     """Resident throughput of one configuration: burn-in 500, `advance` untimed windows, `warmup` untimed
     windows, K timed windows.  Returns a dict (on every active rank)."""
     a = ctx["args"]
@@ -410,6 +434,7 @@ def measure(ctx, Cg, rmode, M, K, advance, warmup, flush, lag=None, ranks=None, 
         job.window()
     ms, per_rank, d = timed_windows(ctx, job, K, flush)
     ck = clocks.stop() if clocks is not None else None
+    dumped = dump_outputs(job, dump) if dump else None
     mean, cov = job.e.moments()
     st = job.e.stats()
     out = {"value": job.N * a.sync * K / (ms * 1e-3), "ms_per_step": ms / K, "per_rank_ms_per_step": per_rank,
@@ -422,7 +447,7 @@ def measure(ctx, Cg, rmode, M, K, advance, warmup, flush, lag=None, ranks=None, 
            "accept_rate": d["accepted"] / max(1, d["tried"]),
            "exchange_wait_ms_per_step": d["exchange_wait_ns"] * 1e-6 / K, "exchange_waits": d["exchange_waits"],
            "posterior_mean": [float(x) for x in mean[:4]], "posterior_var": [float(cov[i, i]) for i in range(min(4, len(mean)))],
-           "clocks": ck}
+           "clocks": ck, "dumped_chains": dumped}
     job.close()
     return out
 
@@ -535,6 +560,9 @@ def main():
     ap.add_argument("--no-modes", action="store_true", help="skip the secondary measurements of the other remote modes")
     ap.add_argument("--no-check", action="store_true", help="N>1: skip the sharded == single-engine check")
     ap.add_argument("--no-place", action="store_true", help="do not move the timed region to a representative share of remote steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed windows, write the headline run's state, running moments and newest history row as "
+                         "DIR/<name>.npy (float64; a fixed seeded sample of chains when all of them would exceed 64 MB)")
     args = ap.parse_args()
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3                         # timing rule: W >= 3
@@ -610,7 +638,7 @@ def main():
                 sys.stderr.write("peer-to-peer exchange unavailable on this box: using the NCCL all-gather exchange\n")
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)       # > 126 MB L2
-    head = measure(ctx, Cg, rmode, args.pool, K, args.advance, Wu, flush, clocks=clocks)
+    head = measure(ctx, Cg, rmode, args.pool, K, args.advance, Wu, flush, clocks=clocks, dump=args.dump_outputs)
     ck = head["clocks"]
 
     # ---- the other remote-proposal configurations, measured the same way (shorter)
@@ -705,6 +733,8 @@ def main():
                 "exchange_wait_ms_per_step": head["exchange_wait_ms_per_step"],
                 "posterior_mean": head["posterior_mean"], "posterior_var": head["posterior_var"],
                 "modes": modes, "sharded_equals_single": check}
+        if args.dump_outputs:
+            line["dump_outputs"] = {"dir": args.dump_outputs, "chains_per_gpu": head["dumped_chains"], "of": Cg}
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

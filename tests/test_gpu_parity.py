@@ -461,23 +461,22 @@ def test_full_size_stationarity(pl, rmode, M):
 
 
 def test_remote_proposals_match_reference_distribution():
-    """PLOCAL = 0.9 (remote proposals on): the engine's normal mode against the REFERENCE
-    ITSELF (oracle/_ref, shim Philox RNG) on the reference's own launch shape (4 ranks x 4
-    chains, all 16 chains in the mixture).  Chains of one run are coupled through the
-    exchange, so the unit of comparison is the RUN: per-run posterior summaries over 48
-    independent seeds each, two-sample KS at p > 0.01."""
+    """PLOCAL = 0.9 (remote proposals on): the engine's normal mode against the reference's
+    algorithm (oracle/mh_oracle.c, which test_oracle.py pins bit for bit to the reference's own
+    outputs stored in tests/golden/) on the reference's own launch shape (4 ranks x 4 chains,
+    all 16 chains in the mixture), the reference side on seeded replay streams.  Chains of one
+    run are coupled through the exchange, so the unit of comparison is the RUN: per-run
+    posterior summaries over 48 independent seeds each, two-sample KS at p > 0.01."""
     from scipy import stats
-    from oracle import ref as refmod
-    if not refmod.available(64):
-        pytest.skip("oracle/_ref not built")
     eng = _engine()
-    ref = refmod.Ref(64)
     R, C, d, nburn, nsamp, nrep = 4, 4, 2, 300, 1500, 48
     pin = tiled_pinit(C, d)
     ref_stat, gpu_stat = [], []
     for k in range(nrep):
-        o = ref.run("dualgaussian", d, C, R, nsamp, nburn, pin, par=[5.0], seed=1000 + k, want_maxl=False)
-        rows = o["rows"].reshape(-1, 3)[:, :]
+        Z, U, I = make_streams(R, C, d, nburn + nsamp, 1000 + k)
+        o = mh.run_replay("dualgaussian", d, C, R, nsamp, nburn, pin, Z, U, I, par=[5.0])
+        assert o["used"][:, 3].sum() == 0                                # no stream overrun
+        rows = o["rows"].reshape(-1, 3)
         ref_stat.append((rows[:, 0].mean(), (rows[:, 0] > 2.5).mean(), rows[:, 0].var()))
         e = eng.Engine(d, R * C, mode="normal", coin_group=4, pool_m=0, seed=5000 + k, history_steps=nsamp)
         e.run(nsamp, nburn, np.tile(pin, (R, 1)), "dualgaussian", [5.0])
