@@ -50,8 +50,10 @@ enum {
   MCGPU_GAUSSIAN = 2,       /* rosenbrock.cc:44-61,  par: mu[2], sig2[2] (optional) */
   MCGPU_DUALGAUSSIAN = 3,   /* rosenbrock.cc:63-78,  par: w (optional, default 5)   */
   MCGPU_GAUSSMIX = 4,       /* new: par = K, mu[K][d], sig2[K][d], w[K]             */
-  MCGPU_HOST_LIKELIHOOD = 100 /* the likelihood is a host callback (a user-written VLFunc, src/vlfunc.hh:9-12):
+  MCGPU_HOST_LIKELIHOOD = 100, /* the likelihood is a host callback (a user-written VLFunc, src/vlfunc.hh:9-12):
                                the engine steps with mcgpu_step_propose / mcgpu_step_accept      */
+  MCGPU_DEVICE_PLUGIN = 101 /* a user functor compiled into a plugin cubin (include/mcgpu_plugin.cuh):
+                               set with mcgpu_set_likelihood_plugin                               */
 };
 
 enum {
@@ -135,6 +137,14 @@ int  mcgpu_set_stream(mcgpu_engine *e, void *cuda_stream);
 
 /* VLFunc &L argument of MCPar::run. */
 int  mcgpu_set_likelihood(mcgpu_engine *e, int lik, const double *par, int npar);
+
+/* A user-written likelihood inside the fused step kernels: cubin_path is a plugin built from one user header
+ * (include/mcgpu_plugin.cuh, `python -m mcpar_b200.plugin`); par[npar] is copied to the device and handed to
+ * the functor unchanged.  The engine then runs as with a built-in likelihood (lik = MCGPU_DEVICE_PLUGIN).
+ * NORMAL mode, thread-per-chain kernels (even nparam <= 16).  MCGPU_EINVAL, before any launch, when the file
+ * cannot be loaded, the plugin was built for another nparam or from other kernel sources (its stamp), or the
+ * mode is VERIFY / REPLAY_LOCAL. */
+int  mcgpu_set_likelihood_plugin(mcgpu_engine *e, const char *cubin_path, const double *par, int npar);
 
 /* MCPar::covar_setup (mcpar.cc:454-484): incov is d x d row-major symmetric PD, or
  * NULL for the identity; the lower Cholesky factor is taken on the host (one-off,
@@ -276,6 +286,9 @@ int  mcgpu_device_ptr(mcgpu_engine *e, int which, void **ptr, size_t *bytes);
  * (src/vlfunc.hh:11): x is npset*nparam chain-major, y is npset. */
 int  mcgpu_loglik(int device, int lik, int nparam, const double *par, int npar, int npset,
                   const double *x, double *y);
+/* The same for a plugin cubin (mcgpu_set_likelihood_plugin); nparam must be the plugin's. */
+int  mcgpu_loglik_plugin(int device, const char *cubin_path, int nparam, const double *par, int npar, int npset,
+                         const double *x, double *y);
 
 /* mcutil::qriguess (src/mcutil.cc:3-34): Sobol points in the box [plo,phi],
  * rank skip-ahead; pout is npset*nparam chain-major on the host. */

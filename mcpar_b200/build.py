@@ -1,8 +1,10 @@
-"""Build libmcgpu.so in-tree with nvcc for sm_100a (no JIT cache, no torch extension).
+"""Build libmcgpu.so in-tree with nvcc for sm_100a (no JIT cache, no torch extension), and the shipped
+likelihood plugins into mcpar_b200/plugins/ (mcpar_b200/plugin.py).
 
   python -m mcpar_b200.build            # build if stale
   python -m mcpar_b200.build --force
 """
+import hashlib
 import os
 import subprocess
 import sys
@@ -18,10 +20,31 @@ NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-ccbin", "/usr/bin/g++",
           "-I", os.path.join(ROOT, "include")]
+# Sources that fix the layout and meaning of what the engine hands a plugin's kernels (StepParams by value,
+# the kernel templates they instantiate).  Their hash is compiled into libmcgpu.so and into every plugin; the
+# engine loads only plugins whose stamp equals its own.
+STAMPED = ["include/mcgpu.h", "mcpar_b200/csrc/mcgpu_device.cuh", "mcpar_b200/csrc/mh_kernels.cuh",
+           "mcpar_b200/csrc/mcgpu_math.cuh", "mcpar_b200/csrc/mcgpu_tables.h", "mcpar_b200/csrc/mh_plugin.cu"]
+
+
+def kernel_stamp(root=ROOT):
+    """64-bit stamp of the STAMPED sources under `root` (contents and relative names only)."""
+    h = hashlib.sha256()
+    for rel in STAMPED:
+        with open(os.path.join(root, rel), "rb") as f:
+            data = f.read()
+        h.update(rel.encode() + b"\0" + str(len(data)).encode() + b"\0" + data)
+    return int.from_bytes(h.digest()[:8], "little")
+
+
+def stamp_define(stamp):
+    return "-DMCGPU_KERNEL_STAMP=0x%016xULL" % stamp
+
+
 UNITS = {                       # translation unit -> extra flags
     "mh_fast.cu": [],
     "mh_exact.cu": ["-fmad=false"],        # operation-by-operation IEEE arithmetic (verification)
-    "mcgpu_api.cu": [],
+    "mcgpu_api.cu": [stamp_define(kernel_stamp())],
 }
 
 
@@ -42,8 +65,14 @@ def stale():
 
 
 def build(force=False, verbose=False):
-    if not force and not stale():
-        return LIB
+    if force or stale():
+        build_lib(verbose)
+    from mcpar_b200 import plugin
+    plugin.build_shipped(force=force)
+    return LIB
+
+
+def build_lib(verbose=False):
     os.makedirs(OBJ, exist_ok=True)
 
     def cc(item):
@@ -67,7 +96,6 @@ def build(force=False, verbose=False):
     if r.returncode != 0:
         raise RuntimeError("link failed:\n%s\n%s" % (r.stdout, r.stderr))
     build_host()
-    return LIB
 
 
 HOST = os.path.join(HERE, "host")

@@ -19,6 +19,10 @@
 #include <deque>
 #include <algorithm>
 
+#ifndef MCGPU_KERNEL_STAMP
+#error "build with mcpar_b200/build.py: it passes -DMCGPU_KERNEL_STAMP (the stamp plugins must carry)"
+#endif
+
 using namespace mcgpu;
 
 namespace {
@@ -40,6 +44,7 @@ struct mcgpu_engine {
 
   // likelihood
   int lik = -1; int lik_k = 0; double lp[8] = {0}; double *lik_dev = nullptr;
+  cudaLibrary_t plugin = nullptr; cudaKernel_t pk[8] = {};   // MCGPU_DEVICE_PLUGIN: the loaded cubin, kernels by PH_* / PK_*
 
   // NORMAL / REPLAY_LOCAL state (SoA) or VERIFY state (AoS per rank)
   double *x = nullptr, *ly = nullptr, *mu = nullptr, *ps = nullptr;
@@ -209,6 +214,93 @@ void fill_step_params(mcgpu_engine *e, StepParams &p)
   p.nburn_total = e->nburn_total;
 }
 
+// ---- device likelihood plugins (mh_plugin.cu compiled per user header into a cubin) --------------------------
+enum { PK_INIT = 6, PK_EVAL = 7 };           // plugin kernels beyond the six step phases PH_*
+
+// The one place that knows the plugin's symbol names: mh_plugin.cu instantiates mcgpu::fast::mh_steps_kernel
+// <MCGPU_DEVICE_PLUGIN, d, RNG_PHILOX = 0, phase> and init_loglik_kernel<MCGPU_DEVICE_PLUGIN, d>.
+std::string plugin_kernel_name(int d, int which)
+{
+  char b[128];
+  if (which == PK_EVAL) return "mcgpu_plugin_loglik";
+  if (which == PK_INIT) snprintf(b, sizeof b, "_ZN5mcgpu4fast18init_loglik_kernelILi%dELi%dEEEvNS_10StepParamsE", MCGPU_DEVICE_PLUGIN, d);
+  else snprintf(b, sizeof b, "_ZN5mcgpu4fast15mh_steps_kernelILi%dELi%dELi0ELi%dEEEvNS_10StepParamsE", MCGPU_DEVICE_PLUGIN, d, which);
+  return b;
+}
+
+// Load a plugin cubin into the current device's context and check it before anything launches from it: it must
+// have been compiled from the kernel sources this library was (StepParams crosses by value) and for d parameters.
+int plugin_open(const char *path, int d, cudaLibrary_t *lib, cudaKernel_t k[8], std::string &err)
+{
+  *lib = nullptr;
+  FILE *f = path ? fopen(path, "rb") : nullptr;
+  if (!f) { err = std::string("plugin: cannot open '") + (path ? path : "(null)") + "'"; return MCGPU_EINVAL; }
+  fclose(f);
+  cudaLibrary_t L = nullptr;
+  cudaError_t s = cudaLibraryLoadFromFile(&L, path, nullptr, nullptr, 0, nullptr, nullptr, 0);
+  if (s != cudaSuccess) { cudaGetLastError(); err = std::string("plugin: cannot load '") + path + "': " + cudaGetErrorString(s); return MCGPU_EINVAL; }
+  void *ps = nullptr, *pn = nullptr; size_t bs = 0, bn = 0;
+  unsigned long long stamp = 0; int np = 0;
+  if (cudaLibraryGetGlobal(&ps, &bs, L, "mcgpu_plugin_stamp") != cudaSuccess || bs != sizeof stamp ||
+      cudaLibraryGetGlobal(&pn, &bn, L, "mcgpu_plugin_nparam") != cudaSuccess || bn != sizeof np ||
+      cudaMemcpy(&stamp, ps, sizeof stamp, cudaMemcpyDeviceToHost) != cudaSuccess ||
+      cudaMemcpy(&np, pn, sizeof np, cudaMemcpyDeviceToHost) != cudaSuccess) {
+    cudaGetLastError(); cudaLibraryUnload(L);
+    err = std::string("plugin: '") + path + "' is not a likelihood plugin (no mcgpu_plugin_stamp / mcgpu_plugin_nparam)";
+    return MCGPU_EINVAL;
+  }
+  char b[256];
+  if (stamp != (unsigned long long)MCGPU_KERNEL_STAMP) {
+    snprintf(b, sizeof b, "plugin: kernel-source stamp %016llx differs from this library's %016llx: rebuild the plugin",
+             stamp, (unsigned long long)MCGPU_KERNEL_STAMP);
+    cudaLibraryUnload(L); err = b; return MCGPU_EINVAL;
+  }
+  if (np != d) {
+    snprintf(b, sizeof b, "plugin: built for nparam = %d, the engine has nparam = %d", np, d);
+    cudaLibraryUnload(L); err = b; return MCGPU_EINVAL;
+  }
+  for (int w = 0; w < 8; ++w)
+    if (cudaLibraryGetKernel(&k[w], L, plugin_kernel_name(d, w).c_str()) != cudaSuccess) {
+      cudaGetLastError(); cudaLibraryUnload(L);
+      err = "plugin: kernel " + plugin_kernel_name(d, w) + " missing from the cubin";
+      return MCGPU_EINVAL;
+    }
+  *lib = L;
+  return MCGPU_OK;
+}
+
+void plugin_release(mcgpu_engine *e)
+{
+  if (e->plugin) cudaLibraryUnload(e->plugin);
+  e->plugin = nullptr;
+}
+
+cudaError_t launch_plugin(mcgpu_engine *e, int which, const StepParams &p, unsigned grid, unsigned block, size_t smem)
+{
+  const void *f = reinterpret_cast<const void *>(e->pk[which]);
+  if (smem > 48 * 1024) {                            // per launch: the attribute is per device
+    cudaError_t s = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (s != cudaSuccess) return s;
+  }
+  void *args[] = {const_cast<StepParams *>(&p)};
+  return cudaLaunchKernel(f, dim3(grid), dim3(block), args, smem, e->stream);
+}
+
+// the grid, block and shared-memory rules of launch_lik_d (mh_dispatch.inl)
+cudaError_t launch_plugin_steps(mcgpu_engine *e, int phase, const StepParams &p)
+{
+  const int block = fast::step_block();
+  const size_t smem = fast::steps_smem_bytes(e->d, p.nsteps, p.pool_m, phase != PH_BURN && phase != PH_LOCAL);
+  return launch_plugin(e, phase, p, (unsigned)((p.C + block - 1) / block), block, smem);
+}
+
+// initial log-likelihoods L(nchain, pvals, lylast), mcpar.cc:53, on the SoA state
+cudaError_t launch_init_any(mcgpu_engine *e, const StepParams &p)
+{
+  if (e->lik == MCGPU_DEVICE_PLUGIN) return launch_plugin(e, PK_INIT, p, (unsigned)((p.C + 255) / 256), 256, 0);
+  return (e->replay_local ? exact::launch_init_loglik : fast::launch_init_loglik)(e->lik, e->d, p, e->stream);
+}
+
 cudaError_t launch_steps_any(mcgpu_engine *e, int phase, const StepParams &p)
 {
   ++e->launches;
@@ -232,6 +324,7 @@ cudaError_t launch_steps_any(mcgpu_engine *e, int phase, const StepParams &p)
   }
   if (e->replay_local) return exact::launch_steps(e->lik, e->d, 1, phase == PH_BURN ? PH_BURN : PH_LOCAL, p, e->stream);
   if (e->remote_mode == 1) phase = phase == PH_MIXED ? PH_MIXED_SUM : (phase == PH_REMOTE ? PH_REMOTE_SUM : phase);
+  if (e->lik == MCGPU_DEVICE_PLUGIN) return launch_plugin_steps(e, phase, p);
   return fast::launch_steps(e->lik, e->d, 0, phase, p, e->stream);
 }
 
@@ -585,6 +678,7 @@ int mcgpu_destroy(mcgpu_engine *e)
   for (void *q : e->peer_opened) cudaIpcCloseMemHandle(q);
   for (int i = 0; i < 2; ++i) { if (e->pin[i]) cudaFreeHost(e->pin[i]); if (e->pin_ev[i]) cudaEventDestroy(e->pin_ev[i]); }
   if (e->side) cudaStreamSynchronize(e->side);
+  plugin_release(e);
   if (e->sink && e->sink_registered) cudaHostUnregister(e->sink);
   if (e->sink_ev) cudaEventDestroy(e->sink_ev);
   for (auto &dr : e->drains) cudaEventDestroy(dr.second);
@@ -631,6 +725,7 @@ int mcgpu_set_likelihood(mcgpu_engine *e, int lik, const double *par, int npar)
     if (!e->wide && e->cfg.pl < 1.0 && fast::steps_smem_bytes(e->d, e->cfg.sync, e->M, true) > 200 * 1024)
       return fail(e, MCGPU_EINVAL, "remote-mixture pool does not fit in shared memory (40 bytes per slot and parameter + 16 per slot): choose pool_m with pool_m*nparam <= 4800");
   }
+  if (e->plugin) { CK(cudaStreamSynchronize(e->stream)); plugin_release(e); }
   if (e->lik_dev) { cudaFree(e->lik_dev); e->lik_dev = nullptr; }
   if (!dev.empty()) {
     CK(cudaMalloc((void**)&e->lik_dev, dev.size() * 8));
@@ -665,6 +760,34 @@ int mcgpu_set_likelihood(mcgpu_engine *e, int lik, const double *par, int npar)
       CK(cudaStreamSynchronize(e->stream));
     }
   }
+  return MCGPU_OK;
+}
+
+int mcgpu_set_likelihood_plugin(mcgpu_engine *e, const char *cubin_path, const double *par, int npar)
+{
+  if (!e) return MCGPU_EINVAL;
+  if (npar < 0 || (npar > 0 && !par)) return fail(e, MCGPU_EINVAL, "par must hold npar reals");
+  if (e->cfg.mode != MCGPU_MODE_NORMAL) return fail(e, MCGPU_EINVAL, "plugin likelihoods run in NORMAL mode only (not VERIFY or REPLAY_LOCAL)");
+  if (e->hostlik) return fail(e, MCGPU_ESTATE, "this engine was set up for a host likelihood: create a new engine");
+  if (e->have_state && e->wide) return fail(e, MCGPU_ESTATE, "likelihood change would change the state layout: create a new engine");
+  if (e->cfg.pl < 1.0 && fast::steps_smem_bytes(e->d, e->cfg.sync, e->M, true) > 200 * 1024)
+    return fail(e, MCGPU_EINVAL, "remote-mixture pool does not fit in shared memory (40 bytes per slot and parameter + 16 per slot): choose pool_m with pool_m*nparam <= 4800");
+  DeviceGuard g(e->dev);
+  cudaLibrary_t lib = nullptr; cudaKernel_t k[8]; std::string err;
+  const int rc = plugin_open(cubin_path, e->d, &lib, k, err);
+  if (rc) { e->err = err; return rc; }
+  CK(cudaStreamSynchronize(e->stream));                   // nothing of the previous likelihood is in flight
+  plugin_release(e);
+  e->plugin = lib; memcpy(e->pk, k, sizeof e->pk);
+  if (e->lik_dev) { cudaFree(e->lik_dev); e->lik_dev = nullptr; }
+  if (npar > 0) {
+    CK(cudaMalloc((void**)&e->lik_dev, (size_t)npar * 8));
+    CK(cudaMemcpyAsync(e->lik_dev, par, (size_t)npar * 8, cudaMemcpyHostToDevice, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+  }
+  memset(e->lp, 0, sizeof e->lp);
+  for (int i = 0; i < npar && i < 8; ++i) e->lp[i] = par[i];
+  e->lik = MCGPU_DEVICE_PLUGIN; e->lik_k = npar; e->wide = false;   // thread-per-chain kernels only
   return MCGPU_OK;
 }
 
@@ -723,7 +846,7 @@ int mcgpu_set_state(mcgpu_engine *e, const double *pinit)
     CK(cudaFreeAsync(tmp, e->stream));
     StepParams p; fill_step_params(e, p);
     e->launches += 2;
-    CK((e->replay_local ? exact::launch_init_loglik : fast::launch_init_loglik)(e->lik, d, p, e->stream));
+    CK(launch_init_any(e, p));
   }
   return state_installed(e);
 }
@@ -1655,6 +1778,31 @@ int mcgpu_loglik(int device, int lik, int nparam, const double *par, int npar, i
   return MCGPU_OK;
 }
 
+int mcgpu_loglik_plugin(int device, const char *cubin_path, int nparam, const double *par, int npar, int npset,
+                        const double *x, double *y)
+{
+  if (!x || !y || npset < 0 || npar < 0 || (npar > 0 && !par)) return fail(nullptr, MCGPU_EINVAL, "null argument");
+  if (mcgpu_device_count() <= device || device < 0) return fail(nullptr, MCGPU_ENODEVICE, "no usable CUDA device (this engine has no CPU path)");
+  DeviceGuard g(device);
+  cudaLibrary_t lib = nullptr; cudaKernel_t k[8]; std::string err;
+  const int rc = plugin_open(cubin_path, nparam, &lib, k, err);
+  if (rc) return fail(nullptr, rc, err.c_str());
+  struct Unload { cudaLibrary_t l; ~Unload() { cudaLibraryUnload(l); } } unload = {lib};
+  if (npset == 0) return MCGPU_OK;
+  double *dx = nullptr, *dy = nullptr, *dp = nullptr;
+  CK0(cudaMalloc((void**)&dx, (size_t)npset * nparam * 8)); CK0(cudaMalloc((void**)&dy, (size_t)npset * 8));
+  if (npar > 0) CK0(cudaMalloc((void**)&dp, (size_t)npar * 8));
+  if (npar > 0) CK0(cudaMemcpyAsync(dp, par, (size_t)npar * 8, cudaMemcpyHostToDevice, 0));
+  CK0(cudaMemcpyAsync(dx, x, (size_t)npset * nparam * 8, cudaMemcpyHostToDevice, 0));
+  const double *cdp = dp, *cdx = dx;
+  void *args[] = {(void *)&cdp, (void *)&npar, (void *)&cdx, (void *)&dy, (void *)&npset};
+  CK0(cudaLaunchKernel(reinterpret_cast<const void *>(k[PK_EVAL]), dim3((unsigned)((npset + 255) / 256)), dim3(256), args, 0, 0));
+  CK0(cudaMemcpyAsync(y, dy, (size_t)npset * 8, cudaMemcpyDeviceToHost, 0));
+  CK0(cudaStreamSynchronize(0));
+  cudaFree(dx); cudaFree(dy); if (dp) cudaFree(dp);
+  return MCGPU_OK;
+}
+
 int mcgpu_qriguess(int device, int rank, int npset, int nparam, const double *plo, const double *phi, double *pout)
 {
   if (!plo || !phi || !pout || npset < 0 || rank < 0) return fail(nullptr, MCGPU_EINVAL, "bad argument");
@@ -1706,7 +1854,7 @@ int mcgpu_set_state_sobol(mcgpu_engine *e, const double *plo, const double *phi,
     CK(exact::launch_loglik_aos(L, e->x, e->ly, (int)e->C, e->stream));   // L(nchain, pvals, lylast), mcpar.cc:53
   } else {
     StepParams p; fill_step_params(e, p);
-    CK((e->replay_local ? exact::launch_init_loglik : fast::launch_init_loglik)(e->lik, d, p, e->stream));
+    CK(launch_init_any(e, p));
   }
   return state_installed(e);
 }

@@ -11,6 +11,7 @@ cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, double2
                              const unsigned long long *arrivals, unsigned long long wait_target, int *xflag,
                              unsigned long long *xstat, cudaStream_t st);
 cudaError_t launch_factor_prep(const double *rm, double *cm, int D, int *diag, cudaStream_t st);
+int step_block();                  // CTA size of the step kernels (also used for plugin launches)
 bool steps_supported(int lik, int d);
 size_t steps_smem_bytes(int d, int nsteps, int pool_m, bool with_pool);
 cudaError_t launch_steps(int lik, int d, int rngk, int phase, const StepParams &p, cudaStream_t st);

@@ -12,7 +12,7 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MCGPU_LIB") or os.path.join(HERE, "libmcgpu.so")   # MCGPU_LIB: A/B experiments with alternative builds
 
-LIK = {"rosenbrock1": 0, "rosenbrock2": 1, "gaussian": 2, "dualgaussian": 3, "gaussmix": 4, "host": 100}
+LIK = {"rosenbrock1": 0, "rosenbrock2": 1, "gaussian": 2, "dualgaussian": 3, "gaussmix": 4, "host": 100, "plugin": 101}
 MODE = {"normal": 0, "verify": 1, "replay_local": 2}
 ERRORS = {-1: "EINVAL", -2: "ENODEVICE", -3: "ECUDA", -4: "ESTATE", -5: "ENOMEM", -6: "ESTREAM",
           -7: "EPEER"}
@@ -30,6 +30,7 @@ EXPORTS = [
     "mcgpu_history_maxlike", "mcgpu_history_moments",
     "mcgpu_checkpoint_size", "mcgpu_checkpoint_save", "mcgpu_checkpoint_load",
     "mcgpu_get_stats", "mcgpu_device_ptr", "mcgpu_loglik", "mcgpu_qriguess",
+    "mcgpu_set_likelihood_plugin", "mcgpu_loglik_plugin",
     "mcgpu_measure_fp64_peak",
 ]
 
@@ -91,13 +92,26 @@ def device_count():
     return load().mcgpu_device_count()
 
 
-def loglik(lik, nparam, x, par=None, device=0):
-    """VLFunc::operator()(npset, x, y) on the GPU (src/vlfunc.hh:11)."""
+def _plugin_path(lik, plugin):
+    if lik == "plugin" and not plugin:
+        raise ValueError('likelihood "plugin" needs plugin=<path of the plugin cubin> (mcpar_b200/plugin.py builds one)')
+    if lik != "plugin" and plugin:
+        raise ValueError('plugin= is given but the likelihood is %r, not "plugin"' % (lik,))
+    return os.fsencode(os.path.abspath(plugin)) if plugin else None
+
+
+def loglik(lik, nparam, x, par=None, device=0, plugin=None):
+    """VLFunc::operator()(npset, x, y) on the GPU (src/vlfunc.hh:11); lik="plugin" evaluates the plugin cubin
+    `plugin` (built for nparam)."""
+    path = _plugin_path(lik, plugin)
     x = np.ascontiguousarray(x, dtype=np.float64).reshape(-1, nparam)
     y = np.empty(x.shape[0], dtype=np.float64)
-    par_a = None if par is None else np.ascontiguousarray(par, dtype=np.float64)
-    _check(load().mcgpu_loglik(device, LIK[lik], nparam, _p(par_a), 0 if par is None else par_a.size,
-                               x.shape[0], _p(x), _p(y)))
+    par_a = None if par is None else np.ascontiguousarray(par, dtype=np.float64).ravel()
+    npar = 0 if par is None else par_a.size
+    if path:
+        _check(load().mcgpu_loglik_plugin(device, path, nparam, _p(par_a), npar, x.shape[0], _p(x), _p(y)))
+    else:
+        _check(load().mcgpu_loglik(device, LIK[lik], nparam, _p(par_a), npar, x.shape[0], _p(x), _p(y)))
     return y
 
 
@@ -199,9 +213,16 @@ class Engine:
     def set_stream(self, cuda_stream):
         self._ck(self.lib.mcgpu_set_stream(self.h, C.c_void_p(cuda_stream)))
 
-    def set_likelihood(self, lik, par=None):
-        par_a = None if par is None else np.ascontiguousarray(par, dtype=np.float64)
-        self._ck(self.lib.mcgpu_set_likelihood(self.h, LIK[lik], _p(par_a), 0 if par is None else par_a.size))
+    def set_likelihood(self, lik, par=None, plugin=None):
+        """lik names a built-in likelihood, or "plugin" with plugin=<cubin path> (a user functor compiled by
+        mcpar_b200/plugin.py; par is handed to it unchanged)."""
+        path = _plugin_path(lik, plugin)
+        par_a = None if par is None else np.ascontiguousarray(par, dtype=np.float64).ravel()
+        npar = 0 if par is None else par_a.size
+        if path:
+            self._ck(self.lib.mcgpu_set_likelihood_plugin(self.h, path, _p(par_a), npar))
+        else:
+            self._ck(self.lib.mcgpu_set_likelihood(self.h, LIK[lik], _p(par_a), npar))
 
     def set_covariance(self, incov=None):
         inc = None if incov is None else np.ascontiguousarray(incov, dtype=np.float64).ravel()
@@ -305,9 +326,9 @@ class Engine:
     def synchronize(self):
         self._ck(self.lib.mcgpu_synchronize(self.h))
 
-    def run(self, nsamp, nburn, pinit, lik, par=None, incov=None):
+    def run(self, nsamp, nburn, pinit, lik, par=None, incov=None, plugin=None):
         """MCPar::run on this engine's chains (single engine: exchange is internal)."""
-        self.set_likelihood(lik, par)
+        self.set_likelihood(lik, par, plugin=plugin)
         self.set_covariance(incov)
         self.set_state(pinit)
         self.burnin(nburn)

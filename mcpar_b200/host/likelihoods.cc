@@ -10,7 +10,9 @@
 int DeviceVLFunc::operator()(int npset, const Real *x, Real *restrict y)
 {
   const std::vector<double> &p = params();
-  const int rc = mcgpu_loglik(device, lik_id(), nparam(), p.empty() ? 0 : &p[0], (int)p.size(), npset, x, y);
+  const int rc = plugin_path()
+      ? mcgpu_loglik_plugin(device, plugin_path(), nparam(), p.empty() ? 0 : &p[0], (int)p.size(), npset, x, y)
+      : mcgpu_loglik(device, lik_id(), nparam(), p.empty() ? 0 : &p[0], (int)p.size(), npset, x, y);
   if (rc != MCGPU_OK) {                      // no CPU fallback: fail loudly
     fprintf(stderr, "VLFunc: GPU likelihood evaluation failed (%d): %s\n", rc, mcgpu_last_error(0));
     abort();
@@ -51,3 +53,10 @@ GaussMix::GaussMix(int nparam, int ncomp, const Real *mu, const Real *sig2, cons
   mpar.insert(mpar.end(), w, w + K);
 }
 int GaussMix::lik_id() const { return MCGPU_GAUSSMIX; }
+
+DevicePlugin::DevicePlugin(const std::string &cubin_path, int nparam, const std::vector<double> &par) : path(cubin_path), n(nparam)
+{
+  if (n < 2 || n > 16 || n % 2 != 0) throw("a device plugin has an even nparam in 2..16");
+  mpar = par;
+}
+int DevicePlugin::lik_id() const { return MCGPU_DEVICE_PLUGIN; }

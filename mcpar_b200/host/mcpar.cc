@@ -129,7 +129,8 @@ int MCPar::run(int nsamp, int nburn, const Real *pinit, VLFunc &L, MCout &outsam
       plugin(&p0[0], &lytrial[0]);                                    // L(nchain, pvals, lylast), mcpar.cc:53
       CHECK(mcgpu_set_state_host(eng, &p0[0], &lytrial[0]));
     } else {
-      CHECK(mcgpu_set_likelihood(eng, dl->lik_id(), par.empty() ? 0 : &par[0], (int)par.size()));
+      if (dl->plugin_path()) CHECK(mcgpu_set_likelihood_plugin(eng, dl->plugin_path(), par.empty() ? 0 : &par[0], (int)par.size()));
+      else CHECK(mcgpu_set_likelihood(eng, dl->lik_id(), par.empty() ? 0 : &par[0], (int)par.size()));
       CHECK(mcgpu_set_covariance(eng, incov));
       CHECK(mcgpu_set_state(eng, &p0[0]));
     }
