@@ -141,9 +141,11 @@ int  mcgpu_set_likelihood(mcgpu_engine *e, int lik, const double *par, int npar)
 /* A user-written likelihood inside the fused step kernels: cubin_path is a plugin built from one user header
  * (include/mcgpu_plugin.cuh, `python -m mcpar_b200.plugin`); par[npar] is copied to the device and handed to
  * the functor unchanged.  The engine then runs as with a built-in likelihood (lik = MCGPU_DEVICE_PLUGIN).
- * NORMAL mode, thread-per-chain kernels (even nparam <= 16).  MCGPU_EINVAL, before any launch, when the file
- * cannot be loaded, the plugin was built for another nparam or from other kernel sources (its stamp), or the
- * mode is VERIFY / REPLAY_LOCAL. */
+ * NORMAL mode.  A thread-per-chain plugin has an even nparam <= 16; a wide plugin (MCGPU_PLUGIN_WIDE) has nparam
+ * 8, 16, 32 or 64 and needs coin_group = 0.  MCGPU_EINVAL, before any launch, when the file cannot be loaded, the
+ * plugin was built for another nparam or from other kernel sources (its stamp), the mode is VERIFY / REPLAY_LOCAL,
+ * or a wide plugin meets coin_group != 0; MCGPU_ESTATE when the plugin's kind would change the layout of an
+ * installed state. */
 int  mcgpu_set_likelihood_plugin(mcgpu_engine *e, const char *cubin_path, const double *par, int npar);
 
 /* MCPar::covar_setup (mcpar.cc:454-484): incov is d x d row-major symmetric PD, or

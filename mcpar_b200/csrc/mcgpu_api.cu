@@ -217,20 +217,30 @@ void fill_step_params(mcgpu_engine *e, StepParams &p)
 // ---- device likelihood plugins (mh_plugin.cu compiled per user header into a cubin) --------------------------
 enum { PK_INIT = 6, PK_EVAL = 7 };           // plugin kernels beyond the six step phases PH_*
 
-// The one place that knows the plugin's symbol names: mh_plugin.cu instantiates mcgpu::fast::mh_steps_kernel
-// <MCGPU_DEVICE_PLUGIN, d, RNG_PHILOX = 0, phase> and init_loglik_kernel<MCGPU_DEVICE_PLUGIN, d>.
-std::string plugin_kernel_name(int d, int which)
+// The one place that knows the plugin's symbol names.  mh_plugin.cu instantiates, for a thread-per-chain plugin,
+// mcgpu::fast::mh_steps_kernel<MCGPU_DEVICE_PLUGIN, d, RNG_PHILOX = 0, phase> for the six phases and
+// init_loglik_kernel<MCGPU_DEVICE_PLUGIN, d>; for a wide plugin mh_wide_kernel<MCGPU_DEVICE_PLUGIN, d, nch, phase> for
+// PH_BURN, PH_LOCAL, PH_REMOTE and PH_REMOTE_SUM, and the batched evaluation kernel gives the initial log-likelihoods
+// of its (AoS) state.  An empty name: the kind has no kernel in that slot.
+std::string plugin_kernel_name(int d, int which, bool wide, int nch)
 {
   char b[128];
-  if (which == PK_EVAL) return "mcgpu_plugin_loglik";
-  if (which == PK_INIT) snprintf(b, sizeof b, "_ZN5mcgpu4fast18init_loglik_kernelILi%dELi%dEEEvNS_10StepParamsE", MCGPU_DEVICE_PLUGIN, d);
-  else snprintf(b, sizeof b, "_ZN5mcgpu4fast15mh_steps_kernelILi%dELi%dELi0ELi%dEEEvNS_10StepParamsE", MCGPU_DEVICE_PLUGIN, d, which);
+  if (which == PK_EVAL || (wide && which == PK_INIT)) return "mcgpu_plugin_loglik";
+  if (wide) {
+    if (which == PH_MIXED || which == PH_MIXED_SUM) return "";
+    snprintf(b, sizeof b, "_ZN5mcgpu4fast14mh_wide_kernelILi%dELi%dELi%dELi%dEEEvNS_10WideParamsE", MCGPU_DEVICE_PLUGIN, d, nch, which);
+  } else if (which == PK_INIT) {
+    snprintf(b, sizeof b, "_ZN5mcgpu4fast18init_loglik_kernelILi%dELi%dEEEvNS_10StepParamsE", MCGPU_DEVICE_PLUGIN, d);
+  } else {
+    snprintf(b, sizeof b, "_ZN5mcgpu4fast15mh_steps_kernelILi%dELi%dELi0ELi%dEEEvNS_10StepParamsE", MCGPU_DEVICE_PLUGIN, d, which);
+  }
   return b;
 }
 
 // Load a plugin cubin into the current device's context and check it before anything launches from it: it must
-// have been compiled from the kernel sources this library was (StepParams crosses by value) and for d parameters.
-int plugin_open(const char *path, int d, cudaLibrary_t *lib, cudaKernel_t k[8], std::string &err)
+// have been compiled from the kernel sources this library was (StepParams / WideParams cross by value), for d
+// parameters and, if wide, with the library's chains per lane group (the launch geometry depends on it).
+int plugin_open(const char *path, int d, cudaLibrary_t *lib, cudaKernel_t k[8], bool *wide, std::string &err)
 {
   *lib = nullptr;
   FILE *f = path ? fopen(path, "rb") : nullptr;
@@ -259,13 +269,31 @@ int plugin_open(const char *path, int d, cudaLibrary_t *lib, cudaKernel_t k[8], 
     snprintf(b, sizeof b, "plugin: built for nparam = %d, the engine has nparam = %d", np, d);
     cudaLibraryUnload(L); err = b; return MCGPU_EINVAL;
   }
-  for (int w = 0; w < 8; ++w)
-    if (cudaLibraryGetKernel(&k[w], L, plugin_kernel_name(d, w).c_str()) != cudaSuccess) {
+  void *pw = nullptr, *pc = nullptr; size_t bw = 0, bc = 0;
+  int iw = 0, nch = 0;
+  if (cudaLibraryGetGlobal(&pw, &bw, L, "mcgpu_plugin_wide") != cudaSuccess || bw != sizeof iw ||
+      cudaLibraryGetGlobal(&pc, &bc, L, "mcgpu_plugin_nch") != cudaSuccess || bc != sizeof nch ||
+      cudaMemcpy(&iw, pw, sizeof iw, cudaMemcpyDeviceToHost) != cudaSuccess ||
+      cudaMemcpy(&nch, pc, sizeof nch, cudaMemcpyDeviceToHost) != cudaSuccess) {
+    cudaGetLastError(); cudaLibraryUnload(L);
+    err = std::string("plugin: '") + path + "' does not say its kind (no mcgpu_plugin_wide / mcgpu_plugin_nch)";
+    return MCGPU_EINVAL;
+  }
+  if (iw && nch != fast::wide_launch(d, 0).nch) {
+    snprintf(b, sizeof b, "plugin: built with %d chains per lane group, this library launches %d: rebuild the plugin",
+             nch, fast::wide_launch(d, 0).nch);
+    cudaLibraryUnload(L); err = b; return MCGPU_EINVAL;
+  }
+  for (int w = 0; w < 8; ++w) {
+    const std::string name = plugin_kernel_name(d, w, iw != 0, nch);
+    k[w] = nullptr;
+    if (!name.empty() && cudaLibraryGetKernel(&k[w], L, name.c_str()) != cudaSuccess) {
       cudaGetLastError(); cudaLibraryUnload(L);
-      err = "plugin: kernel " + plugin_kernel_name(d, w) + " missing from the cubin";
+      err = "plugin: kernel " + name + " missing from the cubin";
       return MCGPU_EINVAL;
     }
-  *lib = L;
+  }
+  *lib = L; *wide = iw != 0;
   return MCGPU_OK;
 }
 
@@ -275,15 +303,26 @@ void plugin_release(mcgpu_engine *e)
   e->plugin = nullptr;
 }
 
-cudaError_t launch_plugin(mcgpu_engine *e, int which, const StepParams &p, unsigned grid, unsigned block, size_t smem)
+template <class Params>        // StepParams (thread-per-chain kernels) or WideParams (wide kernels)
+cudaError_t launch_plugin(mcgpu_engine *e, int which, const Params &p, unsigned grid, unsigned block, size_t smem)
 {
   const void *f = reinterpret_cast<const void *>(e->pk[which]);
   if (smem > 48 * 1024) {                            // per launch: the attribute is per device
     cudaError_t s = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (s != cudaSuccess) return s;
   }
-  void *args[] = {const_cast<StepParams *>(&p)};
+  void *args[] = {const_cast<Params *>(&p)};
   return cudaLaunchKernel(f, dim3(grid), dim3(block), args, smem, e->stream);
+}
+
+// the plugin's batched evaluation mcgpu_plugin_loglik (mh_plugin.cu) of n points x (AoS) into y: one thread per point,
+// or for a wide plugin one lane group of d/2 threads per point in CTAs of 128
+cudaError_t launch_plugin_eval(cudaKernel_t k, bool wide, int d, const double *par, int npar, const double *x, double *y,
+                               int n, cudaStream_t st)
+{
+  const unsigned block = wide ? 128 : 256, per = wide ? block / (d / 2) : block;
+  void *args[] = {(void *)&par, (void *)&npar, (void *)&x, (void *)&y, (void *)&n};
+  return cudaLaunchKernel(reinterpret_cast<const void *>(k), dim3((unsigned)((n + per - 1) / per)), dim3(block), args, 0, st);
 }
 
 // the grid, block and shared-memory rules of launch_lik_d (mh_dispatch.inl)
@@ -320,7 +359,13 @@ cudaError_t launch_steps_any(mcgpu_engine *e, int phase, const StepParams &p)
     w.pnbf = reinterpret_cast<const float*>(w.pf + (size_t)e->d * e->mpad); w.pscal = w.pnbf + e->mpad;
     w.gm2 = reinterpret_cast<const double2*>(e->gm_t);
     w.gm_lw = e->gm_t ? e->gm_t + (size_t)2 * e->d * e->kpad : nullptr; w.kpad = e->kpad;
-    return fast::launch_wide(e->lik, e->d, phase == PH_REMOTE && e->remote_mode == 1 ? PH_REMOTE_SUM : phase, w, e->stream);
+    w.lik_dev = e->lik_dev; w.lik_k = e->lik_k;
+    const int ph = phase == PH_REMOTE && e->remote_mode == 1 ? PH_REMOTE_SUM : phase;
+    if (e->lik == MCGPU_DEVICE_PLUGIN) {
+      const WideLaunch g = fast::wide_launch(e->d, w.C);
+      return launch_plugin(e, ph, w, g.grid, g.block, g.smem);
+    }
+    return fast::launch_wide(e->lik, e->d, ph, w, e->stream);
   }
   if (e->replay_local) return exact::launch_steps(e->lik, e->d, 1, phase == PH_BURN ? PH_BURN : PH_LOCAL, p, e->stream);
   if (e->remote_mode == 1) phase = phase == PH_MIXED ? PH_MIXED_SUM : (phase == PH_REMOTE ? PH_REMOTE_SUM : phase);
@@ -698,6 +743,17 @@ int mcgpu_set_stream(mcgpu_engine *e, void *cuda_stream)
   return MCGPU_OK;
 }
 
+// the wide kernels' derived buffers: column-major factor + "is diagonal" flag, and the prepared pool
+static int wide_buffers(mcgpu_engine *e)
+{
+  const int d = e->d, L = d / 2;
+  if (!e->factor_cm) { CK(cudaMalloc((void**)&e->factor_cm, (size_t)d * d * 8)); CK(cudaMalloc((void**)&e->diag_d, sizeof(int))); }
+  e->mpad = (e->M + L - 1) / L * L;
+  // (mu, h) pairs, sigma, n_s in fp64; then the fp32 copy: (g mu, g) pairs, n_s log2 e, 4 scalars
+  if (!e->pprep) CK(cudaMalloc((void**)&e->pprep, ((size_t)3 * d + 1) * e->mpad * 8 + ((size_t)2 * d + 1) * e->mpad * 4 + 16));
+  return MCGPU_OK;
+}
+
 int mcgpu_set_likelihood(mcgpu_engine *e, int lik, const double *par, int npar)
 {
   if (!e) return MCGPU_EINVAL;
@@ -735,10 +791,7 @@ int mcgpu_set_likelihood(mcgpu_engine *e, int lik, const double *par, int npar)
   e->lik = lik; e->lik_k = K;
   if (e->wide) {
     const int d = e->d, L = d / 2;
-    if (!e->factor_cm) { CK(cudaMalloc((void**)&e->factor_cm, (size_t)d * d * 8)); CK(cudaMalloc((void**)&e->diag_d, sizeof(int))); }
-    e->mpad = (e->M + L - 1) / L * L;
-    // (mu, h) pairs, sigma, n_s in fp64; then the fp32 copy: (g mu, g) pairs, n_s log2 e, 4 scalars
-    if (!e->pprep) CK(cudaMalloc((void**)&e->pprep, ((size_t)3 * d + 1) * e->mpad * 8 + ((size_t)2 * d + 1) * e->mpad * 4 + 16));
+    if (int rc2 = wide_buffers(e)) return rc2;
     if (e->gm_t) { cudaFree(e->gm_t); e->gm_t = nullptr; }
     if (lik == MCGPU_GAUSSMIX) {                        // [d][Kpad] (mu, 1/s2) pairs, then [Kpad] log w; padding has weight 0
       e->kpad = (K + 2 * L - 1) / (2 * L) * (2 * L);
@@ -769,14 +822,18 @@ int mcgpu_set_likelihood_plugin(mcgpu_engine *e, const char *cubin_path, const d
   if (npar < 0 || (npar > 0 && !par)) return fail(e, MCGPU_EINVAL, "par must hold npar reals");
   if (e->cfg.mode != MCGPU_MODE_NORMAL) return fail(e, MCGPU_EINVAL, "plugin likelihoods run in NORMAL mode only (not VERIFY or REPLAY_LOCAL)");
   if (e->hostlik) return fail(e, MCGPU_ESTATE, "this engine was set up for a host likelihood: create a new engine");
-  if (e->have_state && e->wide) return fail(e, MCGPU_ESTATE, "likelihood change would change the state layout: create a new engine");
-  if (e->cfg.pl < 1.0 && fast::steps_smem_bytes(e->d, e->cfg.sync, e->M, true) > 200 * 1024)
-    return fail(e, MCGPU_EINVAL, "remote-mixture pool does not fit in shared memory (40 bytes per slot and parameter + 16 per slot): choose pool_m with pool_m*nparam <= 4800");
   DeviceGuard g(e->dev);
-  cudaLibrary_t lib = nullptr; cudaKernel_t k[8]; std::string err;
-  const int rc = plugin_open(cubin_path, e->d, &lib, k, err);
+  cudaLibrary_t lib = nullptr; cudaKernel_t k[8]; bool wide = false; std::string err;
+  const int rc = plugin_open(cubin_path, e->d, &lib, k, &wide, err);
   if (rc) { e->err = err; return rc; }
+  auto refuse = [&](int code, const char *msg) { cudaLibraryUnload(lib); return fail(e, code, msg); };
+  if (wide && e->cfg.coin_group != 0)                     // the wide kernels draw one local / remote coin per step for the job
+    return refuse(MCGPU_EINVAL, "a wide plugin runs with the job-wide coin only: create the engine with coin_group = 0");
+  if (e->have_state && wide != e->wide) return refuse(MCGPU_ESTATE, "likelihood change would change the state layout: create a new engine");
+  if (!wide && e->cfg.pl < 1.0 && fast::steps_smem_bytes(e->d, e->cfg.sync, e->M, true) > 200 * 1024)   // wide kernels read the pool through L1
+    return refuse(MCGPU_EINVAL, "remote-mixture pool does not fit in shared memory (40 bytes per slot and parameter + 16 per slot): choose pool_m with pool_m*nparam <= 4800");
   CK(cudaStreamSynchronize(e->stream));                   // nothing of the previous likelihood is in flight
+  if (wide) { const int rcw = wide_buffers(e); if (rcw) { cudaLibraryUnload(lib); return rcw; } }
   plugin_release(e);
   e->plugin = lib; memcpy(e->pk, k, sizeof e->pk);
   if (e->lik_dev) { cudaFree(e->lik_dev); e->lik_dev = nullptr; }
@@ -787,7 +844,7 @@ int mcgpu_set_likelihood_plugin(mcgpu_engine *e, const char *cubin_path, const d
   }
   memset(e->lp, 0, sizeof e->lp);
   for (int i = 0; i < npar && i < 8; ++i) e->lp[i] = par[i];
-  e->lik = MCGPU_DEVICE_PLUGIN; e->lik_k = npar; e->wide = false;   // thread-per-chain kernels only
+  e->lik = MCGPU_DEVICE_PLUGIN; e->lik_k = npar; e->wide = wide;
   return MCGPU_OK;
 }
 
@@ -817,6 +874,16 @@ static int state_installed(mcgpu_engine *e)
   return MCGPU_OK;
 }
 
+// initial log-likelihoods L(nchain, pvals, lylast), mcpar.cc:53, on the wide kernels' AoS state: the exact unit for a
+// built-in likelihood, the plugin's batched evaluation for a plugin
+static cudaError_t wide_init_loglik(mcgpu_engine *e)
+{
+  if (e->lik == MCGPU_DEVICE_PLUGIN)
+    return launch_plugin_eval(e->pk[PK_EVAL], true, e->d, e->lik_dev, e->lik_k, e->x, e->ly, (int)e->C, e->stream);
+  LikSpec L; L.lik = e->lik; L.d = e->d; L.k = e->lik_k; memcpy(L.lp, e->lp, sizeof L.lp); L.dev = e->lik_dev;
+  return exact::launch_loglik_aos(L, e->x, e->ly, (int)e->C, e->stream);
+}
+
 int mcgpu_set_state(mcgpu_engine *e, const double *pinit)
 {
   if (!e || !pinit) return MCGPU_EINVAL;
@@ -834,9 +901,8 @@ int mcgpu_set_state(mcgpu_engine *e, const double *pinit)
     }
   } else if (e->wide) {
     CK(cudaMemcpyAsync(e->x, pinit, (size_t)e->C * d * 8, cudaMemcpyHostToDevice, e->stream));
-    LikSpec L; L.lik = e->lik; L.d = d; L.k = e->lik_k; memcpy(L.lp, e->lp, sizeof L.lp); L.dev = e->lik_dev;
     ++e->launches;
-    CK(exact::launch_loglik_aos(L, e->x, e->ly, (int)e->C, e->stream));   // L(nchain, pvals, lylast), mcpar.cc:53
+    CK(wide_init_loglik(e));
   } else {
     double *tmp = nullptr;
     CK(cudaMallocAsync((void**)&tmp, (size_t)e->C * d * 8, e->stream));
@@ -1784,8 +1850,8 @@ int mcgpu_loglik_plugin(int device, const char *cubin_path, int nparam, const do
   if (!x || !y || npset < 0 || npar < 0 || (npar > 0 && !par)) return fail(nullptr, MCGPU_EINVAL, "null argument");
   if (mcgpu_device_count() <= device || device < 0) return fail(nullptr, MCGPU_ENODEVICE, "no usable CUDA device (this engine has no CPU path)");
   DeviceGuard g(device);
-  cudaLibrary_t lib = nullptr; cudaKernel_t k[8]; std::string err;
-  const int rc = plugin_open(cubin_path, nparam, &lib, k, err);
+  cudaLibrary_t lib = nullptr; cudaKernel_t k[8]; bool wide = false; std::string err;
+  const int rc = plugin_open(cubin_path, nparam, &lib, k, &wide, err);
   if (rc) return fail(nullptr, rc, err.c_str());
   struct Unload { cudaLibrary_t l; ~Unload() { cudaLibraryUnload(l); } } unload = {lib};
   if (npset == 0) return MCGPU_OK;
@@ -1794,9 +1860,7 @@ int mcgpu_loglik_plugin(int device, const char *cubin_path, int nparam, const do
   if (npar > 0) CK0(cudaMalloc((void**)&dp, (size_t)npar * 8));
   if (npar > 0) CK0(cudaMemcpyAsync(dp, par, (size_t)npar * 8, cudaMemcpyHostToDevice, 0));
   CK0(cudaMemcpyAsync(dx, x, (size_t)npset * nparam * 8, cudaMemcpyHostToDevice, 0));
-  const double *cdp = dp, *cdx = dx;
-  void *args[] = {(void *)&cdp, (void *)&npar, (void *)&cdx, (void *)&dy, (void *)&npset};
-  CK0(cudaLaunchKernel(reinterpret_cast<const void *>(k[PK_EVAL]), dim3((unsigned)((npset + 255) / 256)), dim3(256), args, 0, 0));
+  CK0(launch_plugin_eval(k[PK_EVAL], wide, nparam, dp, npar, dx, dy, npset, 0));
   CK0(cudaMemcpyAsync(y, dy, (size_t)npset * 8, cudaMemcpyDeviceToHost, 0));
   CK0(cudaStreamSynchronize(0));
   cudaFree(dx); cudaFree(dy); if (dp) cudaFree(dp);
@@ -1850,8 +1914,7 @@ int mcgpu_set_state_sobol(mcgpu_engine *e, const double *plo, const double *phi,
   CK(cudaFreeAsync(dd, e->stream)); CK(cudaFreeAsync(dbox, e->stream));
   ++e->launches;
   if (e->wide) {
-    LikSpec L; L.lik = e->lik; L.d = d; L.k = e->lik_k; memcpy(L.lp, e->lp, sizeof L.lp); L.dev = e->lik_dev;
-    CK(exact::launch_loglik_aos(L, e->x, e->ly, (int)e->C, e->stream));   // L(nchain, pvals, lylast), mcpar.cc:53
+    CK(wide_init_loglik(e));
   } else {
     StepParams p; fill_step_params(e, p);
     CK(launch_init_any(e, p));

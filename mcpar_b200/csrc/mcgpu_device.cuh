@@ -145,7 +145,12 @@ struct WideParams {
   int exact_tests;                 // audit mode: accept / rejection / Hastings-factor decisions always in fp64 (MCGPU_EXACT_TESTS=1)
   // likelihood: GaussMix parameters, component fastest: gm2 [D][Kpad] = (mu, 1/s2) pairs, gm_lw [Kpad] = log w
   const double2 *gm2; const double *gm_lw; int kpad;
+  // device likelihood plugin: its par[] (lik_k reals) on the device
+  const double *lik_dev; int lik_k;
 };
+
+// Grid, block, dynamic shared memory and chains per lane group of a wide-kernel launch (wide_launch, mh_wide.cuh)
+struct WideLaunch { unsigned grid, block; size_t smem; int nch; };
 
 // One step of the host-callback likelihood path (mh_hostlik.cuh)
 struct HostLikParams {

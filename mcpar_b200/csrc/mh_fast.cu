@@ -14,24 +14,16 @@ bool wide_supported(int lik, int d)
   return (lik == MCGPU_ROSENBROCK1 || lik == MCGPU_GAUSSMIX) && (d == 8 || d == 16 || d == 32 || d == 64);
 }
 
-// chains per lane group: register-level reuse of the streamed GaussMix / pool parameters
-#ifndef MCGPU_WIDE_NCH64
-#define MCGPU_WIDE_NCH64 4
-#endif
-template <int D> struct WideNch { static constexpr int value = D >= 64 ? MCGPU_WIDE_NCH64 : (D >= 32 ? 2 : 1); };
-
 template <int LIK, int D>
 static cudaError_t launch_wide_d(int phase, const WideParams &p, cudaStream_t st)
 {
-  constexpr int L = D / 2, NCH = WideNch<D>::value;
-  const int block = 128, gpb = block / L, cpb = gpb * NCH;
-  const unsigned grid = (unsigned)((p.C + cpb - 1) / cpb);
-  const size_t smem = sizeof(double) * ((size_t)MCGPU_MATH_SMEM + (size_t)gpb * 2 * D * NCH);
+  constexpr int NCH = WideNch<D>::value;
+  const WideLaunch g = wide_launch(D, p.C);
   switch (phase) {
-    case PH_BURN:   mh_wide_kernel<LIK, D, NCH, PH_BURN><<<grid, block, smem, st>>>(p); break;
-    case PH_LOCAL:  mh_wide_kernel<LIK, D, NCH, PH_LOCAL><<<grid, block, smem, st>>>(p); break;
-    case PH_REMOTE: mh_wide_kernel<LIK, D, NCH, PH_REMOTE><<<grid, block, smem, st>>>(p); break;
-    case PH_REMOTE_SUM: mh_wide_kernel<LIK, D, NCH, PH_REMOTE_SUM><<<grid, block, smem, st>>>(p); break;
+    case PH_BURN:   mh_wide_kernel<LIK, D, NCH, PH_BURN><<<g.grid, g.block, g.smem, st>>>(p); break;
+    case PH_LOCAL:  mh_wide_kernel<LIK, D, NCH, PH_LOCAL><<<g.grid, g.block, g.smem, st>>>(p); break;
+    case PH_REMOTE: mh_wide_kernel<LIK, D, NCH, PH_REMOTE><<<g.grid, g.block, g.smem, st>>>(p); break;
+    case PH_REMOTE_SUM: mh_wide_kernel<LIK, D, NCH, PH_REMOTE_SUM><<<g.grid, g.block, g.smem, st>>>(p); break;
     default: return cudaErrorInvalidValue;
   }
   return cudaGetLastError();

@@ -6,6 +6,7 @@ enum { PH_BURN = 0, PH_MIXED = 1, PH_LOCAL = 2, PH_REMOTE = 3, PH_MIXED_SUM = 4,
 namespace fast {
 bool wide_supported(int lik, int d);
 cudaError_t launch_wide(int lik, int d, int phase, const WideParams &p, cudaStream_t st);
+WideLaunch wide_launch(int d, long long C);   // the wide kernels' launch rule (built-in likelihoods and plugins)
 cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, double2 *pmh, double *psd, double *pnb,
                              float2 *pf, float *pnbf, float *pscal,
                              const unsigned long long *arrivals, unsigned long long wait_target, int *xflag,

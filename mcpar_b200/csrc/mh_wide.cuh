@@ -86,6 +86,11 @@ __device__ __forceinline__ void load_staged(const double *s, double (&v)[NCH])
   }
 }
 
+// A wide device likelihood plugin (LIK = MCGPU_DEVICE_PLUGIN): partial(x, xs, p, part) is share `part` of the
+// log-likelihood at the point x[i * xs].  Declared only: mh_plugin.cu specialises it around the user's
+// UserLik::partial (include/mcgpu_plugin.cuh).
+template <int LIK, int D> struct WideLik;
+
 // log-likelihoods of the group's NCH chains; their points are staged in sx[i*NCH + c] and held
 // as (x0[c], x1[c]) per lane.  Every lane of the group returns the same values.
 template <int LIK, int D, int NCH>
@@ -93,13 +98,16 @@ __device__ __forceinline__ void wide_loglik(const double (&x0)[NCH], const doubl
                                             const WideParams &p, const MathTables &T, double (&out)[NCH])
 {
   constexpr int L = D / 2;
-  if (LIK == MCGPU_ROSENBROCK1) {               // rosenbrock.cc:4-21: the pair (2r, 2r+1) lives in lane r
+  if constexpr (LIK == MCGPU_ROSENBROCK1) {     // rosenbrock.cc:4-21: the pair (2r, 2r+1) lives in lane r
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
       const double t1 = 1 - x0[c];
       const double t2 = x1[c] - x0[c] * x0[c];
       out[c] = -group_sum<L>(t1 * t1 + 100.0 * t2 * t2);
     }
+  } else if constexpr (LIK == MCGPU_DEVICE_PLUGIN) {   // lane r returns share r; the butterfly order fixes the sum
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) out[c] = group_sum<L>(WideLik<LIK, D>::partial(sx + c, NCH, p, r));
   } else {
     // GaussMix: lane r evaluates components r, r+L, ... two at a time (kpad is a multiple of 2L;
     // padding components carry c = -inf).  The exponent is expanded once on the host,
@@ -298,6 +306,26 @@ __device__ __noinline__ double2 wide_pool_exact_sum(const double *sx, int c, int
     qs += gv; qm = gv > qm ? gv : qm;
   }
   return make_double2(group_sum<L>(qs), group_max<L>(qm));      // (sum, max)
+}
+
+// chains per lane group: register-level reuse of the streamed GaussMix / pool parameters
+#ifndef MCGPU_WIDE_NCH64
+#define MCGPU_WIDE_NCH64 4
+#endif
+constexpr int wide_nch(int d) { return d >= 64 ? MCGPU_WIDE_NCH64 : (d >= 32 ? 2 : 1); }
+template <int D> struct WideNch { static constexpr int value = wide_nch(D); };
+
+// The launch rule of mh_wide_kernel<LIK, d, WideNch<d>, PHASE>, for built-in likelihoods (mh_fast.cu) and wide
+// plugins (mcgpu_api.cu) alike: 128 threads, 128 / L lane groups per CTA, NCH chains per group, and in shared
+// memory the math tables plus each group's staged points sx[d][NCH] and normals sz[d][NCH].
+WideLaunch wide_launch(int d, long long C)
+{
+  const int L = d / 2, block = 128, gpb = block / L;
+  WideLaunch w;
+  w.nch = wide_nch(d); w.block = block;
+  w.grid = (unsigned)((C + gpb * w.nch - 1) / (gpb * w.nch));
+  w.smem = sizeof(double) * ((size_t)MCGPU_MATH_SMEM + (size_t)gpb * 2 * d * w.nch);
+  return w;
 }
 
 #ifndef MCGPU_WIDE_MINB

@@ -56,7 +56,8 @@ int GaussMix::lik_id() const { return MCGPU_GAUSSMIX; }
 
 DevicePlugin::DevicePlugin(const std::string &cubin_path, int nparam, const std::vector<double> &par) : path(cubin_path), n(nparam)
 {
-  if (n < 2 || n > 16 || n % 2 != 0) throw("a device plugin has an even nparam in 2..16");
+  if (n < 2 || n % 2 != 0 || (n > 16 && n != 32 && n != 64))
+    throw("a device plugin has an even nparam in 2..16 (thread-per-chain) or 8, 16, 32 or 64 (wide)");
   mpar = par;
 }
 int DevicePlugin::lik_id() const { return MCGPU_DEVICE_PLUGIN; }

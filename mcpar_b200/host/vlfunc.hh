@@ -37,7 +37,8 @@ protected:
 
 // A user-written likelihood compiled into a plugin cubin (include/mcgpu_plugin.cuh, python -m mcpar_b200.plugin):
 // MCPar::run loads it into every engine (mcgpu_set_likelihood_plugin) and operator() evaluates it on the GPU
-// (mcgpu_loglik_plugin).  par is handed to the functor unchanged.
+// (mcgpu_loglik_plugin).  par is handed to the functor unchanged.  A wide plugin (MCGPU_PLUGIN_WIDE) runs with the
+// job-wide coin only: set MCPar::coin_group = 0 (the default, -1, draws one coin per rank).
 class DevicePlugin : public DeviceVLFunc {
   const std::string path; const int n;
 public:

@@ -1,5 +1,6 @@
 """Build a device likelihood plugin: a cubin of the production step kernels instantiated with the functor of ONE
-user header (the contract is include/mcgpu_plugin.cuh).  Load it with Engine.set_likelihood("plugin", par,
+user header (the contract is include/mcgpu_plugin.cuh: thread-per-chain plugins at even nparam <= 16, wide plugins
+-- MCGPU_PLUGIN_WIDE -- at nparam 8, 16, 32 or 64).  Load it with Engine.set_likelihood("plugin", par,
 plugin=path) or mcgpu_set_likelihood_plugin.
 
   python -m mcpar_b200.plugin mylik.cuh -o mylik.cubin [--nparam N] [--force]
@@ -25,14 +26,18 @@ SHIPPED = [
     (os.path.join(b.ROOT, "examples", "likelihoods", "logistic.cuh"), None, "logistic.cubin"),
     (os.path.join(b.ROOT, "tests", "plugins", "rosen1_restated.cuh"), 2, "rosen1_restated_d2.cubin"),
     (os.path.join(b.ROOT, "tests", "plugins", "rosen1_restated.cuh"), 16, "rosen1_restated_d16.cubin"),
+    (os.path.join(b.ROOT, "examples", "likelihoods", "logistic_wide.cuh"), None, "logistic_wide.cubin"),
+    (os.path.join(b.ROOT, "tests", "plugins", "rosen1_wide.cuh"), 16, "rosen1_wide_d16.cubin"),
+    (os.path.join(b.ROOT, "tests", "plugins", "rosen1_wide.cuh"), 64, "rosen1_wide_d64.cubin"),
 ]
 
 
 def command(header, out, nparam=None, stamp=None):
     """The nvcc command that compiles `header` into the plugin cubin `out`."""
     header = os.path.abspath(header)
-    if nparam is not None and (not isinstance(nparam, int) or nparam < 2 or nparam > 16 or nparam % 2):
-        raise ValueError("nparam must be an even integer in 2..16 (thread-per-chain kernels), got %r" % (nparam,))
+    if nparam is not None and (not isinstance(nparam, int) or nparam < 2 or nparam % 2 or (nparam > 16 and nparam not in (32, 64))):
+        raise ValueError("nparam must be an even integer in 2..16 (thread-per-chain plugins) or 8, 16, 32 or 64 "
+                         "(wide plugins), got %r" % (nparam,))
     cmd = [b.NVCC] + b.ARCH + b.COMMON + ["-I", os.path.dirname(header), "-include", header,
                                           b.stamp_define(b.kernel_stamp() if stamp is None else stamp)]
     if nparam is not None:
