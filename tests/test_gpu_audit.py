@@ -17,7 +17,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 @pytest.mark.parametrize("case", ["dgauss", "rosen2", "rosen2_groups", "rosen4",
                                   "dgauss_sum", "rosen2_sum256", "rosen2_sum_groups", "rosen4_sum",
-                                  "rosen16_ref", "rosen16_sum", "gmix64_sum", "gmix64_sum256"])
+                                  "rosen16_ref", "rosen16_sum", "gmix64_sum", "gmix64_sum256",
+                                  "rosen32_ref", "rosen32_sum", "rosen64_ref", "rosen64_sum", "gmix64_k80_ref", "gmix64_k80_sum",
+                                  "rosen16_groups_ref", "rosen16_groups_sum", "rosen2_sync40_ref", "rosen2_sync40_sum"])
 def test_fp32_bounded_decisions_equal_fp64_decisions(case, tmp_path):
     outs = {}
     for mode in ("0", "1"):

@@ -8,6 +8,7 @@ log-likelihoods within 1e-12 relative (north star).
 import numpy as np
 import pytest
 
+import kernel_matrix as km
 from conftest import make_streams, tiled_pinit
 from oracle import mh
 
@@ -167,21 +168,17 @@ def test_stream_overrun_is_an_error():
 
 
 # ---------------------------------------------------------------- production kernel, replayed
-@pytest.mark.parametrize("lik,d,C,par,incov", [
-    ("rosenbrock1", 2, 96, None, None),
-    ("dualgaussian", 2, 200, [5.0], None),
-    ("rosenbrock1", 16, 64, None, "rosen16"),
-    ("gaussian", 2, 33, [0.5, -0.5, 1.5, 0.7], None),
-])
+@pytest.mark.parametrize("lik,d,C,par,incov", [pytest.param(c.lik, c.d, c.C, c.par, c.incov, id=c.id) for c in km.REPLAY])
 def test_production_kernel_replay_local(lik, d, C, par, incov):
     """The production step kernel (exact-arithmetic instantiation) fed the reference's
     streams at the reference's offsets, all-local run (pl = 1): one rank of C chains."""
     eng = _engine()
-    if incov == "rosen16":
-        blk = (2.38 ** 2 / 16) * np.array([[0.5, 1.0], [1.0, 2.505]])
-        incov = np.kron(np.eye(8), blk)
-    nburn, nsamp = 230, 75
     pin = tiled_pinit(C, d)
+    if incov == "rosen16":
+        incov = km.rosen_factor(16)
+    if isinstance(par, str):                         # GaussMix spec: chains start on the means
+        par, incov, pin = km.model(lik, d, C, par)
+    nburn, nsamp = 230, 75
     Z, U, I = make_streams(1, C, d, nsamp + nburn, 11, mult=2)
     o = mh.run_replay(lik, d, C, 1, nsamp, nburn, pin, Z, U, I, incov=incov, par=par, pl=1.0, trace=True)
     e = eng.Engine(d, C, mode="replay_local", pl=1.0, history_steps=nsamp)
@@ -189,7 +186,7 @@ def test_production_kernel_replay_local(lik, d, C, par, incov):
     e.set_streams(0, Z[0], U[0])
     e.burnin(nburn); e.sample_begin(nsamp); e.sample(nsamp); e.synchronize()
     st = e.state()
-    poly = lik != "dualgaussian"
+    poly = lik not in ("dualgaussian", "gaussmix")
     assert np.array_equal(st["p"], o["p"][0])
     assert np.array_equal(e.factor(), o["cov"][0]), "burn-in tuning history differs"
     assert np.array_equal(st["mu"], o["mu"][0]) and np.array_equal(st["psum2"], o["psum2"][0])
@@ -202,58 +199,30 @@ def test_production_kernel_replay_local(lik, d, C, par, incov):
 
 
 # ---------------------------------------------------------------- normal mode vs counter oracle
-@pytest.mark.parametrize("lik,d,N,par,pool_m,pl,cg,rmode,lag", [
-    ("rosenbrock1", 2, 256, None, 0, 0.9, 32, 0, 0),
-    ("rosenbrock1", 2, 512, None, 16, 0.7, 32, 0, 0),
-    ("dualgaussian", 2, 256, [5.0], 8, 0.8, 32, 0, 0),
-    ("rosenbrock1", 4, 128, None, 8, 0.8, 32, 0, 0),
-    ("dualgaussian", 2, 256, [5.0], 8, 0.8, 4, 0, 0),       # rank-sized coin groups (mixed warps)
-    ("dualgaussian", 2, 512, [5.0], 16, 0.7, 0, 0, 0),      # job-wide coin: host-planned local / remote launches
-    ("rosenbrock1", 2, 200, None, 10, 0.6, 0, 0, 0),        # ragged: chains not a multiple of 32, pool not of 8
-    ("rosenbrock1", 16, 72, "rosen16", 8, 0.7, 0, 0, 0),    # wide kernel: 8 lanes per chain, full lower factor
-    ("rosenbrock1", 8, 40, None, 5, 0.7, 0, 0, 0),          # wide kernel: 4 lanes per chain, diagonal factor
-    ("gaussmix", 64, 24, "gmix64", 6, 0.7, 0, 0, 0),        # wide kernel: one chain per warp, K = 64 mixture; pool M < D/2 lanes
-    ("gaussmix", 16, 48, "gmix16", 8, 0.8, 0, 0, 0),
-    ("dualgaussian", 2, 512, [5.0], 16, 0.7, 0, 0, 1),      # pool read one exchange late
-    ("rosenbrock1", 2, 256, None, 8, 0.7, 32, 0, 1),
-    # remote mode 1: sum-mixture independence proposal with normalised components (no rejection loop)
-    ("dualgaussian", 2, 512, [5.0], 16, 0.7, 0, 1, 0),
-    ("dualgaussian", 2, 512, [5.0], 64, 0.6, 0, 1, 1),
-    ("rosenbrock1", 2, 200, None, 10, 0.6, 0, 1, 0),        # ragged
-    ("rosenbrock1", 2, 256, None, 0, 0.8, 32, 1, 0),        # every chain in the pool, per-group coins
-    ("dualgaussian", 2, 256, [5.0], 8, 0.8, 4, 1, 1),       # rank-sized coin groups (mixed warps), lagged pool
-    ("rosenbrock1", 4, 128, None, 8, 0.8, 32, 1, 0),
-    ("rosenbrock1", 16, 72, "rosen16", 8, 0.7, 0, 1, 0),    # wide kernels in remote mode 1
-    ("rosenbrock1", 8, 40, None, 5, 0.7, 0, 1, 1),
-    ("gaussmix", 64, 24, "gmix64", 6, 0.7, 0, 1, 0),
-    ("gaussmix", 64, 136, "gmix64", 40, 0.7, 0, 1, 1),
-    ("gaussmix", 64, 256, "gmix64", 0, 0.7, 0, 1, 0),       # every chain in the pool: M = 256, one pool slot per mixture-warp thread
-    ("gaussmix", 16, 48, "gmix16", 8, 0.8, 0, 1, 0),
-])
-def test_normal_mode_matches_counter_oracle(lik, d, N, par, pool_m, pl, cg, rmode, lag):
+@pytest.mark.parametrize("lik,d,N,par,pool_m,pl,cg,rmode,lag,sync,thin,nsamp,expanded", [
+    pytest.param(c.lik, c.d, c.N, c.par, c.pool_m, c.pl, c.cg, c.rmode, c.lag, c.sync, c.thin, c.nsamp,
+                 any(k[0] != "steps" for k in c.claims), id=c.id) for c in km.CASES])
+def test_normal_mode_matches_counter_oracle(lik, d, N, par, pool_m, pl, cg, rmode, lag, sync, thin, nsamp, expanded):
     """Same Philox draws on both sides: identical accept sequences; values agree to
-    rounding (host libm vs CUDA libm differ in the last ulp of log/sin/cos/exp)."""
+    rounding (host libm vs CUDA libm differ in the last ulp of log/sin/cos/exp).  Every kept
+    log-likelihood and the final state's are the likelihood of their own row, to the kernel's
+    fp64 error bound against an extended-precision evaluation.  The cases and the kernels
+    each one launches: tests/kernel_matrix.py (`expanded`: a wide or cooperative kernel evaluates the run's
+    GaussMix in the expanded form)."""
     eng = _engine()
-    nburn, nsamp = 120, 60
-    pin = tiled_pinit(N, d)
-    incov = None
-    if par == "rosen16":
-        par, incov = None, np.kron(np.eye(8), (2.38 ** 2 / 16) * np.array([[0.5, 1.0], [1.0, 2.505]]))
-    elif isinstance(par, str):                       # K-component mixture in d dimensions, chains start on the means
-        K = {"gmix64": 64, "gmix16": 5}[par]
-        rng = np.random.default_rng(8)
-        gmu = rng.uniform(-5, 5, (K, d)); gs2 = rng.uniform(0.5, 2.0, (K, d))
-        par = mh.gaussmix_params(K, d, gmu, gs2, np.ones(K))
-        pin = gmu[np.arange(N) % K].copy()
-        incov = np.eye(d) * (2.38 ** 2 / d)
+    nburn = km.NBURN
+    kept = (nsamp + thin - 1) // thin
+    par, incov, pin = km.model(lik, d, N, par)
     o = mh.run_counter(lik, d, N, nsamp, nburn, pin, incov=incov, par=par, pool_m=pool_m, pl=pl, coin_group=cg, trace=True,
-                       remote_mode=rmode, pool_lag=lag)
-    e = eng.Engine(d, N, mode="normal", pool_m=pool_m, pl=pl, coin_group=cg, history_steps=nsamp, remote_mode=rmode, pool_lag=lag)
+                       remote_mode=rmode, pool_lag=lag, sync=sync, thin=thin)
+    e = eng.Engine(d, N, mode="normal", pool_m=pool_m, pl=pl, coin_group=cg, history_steps=kept, remote_mode=rmode,
+                   pool_lag=lag, sync=sync, thin=thin)
     e.run(nsamp, nburn, pin, lik, par, incov)
     st = e.state()
     h = e.history()
     # accept pattern of the main phase from the history: a row changed iff accepted
     same_state = np.all(np.isclose(h[:, :, :d], o["rows"][:, :, :d], rtol=1e-7, atol=1e-9), axis=-1)
+    print("rows agreeing with the oracle: %.5f" % same_state.mean())
     assert same_state.mean() > 0.999, "trajectories diverged: %.4f agree" % same_state.mean()
     # log-likelihood column of the rows whose state agrees: the kernels' table-driven fp64 math (and the
     # one-exponential form of DualGaussian) against the host libm evaluation of the reference's formula
@@ -282,6 +251,16 @@ def test_normal_mode_matches_counter_oracle(lik, d, N, par, pool_m, pl, cg, rmod
     assert s["exact_fallbacks"] >= 0
     pool = e.musig()
     assert np.allclose(pool, o["pool"], rtol=1e-6, atol=1e-8) or same_state[-1].mean() > 0.995
+    # every kept row and the final state: ly is log L of the row's own point, within the kernel's rounding bound
+    # (a kernel that stores x' with the old log-likelihood, or a partly live lane group that writes stale values, fails)
+    x = np.concatenate([h[:, :, :d].reshape(-1, d), st["p"]])
+    y = np.concatenate([h[:, :, d].ravel(), st["ly"]])
+    L, S, c = km.loglik_ld(lik, d, x, par, expanded)
+    inf = np.isinf(L)
+    assert np.array_equal(np.isinf(y), inf) and np.all(y[inf] == L[inf])
+    ratio = (np.abs(y[~inf] - L[~inf]) / (c * km.EPS * S[~inf])).astype(float)
+    print("max |ly - L| / (c eps S) = %.3g  (c = %d, max S = %.3g)" % (ratio.max(), c, float(S.max())))
+    assert ratio.max() <= 1.0, "log-likelihood off its row by %.3g times its rounding bound" % ratio.max()
     e.close()
 
 
