@@ -21,7 +21,7 @@ ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-ccbin", "/usr/bin/g++",
           "-I", os.path.join(ROOT, "include")]
 # Sources that fix the layout and meaning of what the engine hands a plugin's kernels (StepParams and WideParams by
-# value, the kernel templates they instantiate, the wide kernels' launch rule).  Their hash is compiled into libmcgpu.so and into every plugin; the
+# value, the kernel templates they instantiate, both kernel families' launch rules).  Their hash is compiled into libmcgpu.so and into every plugin; the
 # engine loads only plugins whose stamp equals its own.
 STAMPED = ["include/mcgpu.h", "mcpar_b200/csrc/mcgpu_device.cuh", "mcpar_b200/csrc/mh_kernels.cuh",
            "mcpar_b200/csrc/mcgpu_math.cuh", "mcpar_b200/csrc/mcgpu_tables.h", "mcpar_b200/csrc/mh_plugin.cu",

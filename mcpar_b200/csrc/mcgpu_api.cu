@@ -52,7 +52,7 @@ struct mcgpu_engine {
   unsigned long long *counts = nullptr;   // [0,1] window, [2,3] cumulative, [4,5] main-phase stats, [6,7] remote chain-steps / candidate iterations, [8,9] exchange wait ns / waits, [10] exact-path fallbacks of the bounded tests
   // exchange region (one allocation, IPC-exportable): NPOOL pool buffers [M][d][2] + the arrival counter
   char *xchg = nullptr; size_t pool_bytes = 0, xchg_bytes = 0;
-  double *pool[4] = {nullptr, nullptr, nullptr, nullptr}; int M = 0; long long stride = 1; bool pool_in_smem = true;
+  double *pool[4] = {nullptr, nullptr, nullptr, nullptr}; int M = 0; long long stride = 1;
   long long npub = 0;                      // publications completed since create: publication k lives in pool[k % nbuf]
   int lag = 0, remote_mode = 0;            // cfg.pool_lag, cfg.remote_mode
   bool p2p = false, p2p_local = false; int p2p_world = 0; char **peers_d = nullptr; std::vector<void*> peer_opened; int *xflag_d = nullptr;
@@ -205,7 +205,7 @@ void fill_step_params(mcgpu_engine *e, StepParams &p)
   p.sync = e->cfg.sync; p.coin_group = e->cfg.coin_group; p.pl = e->cfg.pl;
   p.first_remote_t = e->cfg.sync * (1 + e->lag);
   p.hist_cap = (int)std::max<long long>(e->hist_cap, 1);
-  p.pool_m = e->M; p.pool_stride = e->stride; p.pool_in_smem = e->pool_in_smem;
+  p.pool_m = e->M; p.pool_stride = e->stride;
   p.thin = e->cfg.thin;
   static const int exact_tests = getenv("MCGPU_EXACT_TESTS") ? atoi(getenv("MCGPU_EXACT_TESTS")) : 0;
   p.exact_tests = exact_tests;
@@ -215,13 +215,14 @@ void fill_step_params(mcgpu_engine *e, StepParams &p)
 }
 
 // ---- device likelihood plugins (mh_plugin.cu compiled per user header into a cubin) --------------------------
-enum { PK_INIT = 6, PK_EVAL = 7 };           // plugin kernels beyond the six step phases PH_*
+enum { PK_INIT = 6, PK_EVAL = 7 };           // plugin kernels beyond the step phases PH_* (0..5)
 
 // The one place that knows the plugin's symbol names.  mh_plugin.cu instantiates, for a thread-per-chain plugin,
-// mcgpu::fast::mh_steps_kernel<MCGPU_DEVICE_PLUGIN, d, RNG_PHILOX = 0, phase> for the six phases and
-// init_loglik_kernel<MCGPU_DEVICE_PLUGIN, d>; for a wide plugin mh_wide_kernel<MCGPU_DEVICE_PLUGIN, d, nch, phase> for
-// PH_BURN, PH_LOCAL, PH_REMOTE and PH_REMOTE_SUM, and the batched evaluation kernel gives the initial log-likelihoods
-// of its (AoS) state.  An empty name: the kind has no kernel in that slot.
+// mcgpu::fast::mh_steps_kernel<MCGPU_DEVICE_PLUGIN, d, RNG_PHILOX = 0, phase> for PH_BURN, PH_MIXED, PH_LOCAL and
+// PH_MIXED_SUM, and init_loglik_kernel<MCGPU_DEVICE_PLUGIN, d>; for a wide plugin
+// mh_wide_kernel<MCGPU_DEVICE_PLUGIN, d, nch, phase> for PH_BURN, PH_LOCAL, PH_REMOTE and PH_REMOTE_SUM, and the
+// batched evaluation kernel gives the initial log-likelihoods of its (AoS) state.  An empty name: the kind has no
+// kernel in that slot.
 std::string plugin_kernel_name(int d, int which, bool wide, int nch)
 {
   char b[128];
@@ -229,6 +230,8 @@ std::string plugin_kernel_name(int d, int which, bool wide, int nch)
   if (wide) {
     if (which == PH_MIXED || which == PH_MIXED_SUM) return "";
     snprintf(b, sizeof b, "_ZN5mcgpu4fast14mh_wide_kernelILi%dELi%dELi%dELi%dEEEvNS_10WideParamsE", MCGPU_DEVICE_PLUGIN, d, nch, which);
+  } else if (which == PH_REMOTE || which == PH_REMOTE_SUM) {
+    return "";
   } else if (which == PK_INIT) {
     snprintf(b, sizeof b, "_ZN5mcgpu4fast18init_loglik_kernelILi%dELi%dEEEvNS_10StepParamsE", MCGPU_DEVICE_PLUGIN, d);
   } else {
@@ -325,14 +328,6 @@ cudaError_t launch_plugin_eval(cudaKernel_t k, bool wide, int d, const double *p
   return cudaLaunchKernel(reinterpret_cast<const void *>(k), dim3((unsigned)((n + per - 1) / per)), dim3(block), args, 0, st);
 }
 
-// the grid, block and shared-memory rules of launch_lik_d (mh_dispatch.inl)
-cudaError_t launch_plugin_steps(mcgpu_engine *e, int phase, const StepParams &p)
-{
-  const int block = fast::step_block();
-  const size_t smem = fast::steps_smem_bytes(e->d, p.nsteps, p.pool_m, phase != PH_BURN && phase != PH_LOCAL);
-  return launch_plugin(e, phase, p, (unsigned)((p.C + block - 1) / block), block, smem);
-}
-
 // initial log-likelihoods L(nchain, pvals, lylast), mcpar.cc:53, on the SoA state
 cudaError_t launch_init_any(mcgpu_engine *e, const StepParams &p)
 {
@@ -368,14 +363,17 @@ cudaError_t launch_steps_any(mcgpu_engine *e, int phase, const StepParams &p)
     return fast::launch_wide(e->lik, e->d, ph, w, e->stream);
   }
   if (e->replay_local) return exact::launch_steps(e->lik, e->d, 1, phase == PH_BURN ? PH_BURN : PH_LOCAL, p, e->stream);
-  if (e->remote_mode == 1) phase = phase == PH_MIXED ? PH_MIXED_SUM : (phase == PH_REMOTE ? PH_REMOTE_SUM : phase);
-  if (e->lik == MCGPU_DEVICE_PLUGIN) return launch_plugin_steps(e, phase, p);
+  if (e->remote_mode == 1 && phase == PH_MIXED) phase = PH_MIXED_SUM;
+  if (e->lik == MCGPU_DEVICE_PLUGIN) {
+    const StepLaunch g = fast::steps_launch(e->d, p.C, p.nsteps, p.pool_m, phase);
+    return launch_plugin(e, phase, p, g.grid, g.block, g.smem);
+  }
   return fast::launch_steps(e->lik, e->d, 0, phase, p, e->stream);
 }
 
 // Host copy of the device's Philox4x32-10 (mcgpu_device.cuh): with a job-wide coin the host
-// evaluates each step's local/remote draw itself and plans PH_LOCAL / PH_REMOTE launches
-// without a device round trip.
+// evaluates each step's local/remote draw itself and plans the window's launches without a
+// device round trip.
 double host_coin(const mcgpu_engine *e, uint32_t step)
 {
   // the coin is word 2*NP+1 of chain 0's local stream (mcgpu_device.cuh "draws")
@@ -649,7 +647,6 @@ int mcgpu_create(const mcgpu_config *cfg, mcgpu_engine **out)
     if (never_remote && cfg->pool_m <= 0) e->M = 1;        // pool is never read: keep one slot
     if (!never_remote && cfg->pool_m <= 0 && e->N > (1 << 20)) return bail(MCGPU_EINVAL, "pool_m = 0 (all chains) is limited to 2^20 chains; choose a pool size");
     e->stride = e->N / e->M;
-    e->pool_in_smem = true;
     TRY(dalloc(e, &e->x, (size_t)d * e->ld)); TRY(dalloc(e, &e->ly, (size_t)e->ld));
     TRY(dalloc(e, &e->mu, (size_t)d * e->ld)); TRY(dalloc(e, &e->ps, (size_t)d * e->ld));
     TRY(dalloc(e, &e->factor, (size_t)d * d)); TRY(dalloc(e, &e->counts, 12));
@@ -1114,7 +1111,7 @@ int mcgpu_sample(mcgpu_engine *e, int nsteps)
         p.step0 = (uint32_t)(e->nburn_total + e->t_main); p.nsteps = n; p.t0 = (int)e->t_main;
         p.pool_next = publish;
         CK(launch_steps_any(e, PH_MIXED, p));
-      } else {                                               // job-wide coin: runs of local / remote steps
+      } else {                                               // job-wide coin: the host cuts the window into segments
         // wide kernels read the pool as (mu, -1/2sig^2, sig), slot-fastest: prepared right before the window's
         // first remote launch (with a peer-to-peer exchange that kernel also waits for the arrivals, so the
         // window's leading local steps overlap the exchange)
@@ -1131,30 +1128,30 @@ int mcgpu_sample(mcgpu_engine *e, int nsteps)
         auto is_remote = [&](long long tt) {
           return tt >= (long long)sync * (1 + e->lag) && !(host_coin(e, (uint32_t)(e->nburn_total + tt)) <= e->cfg.pl);   // mcpar.cc:142-152
         };
-        static const int plan = getenv("MCGPU_PLAN") ? atoi(getenv("MCGPU_PLAN")) : 1;
-        uint32_t mask = 0;
-        for (int k = 0; k < n && k < 32; ++k) if (is_remote(e->t_main + k)) mask |= 1u << k;
-        if (plan && !e->wide && n <= 32) {
-          // one launch per window: the lean local kernel when no step of the window is remote,
-          // otherwise the two-path kernel with the host-drawn plan (uniform branches)
-          p.step0 = (uint32_t)(e->nburn_total + e->t_main); p.nsteps = n; p.t0 = (int)e->t_main;
-          p.pool_next = publish;
-          p.plan_mask = mask; p.plan_valid = 1;
-          CK(launch_steps_any(e, mask ? PH_MIXED : PH_LOCAL, p));
-        } else {
-          int k = 0;
-          while (k < n) {
-            const long long t = e->t_main + k;
+        int k = 0;
+        while (k < n) {
+          const long long t = e->t_main + k;
+          int len, phase;
+          if (e->wide) {                                     // runs of local / remote steps, one launch each
             const bool rem = is_remote(t);
-            int len = 1;
+            len = 1;
             while (k + len < n && is_remote(t + len) == rem) ++len;
-            p.step0 = (uint32_t)(e->nburn_total + t); p.nsteps = len; p.t0 = (int)t;
-            p.hist_ring0 = e->hist ? (int)((t / e->cfg.thin) % e->hist_cap) : 0;
-            p.pool_next = (k + len == n) ? publish : nullptr;
             if (rem && !prepped) CK(pool_prep());
-            CK(launch_steps_any(e, rem ? PH_REMOTE : PH_LOCAL, p));
-            k += len;
+            phase = rem ? PH_REMOTE : PH_LOCAL;
+          } else {
+            // chunks of up to 32 steps (the plan's width): the lean local kernel when no step of the chunk is
+            // remote, otherwise the two-path kernel with the host-drawn plan (uniform branches)
+            len = std::min(n - k, 32);
+            uint32_t mask = 0;
+            for (int i = 0; i < len; ++i) if (is_remote(t + i)) mask |= 1u << i;
+            p.plan_mask = mask; p.plan_valid = 1;
+            phase = mask ? PH_MIXED : PH_LOCAL;
           }
+          p.step0 = (uint32_t)(e->nburn_total + t); p.nsteps = len; p.t0 = (int)t;
+          p.hist_ring0 = e->hist ? (int)((t / e->cfg.thin) % e->hist_cap) : 0;
+          p.pool_next = (k + len == n) ? publish : nullptr;
+          CK(launch_steps_any(e, phase, p));
+          k += len;
         }
       }
     }

@@ -106,7 +106,6 @@ struct StepParams {
   const unsigned long long *arrivals; unsigned long long wait_target, pub_wait_target; int *xflag;
   unsigned long long *xstat;       // {ns CTA 0 spent waiting for arrivals, launches that waited}
   int pool_m; long long pool_stride;
-  int pool_in_smem;
   int exact_tests;                 // audit mode: accept / rejection tests always in fp64 (MCGPU_EXACT_TESTS=1)
   // sample history: rows (p..., logL), kept step major, then hosted chain
   // (a ring of hist_cap kept steps; the first kept step of this launch goes to ring row hist_ring0)
@@ -151,6 +150,8 @@ struct WideParams {
 
 // Grid, block, dynamic shared memory and chains per lane group of a wide-kernel launch (wide_launch, mh_wide.cuh)
 struct WideLaunch { unsigned grid, block; size_t smem; int nch; };
+// Grid, block and dynamic shared memory of a thread-per-chain step-kernel launch (steps_launch, mh_kernels.cuh)
+struct StepLaunch { unsigned grid, block; size_t smem; };
 
 // One step of the host-callback likelihood path (mh_hostlik.cuh)
 struct HostLikParams {

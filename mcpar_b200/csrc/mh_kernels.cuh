@@ -16,6 +16,7 @@
 // Kernel 2  mh_verify_kernel                  verification mode: one CTA per emulated
 //           MPI rank, the reference's lock-step stream protocol (SURVEY.md 8c).
 #pragma once
+#include <stdlib.h>
 #include "mcgpu_device.cuh"
 #include "../../include/mcgpu.h"
 #ifndef MCGPU_EXACT_TU
@@ -438,12 +439,12 @@ __device__ __forceinline__ bool remote_candidate(uint32_t tlo, uint32_t thi, uin
 //   PH_MIXED   main steps, one local/remote coin per group of <= 32 chains (a warp may hold
 //              both kinds of step)                                                  mcpar.cc:113-210
 //   PH_LOCAL   main steps known to be local for every chain (job-wide coin, or t < SYNCSTEP)
-//   PH_REMOTE  main steps known to be remote for every chain (job-wide coin)
 // With a job-wide coin (coin_group = 0: "one coin per rank per step", the rank being the whole
 // job) the host knows each step's kind in advance -- the coin is a counter-based draw -- and
-// launches lean PH_LOCAL kernels (no remote code, few registers, full occupancy) and dedicated
-// PH_REMOTE kernels instead of the mixed one.
-//   PH_MIXED_SUM / PH_REMOTE_SUM  the same two with remote mode 1: the sum-mixture proposal below
+// launches chunks of up to 32 steps: the lean PH_LOCAL kernel (no remote code, few registers,
+// full occupancy) when no step of the chunk is remote, otherwise PH_MIXED with the chunk's plan.
+//   PH_MIXED_SUM  PH_MIXED with remote mode 1: the sum-mixture proposal below
+// PH_REMOTE / PH_REMOTE_SUM (all steps remote) are phases of the wide kernels only (mh_wide.cuh).
 enum { PH_BURN = 0, PH_MIXED = 1, PH_LOCAL = 2, PH_REMOTE = 3, PH_MIXED_SUM = 4, PH_REMOTE_SUM = 5 };
 
 // ---- remote mode 1: sum-mixture independence proposal ----------------------------------------------
@@ -609,10 +610,9 @@ __global__ void __launch_bounds__(128, (D <= 2 ? ((PHASE == PH_BURN || PHASE == 
 mh_steps_kernel(const StepParams p)
 {
   constexpr bool MAIN = PHASE != PH_BURN;
-  constexpr bool SUMMIX = PHASE == PH_MIXED_SUM || PHASE == PH_REMOTE_SUM;       // remote mode 1
+  constexpr bool SUMMIX = PHASE == PH_MIXED_SUM;                                  // remote mode 1
   constexpr bool MIXED = PHASE == PH_MIXED || PHASE == PH_MIXED_SUM;
-  constexpr bool ALLREMOTE = PHASE == PH_REMOTE || PHASE == PH_REMOTE_SUM;
-  constexpr bool CAN_REMOTE = RNGK == RNG_PHILOX && (MIXED || ALLREMOTE);
+  constexpr bool CAN_REMOTE = RNGK == RNG_PHILOX && MIXED;
   extern __shared__ __align__(16) double smem[];
   __shared__ unsigned char s_rank[4][32];               // per warp: lanes of the chains still in the remote loop
   __shared__ unsigned int s_stat[3];                    // remote chain-steps of this CTA, the candidates they tried, exact-path fallbacks
@@ -675,7 +675,7 @@ mh_steps_kernel(const StepParams p)
     const uint32_t step = p.step0 + (uint32_t)k;
     const int t = p.t0 + k;
     double u_acc;
-    bool remote = ALLREMOTE;
+    bool remote = false;
     long long zoff = 0;
     constexpr int NP = (D + 1) / 2;                   // normal pairs per proposal
     constexpr int ABLK = (2 * NP) / 4, AW = (2 * NP) % 4;   // accept uniform: word 2*NP of the local stream
@@ -949,6 +949,35 @@ mh_steps_kernel(const StepParams p)
       if (s_stat[2]) atomicAdd(p.counts + 6, (unsigned long long)s_stat[2]);
     }
   }
+}
+
+// CTA size of the step kernels (<= 128, the kernels' launch bound); MCGPU_BLOCK env overrides for tuning
+int step_block()
+{
+  static int b = 0;
+  if (!b) { const char *e = getenv("MCGPU_BLOCK"); b = e ? atoi(e) : 128; if (b != 32 && b != 64 && b != 128) b = 128; }
+  return b;
+}
+
+// smem: the math tables, the [d*d] factor, the [nsteps] 1/pwgt table and, for the phases that can take a remote
+// step, the pool: (mu, h) + sigma in fp64, (g mu, g) + (sigma, mu) in fp32 = 40 bytes per slot and parameter,
+// + n_s (fp64) and nb_s (fp32) per slot
+size_t steps_smem_bytes(int d, int nsteps, int pool_m, bool with_pool)
+{
+  const size_t mpad = (size_t)((pool_m + 7) & ~7);
+  return sizeof(double) * ((size_t)MCGPU_MATH_SMEM + (size_t)d * d + (size_t)((nsteps + 1) & ~1) + (with_pool ? mpad * d * 5 + mpad * 2 : 0));
+}
+
+// The launch rule of mh_steps_kernel<LIK, d, RNG, phase>, for built-in likelihoods (mh_dispatch.inl) and
+// thread-per-chain plugins (mcgpu_api.cu) alike: one thread per chain in CTAs of step_block() threads.
+StepLaunch steps_launch(int d, long long C, int nsteps, int pool_m, int phase)
+{
+  StepLaunch s;
+  const int block = step_block();
+  s.block = (unsigned)block;
+  s.grid = (unsigned)((C + block - 1) / block);
+  s.smem = steps_smem_bytes(d, nsteps, pool_m, phase != PH_BURN && phase != PH_LOCAL);
+  return s;
 }
 
 // Burn-in tuning, mcpar.cc:78-96, applied at a window boundary.

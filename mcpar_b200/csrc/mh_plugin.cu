@@ -82,9 +82,7 @@ template <> struct Lik<MCGPU_DEVICE_PLUGIN, PD> {
 template __global__ void mh_steps_kernel<MCGPU_DEVICE_PLUGIN, PD, RNG_PHILOX, PH_BURN>(const StepParams);
 template __global__ void mh_steps_kernel<MCGPU_DEVICE_PLUGIN, PD, RNG_PHILOX, PH_MIXED>(const StepParams);
 template __global__ void mh_steps_kernel<MCGPU_DEVICE_PLUGIN, PD, RNG_PHILOX, PH_LOCAL>(const StepParams);
-template __global__ void mh_steps_kernel<MCGPU_DEVICE_PLUGIN, PD, RNG_PHILOX, PH_REMOTE>(const StepParams);
 template __global__ void mh_steps_kernel<MCGPU_DEVICE_PLUGIN, PD, RNG_PHILOX, PH_MIXED_SUM>(const StepParams);
-template __global__ void mh_steps_kernel<MCGPU_DEVICE_PLUGIN, PD, RNG_PHILOX, PH_REMOTE_SUM>(const StepParams);
 template __global__ void init_loglik_kernel<MCGPU_DEVICE_PLUGIN, PD>(const StepParams);
 
 }}  // namespace mcgpu::fast

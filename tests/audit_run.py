@@ -49,7 +49,7 @@ CASES = {
     "rosen64_sum": ("rosenbrock1", None, 64, 250, 16, 0.5, 0, 150, 100, 1),
     "gmix64_k80_ref": ("gaussmix", None, 64, 200, 40, 0.5, 0, 100, 100, 0, 10, 80),
     "gmix64_k80_sum": ("gaussmix", None, 64, 200, 40, 0.5, 0, 100, 100, 1, 10, 80),
-    # thread-per-chain at d = 16 (per-group coins), and the split path's REMOTE / REMOTE_SUM launches (windows > 32 steps)
+    # thread-per-chain at d = 16 (per-group coins), and windows > 32 steps (job-wide coin: chunks of up to 32 steps)
     "rosen16_groups_ref": ("rosenbrock1", None, 16, 512, 8, 0.5, 8, 150, 100, 0),
     "rosen16_groups_sum": ("rosenbrock1", None, 16, 512, 8, 0.5, 8, 150, 100, 1),
     "rosen2_sync40_ref": ("rosenbrock1", None, 2, 4096, 32, 0.5, 0, 150, 200, 0, 40),

@@ -141,25 +141,28 @@ _L = [
 ]
 CASES = [_legacy(i, *c) for i, c in enumerate(_L)]
 
-# Thread-per-chain kernels in all six phases.  A window longer than 32 steps under the job-wide coin runs as separate
-# LOCAL / REMOTE(_SUM) launches (mcgpu_sample's split path): sync 40, 160 main steps after the sync (1 + lag) local lead-in.
+# Thread-per-chain kernels in all their phases.  A window longer than 32 steps under the job-wide coin runs as chunks of at
+# most 32 steps (the width of the plan mask), each one LOCAL or MIXED(_SUM) launch: sync 40 (chunks of 32 + 8), 160 main
+# steps after the sync (1 + lag) local lead-in.
 for _lik, _d, _N, _par in [("gaussian", 2, 96, [1.0, -1.0, 0.5, 2.0]), ("gaussmix", 2, 96, "gmix2"), ("gaussmix", 4, 80, "gmix4")]:
     _k = {"gaussian": GA, "gaussmix": GM}[_lik]
     _n = "%s%d" % (_lik, _d)
     CASES += [
-        _case(_n + "-split-ref", _lik, _d, _N, _par, 8, 0.7, 0, 0, 0, 40, 1, 160, steps(_k, _d, B, L_, R_)),
-        _case(_n + "-split-sum-lag1", _lik, _d, _N, _par, 8, 0.7, 0, 1, 1, 40, 1, 160, steps(_k, _d, B, L_, RS)),
+        _case(_n + "-sync40-ref", _lik, _d, _N, _par, 8, 0.7, 0, 0, 0, 40, 1, 160, steps(_k, _d, B, L_, M_)),
+        _case(_n + "-sync40-sum-lag1", _lik, _d, _N, _par, 8, 0.7, 0, 1, 1, 40, 1, 160, steps(_k, _d, B, L_, MS)),
         _case(_n + "-groups-ref", _lik, _d, _N, _par, 8, 0.7, 8, 0, 0, 10, 1, 60, steps(_k, _d, B, M_)),
         _case(_n + "-groups-sum", _lik, _d, _N, _par, 8, 0.7, 8, 1, 0, 10, 1, 60, steps(_k, _d, B, MS)),
     ]
-# the split path of the other thread-per-chain likelihoods
+# the same windows for the other thread-per-chain likelihoods, and sync 70: chunks of 32 + 32 + 6 steps, so a middle chunk
+# that neither starts nor ends its window, with thin 3 putting the chunks' first steps off the kept rows (t0 = 32, 64)
 CASES += [
-    _case("rosenbrock12-split-ref", "rosenbrock1", 2, 128, None, 8, 0.7, 0, 0, 0, 40, 1, 160, steps(R1, 2, B, L_, R_)),
-    _case("rosenbrock12-split-sum", "rosenbrock1", 2, 128, None, 8, 0.7, 0, 1, 0, 40, 1, 160, steps(R1, 2, B, L_, RS)),
-    _case("rosenbrock14-split-ref", "rosenbrock1", 4, 96, None, 8, 0.7, 0, 0, 0, 40, 1, 160, steps(R1, 4, B, L_, R_)),
-    _case("rosenbrock14-split-sum-lag1", "rosenbrock1", 4, 96, None, 8, 0.7, 0, 1, 1, 40, 1, 160, steps(R1, 4, B, L_, RS)),
-    _case("dualgaussian2-split-ref", "dualgaussian", 2, 128, [5.0], 8, 0.7, 0, 0, 0, 40, 1, 160, steps(DG, 2, B, L_, R_)),
-    _case("dualgaussian2-split-sum", "dualgaussian", 2, 128, [5.0], 8, 0.7, 0, 1, 0, 40, 1, 160, steps(DG, 2, B, L_, RS)),
+    _case("rosenbrock12-sync40-ref", "rosenbrock1", 2, 128, None, 8, 0.7, 0, 0, 0, 40, 1, 160, steps(R1, 2, B, L_, M_)),
+    _case("rosenbrock12-sync40-sum", "rosenbrock1", 2, 128, None, 8, 0.7, 0, 1, 0, 40, 1, 160, steps(R1, 2, B, L_, MS)),
+    _case("rosenbrock14-sync40-ref", "rosenbrock1", 4, 96, None, 8, 0.7, 0, 0, 0, 40, 1, 160, steps(R1, 4, B, L_, M_)),
+    _case("rosenbrock14-sync40-sum-lag1", "rosenbrock1", 4, 96, None, 8, 0.7, 0, 1, 1, 40, 1, 160, steps(R1, 4, B, L_, MS)),
+    _case("dualgaussian2-sync40-ref", "dualgaussian", 2, 128, [5.0], 8, 0.7, 0, 0, 0, 40, 1, 160, steps(DG, 2, B, L_, M_)),
+    _case("dualgaussian2-sync40-sum", "dualgaussian", 2, 128, [5.0], 8, 0.7, 0, 1, 0, 40, 1, 160, steps(DG, 2, B, L_, MS)),
+    _case("rosenbrock12-sync70-thin3", "rosenbrock1", 2, 200, None, 10, 0.6, 0, 0, 0, 70, 3, 210, steps(R1, 2, B, L_, M_)),
 ]
 # thread-per-chain kernels at d >= 8: only per-group coins launch them (the job-wide coin takes the wide kernels)
 for _lik, _d, _par in [("rosenbrock1", 8, None), ("rosenbrock1", 16, "rosen16"), ("gaussmix", 8, "gmix8"), ("gaussmix", 16, "gmix16w")]:

@@ -64,7 +64,7 @@ def _assert_same(a, b):
 
 
 @pytest.mark.parametrize("d,N,cg,mode,lag", [
-    (2, 1000, 0, 0, 0),           # ragged N, job-wide coin: lean local / remote kernels
+    (2, 1000, 0, 0, 0),           # ragged N, job-wide coin: lean local / planned mixed kernels
     (2, 1000, 4, 1, 1),           # per-group coins, sum-mixture proposal, lagged pool
     (2, 256, 0, 1, 0),
     (2, 256, 4, 0, 1),

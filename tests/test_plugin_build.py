@@ -15,10 +15,10 @@ CUOBJDUMP = os.path.join(os.path.dirname(os.environ.get("NVCC", "/usr/local/cuda
 LOGISTIC = os.path.join(ROOT, "examples", "likelihoods", "logistic.cuh")
 ROSEN = os.path.join(ROOT, "tests", "plugins", "rosen1_restated.cuh")
 
-# what mcgpu_api.cu (plugin_kernel_name) looks up, pinned: mh_steps_kernel<101, d, RNG_PHILOX, phase> for the six
-# phases, init_loglik_kernel<101, d> and the batched evaluation
+# what mcgpu_api.cu (plugin_kernel_name) looks up, pinned: mh_steps_kernel<101, d, RNG_PHILOX, phase> for PH_BURN = 0,
+# PH_MIXED = 1, PH_LOCAL = 2 and PH_MIXED_SUM = 4, init_loglik_kernel<101, d> and the batched evaluation
 def _names(d):
-    steps = ["_ZN5mcgpu4fast15mh_steps_kernelILi101ELi%dELi0ELi%dEEEvNS_10StepParamsE" % (d, ph) for ph in range(6)]
+    steps = ["_ZN5mcgpu4fast15mh_steps_kernelILi101ELi%dELi0ELi%dEEEvNS_10StepParamsE" % (d, ph) for ph in (0, 1, 2, 4)]
     return steps + ["_ZN5mcgpu4fast18init_loglik_kernelILi101ELi%dEEEvNS_10StepParamsE" % d, "mcgpu_plugin_loglik"]
 
 
@@ -26,9 +26,7 @@ NAMES_D6 = [
     "_ZN5mcgpu4fast15mh_steps_kernelILi101ELi6ELi0ELi0EEEvNS_10StepParamsE",
     "_ZN5mcgpu4fast15mh_steps_kernelILi101ELi6ELi0ELi1EEEvNS_10StepParamsE",
     "_ZN5mcgpu4fast15mh_steps_kernelILi101ELi6ELi0ELi2EEEvNS_10StepParamsE",
-    "_ZN5mcgpu4fast15mh_steps_kernelILi101ELi6ELi0ELi3EEEvNS_10StepParamsE",
     "_ZN5mcgpu4fast15mh_steps_kernelILi101ELi6ELi0ELi4EEEvNS_10StepParamsE",
-    "_ZN5mcgpu4fast15mh_steps_kernelILi101ELi6ELi0ELi5EEEvNS_10StepParamsE",
     "_ZN5mcgpu4fast18init_loglik_kernelILi101ELi6EEEvNS_10StepParamsE",
     "mcgpu_plugin_loglik",
 ]
@@ -72,7 +70,7 @@ def test_plugin_step_kernels_do_not_spill(built):
             continue
         props = re.findall(r"Function properties for (\S+)\n\s*(\d+) bytes stack frame, (\d+) bytes spill stores, (\d+) bytes spill loads", log)
         steps = [p for p in props if "mh_steps_kernelILi101" in p[0]]
-        assert len(steps) == 6, (d, len(steps))
+        assert len(steps) == 4, (d, len(steps))
         for name, _, st, ld in steps:
             assert st == "0" and ld == "0", (d, name, st, ld)
 
