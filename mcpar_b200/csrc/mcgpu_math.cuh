@@ -47,6 +47,15 @@ MCGPU_HD double mc_make(int hi, int lo) {
 #endif
 }
 
+// (float)u32_mid(w) = fp32 rounding of (w + 1/2) 2^-32, without the fp64 pipe.  The top 24 bits of w and
+// (low 8 bits + 1/2) are both exact in fp32, and so are their products with 2^-32, so the one rounding of
+// the final sum is the rounding of (w + 1/2) 2^-32 itself, with or without FMA contraction.  Equal for all
+// 2^32 words: tests/test_u32_mid.py.
+MCGPU_HD float u32_mid_f32(uint32_t w) {
+  const float lo = (float)(w & 0xffu) * 2.3283064365386963e-10f + 1.1641532182693481e-10f;   // (w mod 2^8 + 1/2) 2^-32
+  return (float)(w & 0xffffff00u) * 2.3283064365386963e-10f + lo;
+}
+
 #define MCGPU_MAGIC 6755399441055744.0      /* 1.5 * 2^52: adding it leaves rint(x) in the low word */
 
 // Scalar coefficients live in CONSTANT memory on the device so that DFMA takes them as

@@ -299,7 +299,8 @@ __device__ __forceinline__ float cos_approx(float x) { float y; asm("cos.approx.
 //   <= 1.7e-6 min(1/r~, 770) + 2.4e-6 r~.
 __device__ __forceinline__ float normal_pair_f32(uint32_t wa, uint32_t wb, float &z0, float &z1, float &lg)
 {
-  const float v = ((float)wa + 1.0f) * 2.3283064365386963e-10f;                 // (0, 1]
+  // ((float)wa + 1) 2^-32 in one FFMA: scaling by 2^-32 is exact here, so the single rounding is that of the sum
+  const float v = fmaf((float)wa, 2.3283064365386963e-10f, 2.3283064365386963e-10f);   // (0, 1]
   lg = lg2_approx(v);                                                           // = -(z0^2 + z1^2)/2 * log2(e), in [-32, 0]
   const float L = -1.3862943611198906f * lg;
   const float rs = fminf(rsqrt_approx(L), 770.0f);                              // 1/r, capped at 1/1.3e-3 (also L = 0: inf)
@@ -309,13 +310,38 @@ __device__ __forceinline__ float normal_pair_f32(uint32_t wa, uint32_t wb, float
   return fmaf(2.4e-6f, r, 1.7e-6f * rs);
 }
 
+// The fp32 pool copy sPf (stage_pool) holds the slots in pairs: sPf[(s / 2) D + i] = (g mu_si, g mu_s'i, g_si, g_s'i)
+// for the even slot s and s' = s + 1 (the pool is padded to a multiple of 8 slots), so one FFMA2 evaluates a
+// parameter for both slots of a pair.  Each lane of FFMA2 is the same IEEE round-to-nearest fma as fmaf, so
+// every value below is bit for bit that of the slot-by-slot scalar loop.
+// Returns acc_s - sum_i (g mu_si - g_si x_i)^2 for the pair (s, s + 1), s even, summed over i = 0, 1, ... in
+// order; xx[i] = (x_i, x_i).
+template <int D>
+__device__ __forceinline__ float2 pool_pair(const float4 *sPf, int s, const float2 (&xx)[D], float2 acc)
+{
+#pragma unroll
+  for (int i = 0; i < D; ++i) {
+    const float4 f = sPf[(s >> 1) * D + i];
+    const float2 y = __ffma2_rn(make_float2(-f.z, -f.w), xx[i], make_float2(f.x, f.y));   // g (mu - x)
+    acc = __ffma2_rn(make_float2(-y.x, -y.y), y, acc);
+  }
+  return acc;
+}
+
+// (g mu_ci, g_ci) of one slot c of the paired layout above
+__device__ __forceinline__ float2 pool_slot(const float4 *sPf, int D, int c, int i)
+{
+  const float *f = reinterpret_cast<const float *>(sPf + (c >> 1) * D + i) + (c & 1);
+  return make_float2(f[0], f[2]);
+}
+
 // One candidate of the remote rejection loop (genRemote, mcpar.cc:331-409), decision only: draw the
 // component c, the uniform u and the normals z from the candidate's Philox blocks, form
 // x' = mu_c + sigma_c z and decide  u < max_s Q_s(x') / sum_s Q_s(x')  over the pool.  Rejected candidates
 // leave no trace and the accepted one is re-materialised in fp64 by its chain afterwards, so everything
-// here runs in fp32 on an fp32 copy of the pool -- sPf = (g mu, g) with g = sqrt(log2(e)/(2 sigma^2)), sSf = (sigma, mu),
-// padded to a multiple of 8 slots whose Q is 0; SFU log2/sqrt/sin/cos/exp2; chunks of 8 slots for ILP with
-// one rescale per chunk -- under a rigorous bound on the relative error of
+// here runs in fp32 on an fp32 copy of the pool -- sPf = (g mu, g) with g = sqrt(log2(e)/(2 sigma^2)) in slot pairs
+// (pool_pair), sSf = (sigma, mu), padded to a multiple of 8 slots whose Q is 0; SFU log2/sqrt/sin/cos/exp2; chunks of
+// 8 slots for ILP with one rescale per chunk -- under a rigorous bound on the relative error of
 //     R = sum_s exp(a_s - max a),   a_s = -sum_i (mu_si - x'_i)^2 / (2 sigma_si^2);
 // when the bound does not settle u the candidate is redone exactly in fp64 (remote_exact).
 // Error bound.  mu_s - x' (formed as (g mu - g x') / g) is off by at most delta = zerr sigma_c,max (normals,
@@ -327,17 +353,23 @@ __device__ __forceinline__ float normal_pair_f32(uint32_t wa, uint32_t wb, float
 // < 1e-6 M.  eps below covers all of it with margin.  theta >= 2e-3 (components far tighter than others or
 // than their distance from the origin: e.g. the first window, where sigma ~ 1e-7) goes to the exact test.
 // tests/test_gpu_audit.py checks the decisions against an all-fp64 run of the same kernels.
+// The launch-uniform inputs come from the caller, once per remote step: mu_max, isig_max (s_scal), eps0 =
+// (1.01e-4 + 1e-5 D) + 2e-5 M (remote_eps0), Mpad, and bounded = !p.exact_tests.
+template <int D>
+__device__ __forceinline__ float remote_eps0(int M) { return fmaf(2.0e-5f, (float)M, 1.01e-4f + 1.0e-5f * (float)D); }
+
 template <int D, bool RK>
 __device__ __forceinline__ bool remote_candidate(uint32_t tlo, uint32_t thi, uint32_t step, uint32_t slot, const StepParams &p,
-                                                 const float2 *sPf, const float2 *sSf, const double2 *sPmh, const double *sPs,
-                                                 float mu_max, float isig_max, const MathTables &T, unsigned int *s_fallback)
+                                                 const float4 *sPf, const float2 *sSf, const double2 *sPmh, const double *sPs,
+                                                 float mu_max, float isig_max, float eps0, int Mpad, bool bounded,
+                                                 const MathTables &T, unsigned int *s_fallback)
 {
   constexpr int CH = 8;
   constexpr int NP = (D + 1) / 2;
-  const int M = p.pool_m, Mpad = (M + CH - 1) & ~(CH - 1);
+  const int M = p.pool_m;
   Words blk = philox_d<D, RK>(tlo, thi, step, slot, p);
   const int c = (int)__umulhi(blk.w0, (uint32_t)M);                 // viRngUniform(0, tchains), mcpar.cc:337
-  const double u = u32_mid(blk.w1);                                 // vsRngUniform, mcpar.cc:401
+  const uint32_t uw = blk.w1;                                       // vsRngUniform, mcpar.cc:401: u = u32_mid(uw)
   float xf[D], xabs = 0.0f, sgmax = 0.0f, zerr = 0.0f, ref = 0.0f;
 #pragma unroll
   for (int q = 0; q < NP; ++q) {                                    // pair q = words (2+2q, 3+2q) of the candidate's stream
@@ -357,10 +389,12 @@ __device__ __forceinline__ bool remote_candidate(uint32_t tlo, uint32_t thi, uin
       xabs = fmaxf(xabs, fabsf(xf[i])); sgmax = fmaxf(sgmax, sm.x);
     }
   }
-  const float theta = (1.9e-7f * (mu_max + xabs) + zerr * sgmax) * isig_max;
+  float2 xx[D];
+#pragma unroll
+  for (int i = 0; i < D; ++i) xx[i] = make_float2(xf[i], xf[i]);
+  const float theta = fmaf(1.9e-7f, mu_max + xabs, zerr * sgmax) * isig_max;
   // the comparison itself runs in fp32 as well: u rounded to fp32 and three fp32 roundings add < 3e-7 to eps
-  const float epsf = (1.01e-4f + 1.0e-5f * (float)D) + 2.0e-5f * (float)M + theta * (21.3f * sqrtf((float)D));
-  const double eps = (double)epsf;
+  const float epsf = fmaf(theta, 21.3f * sqrtf((float)D), eps0);
   if constexpr (D <= 4) {
     // Exponents are taken relative to the picked component's own a_c = log2 v (>= -32 per normal pair), which
     // the Box-Muller step already has: 2^(a_s - a_c) <= 2^64 cannot overflow, so the sum needs no running
@@ -369,42 +403,36 @@ __device__ __forceinline__ bool remote_candidate(uint32_t tlo, uint32_t thi, uin
     // the candidate is rejected as soon as u S (1 - eps) >= 2^(-a_c), without the rest of the pool (at the
     // plateau max/sum ~ 1/M, so most candidates leave after the first chunks; the FPEPS offsets of
     // mcpar.cc:357-358 only lower the ratio further).
-    const bool fastok = theta < 2.0e-3f && !p.exact_tests;
-    const float uf_lo = (float)u * (1.0f - epsf) * (1.0f - 2.0e-7f), ebound = ex2_approx(-ref) * (1.0f + 1.0e-6f);
+    const bool fastok = theta < 2.0e-3f && bounded;
+    const float uf = u32_mid_f32(uw);                                // (float)u
+    const float uf_lo = uf * (1.0f - epsf) * (1.0f - 2.0e-7f), ebound = ex2_approx(-ref) * (1.0f + 1.0e-6f);
+    const float2 acc0 = make_float2(-ref, -ref);
     float mr = -INFINITY, S = 0.0f;                    // max_s and sum_s of 2^(a_s - a_c)
-    for (int s0 = 0; s0 < Mpad; s0 += CH) {
-      if (fastok && uf_lo * S >= ebound) return false;
+    for (int s0 = 0; s0 < Mpad;) {                     // (before the first chunk S = 0 and ebound >= 1: no test)
 #pragma unroll
-      for (int q = 0; q < CH; ++q) {
-        float acc = -ref;
-        if constexpr (D == 2) {                        // one 16-byte shared-memory load per slot (sPf is 16-byte aligned)
-          const float4 f = reinterpret_cast<const float4 *>(sPf)[s0 + q];
-          const float y0 = fmaf(-f.y, xf[0], f.x), y1 = fmaf(-f.w, xf[1], f.z);   // g (mu - x'): two FFMA per dimension
-          acc = fmaf(-y0, y0, acc); acc = fmaf(-y1, y1, acc);
-        } else {
-#pragma unroll
-          for (int i = 0; i < D; ++i) { const float2 f = sPf[(s0 + q) * D + i]; const float y = fmaf(-f.y, xf[i], f.x); acc = fmaf(-y, y, acc); }
-        }
-        mr = fmaxf(mr, acc);
-        S += ex2_approx(acc);
+      for (int q = 0; q < CH; q += 2) {
+        const float2 acc = pool_pair<D>(sPf, s0 + q, xx, acc0);
+        mr = fmaxf(mr, acc.x); S += ex2_approx(acc.x);
+        mr = fmaxf(mr, acc.y); S += ex2_approx(acc.y);
       }
+      s0 += CH;
+      if (s0 < Mpad && fastok && uf_lo * S >= ebound) return false;
     }
     if (mr + ref > -14.0f && fastok) {                 // max a > -9.7: then FPEPS/qmax < 2e-10 (mcpar.cc:357-358 offsets)
-      const float uf = (float)u, E = ex2_approx(mr);                // R = S / E
+      const float E = ex2_approx(mr);                               // R = S / E
       if (uf * fmaf(S, 1.0f + epsf, 3.0e-10f * E) < E) return true;  // u < r_lo
       if (uf * (S * (1.0f - epsf)) >= E) return false;               // u >= r_hi
     }
   } else {
+    const double u = u32_mid(uw), eps = (double)epsf;
     float m = -INFINITY;                               // running max of a_s * log2(e)
     float S = 0.0f;                                    // sum_s 2^(a_s - m)
     for (int s0 = 0; s0 < Mpad; s0 += CH) {
       float a[CH];
 #pragma unroll
-      for (int q = 0; q < CH; ++q) {
-        float acc = 0.0f;
-#pragma unroll
-        for (int i = 0; i < D; ++i) { const float2 f = sPf[(s0 + q) * D + i]; const float y = fmaf(-f.y, xf[i], f.x); acc = fmaf(-y, y, acc); }
-        a[q] = acc;
+      for (int q = 0; q < CH; q += 2) {
+        const float2 acc = pool_pair<D>(sPf, s0 + q, xx, make_float2(0.0f, 0.0f));
+        a[q] = acc.x; a[q + 1] = acc.y;
       }
       float mc = a[0];
 #pragma unroll
@@ -417,7 +445,7 @@ __device__ __forceinline__ bool remote_candidate(uint32_t tlo, uint32_t thi, uin
       S = gt ? fmaf(S, e, sc) : fmaf(sc, e, S);
       m = gt ? mc : m;
     }
-    if (m > -14.0f && theta < 2.0e-3f && !p.exact_tests) {
+    if (m > -14.0f && theta < 2.0e-3f && bounded) {
       const double Sd = (double)S;
       if (u * (Sd * (1.0 + eps) + 3.0e-10) < 1.0) return true;      // u < r_lo
       if (u * (Sd * (1.0 - eps)) >= 1.0) return false;              // u >= r_hi
@@ -490,41 +518,30 @@ __device__ __noinline__ double summix_lse_exact(const PointD<D> x, const double2
 
 template <int D>
 __device__ __forceinline__ bool summix_bounds(const double (&xo)[D], const double (&xn)[D], int c, int M,
-                                              const float2 *sPf, const float *sNb, const float *s_scal,
+                                              const float4 *sPf, const float *sNb, const float *s_scal,
                                               float &cf_lo, float &cf_hi)
 {
   constexpr int CH = 8;
   const int Mpad = (M + CH - 1) & ~(CH - 1);
   float xof[D], xnf[D], xabs_o = 0.0f, xabs_n = 0.0f;
+  float2 xxo[D], xxn[D];
 #pragma unroll
   for (int i = 0; i < D; ++i) {
     xof[i] = (float)xo[i]; xnf[i] = (float)xn[i];
     xabs_o = fmaxf(xabs_o, fabsf(xof[i])); xabs_n = fmaxf(xabs_n, fabsf(xnf[i]));
+    xxo[i] = make_float2(xof[i], xof[i]); xxn[i] = make_float2(xnf[i], xnf[i]);
   }
   float ref = sNb[c];                                  // A_c(x'): the level both sums are taken relative to
 #pragma unroll
-  for (int i = 0; i < D; ++i) { const float2 f = sPf[c * D + i]; const float y = fmaf(-f.y, xnf[i], f.x); ref = fmaf(-y, y, ref); }
+  for (int i = 0; i < D; ++i) { const float2 f = pool_slot(sPf, D, c, i); const float y = fmaf(-f.y, xnf[i], f.x); ref = fmaf(-y, y, ref); }
   float Sn[4] = {0.0f, 0.0f, 0.0f, 0.0f}, So[4] = {0.0f, 0.0f, 0.0f, 0.0f};
   for (int s0 = 0; s0 < Mpad; s0 += CH) {
 #pragma unroll
-    for (int q = 0; q < CH; ++q) {
-      const float base = sNb[s0 + q] - ref;
-      float an = base, ao = base;
-      if constexpr (D == 2) {                          // one 16-byte shared-memory load per slot
-        const float4 f = reinterpret_cast<const float4 *>(sPf)[s0 + q];
-        const float yn0 = fmaf(-f.y, xnf[0], f.x), yn1 = fmaf(-f.w, xnf[1], f.z);
-        const float yo0 = fmaf(-f.y, xof[0], f.x), yo1 = fmaf(-f.w, xof[1], f.z);
-        an = fmaf(-yn0, yn0, an); an = fmaf(-yn1, yn1, an);
-        ao = fmaf(-yo0, yo0, ao); ao = fmaf(-yo1, yo1, ao);
-      } else {
-#pragma unroll
-        for (int i = 0; i < D; ++i) {
-          const float2 f = sPf[(s0 + q) * D + i];
-          const float yn = fmaf(-f.y, xnf[i], f.x), yo = fmaf(-f.y, xof[i], f.x);
-          an = fmaf(-yn, yn, an); ao = fmaf(-yo, yo, ao);
-        }
-      }
-      Sn[q & 3] += ex2_approx(an); So[q & 3] += ex2_approx(ao);
+    for (int q = 0; q < CH; q += 2) {                  // a slot pair: both points, both slots, in packed fp32 (pool_pair)
+      const float2 base = make_float2(sNb[s0 + q] - ref, sNb[s0 + q + 1] - ref);
+      const float2 an = pool_pair<D>(sPf, s0 + q, xxn, base), ao = pool_pair<D>(sPf, s0 + q, xxo, base);
+      Sn[q & 3] += ex2_approx(an.x); So[q & 3] += ex2_approx(ao.x);
+      Sn[(q + 1) & 3] += ex2_approx(an.y); So[(q + 1) & 3] += ex2_approx(ao.y);
     }
   }
   const float sn = (Sn[0] + Sn[1]) + (Sn[2] + Sn[3]), so = (So[0] + So[1]) + (So[2] + So[3]);
@@ -564,7 +581,7 @@ __device__ __forceinline__ int accept_test_bounded(double u, double delta, float
 template <int D>
 __device__ __noinline__ bool stage_pool(const double *pool_cur, int pool_m, const unsigned long long *arrivals,
                                         unsigned long long wait_target, int *xflag, unsigned long long *xstat,
-                                        double2 *sPmh, double *sPs, float2 *sPf, float2 *sSf, double *sPn, float *sNb,
+                                        double2 *sPmh, double *sPs, float4 *sPf, float2 *sSf, double *sPn, float *sNb,
                                         float *s_scal, int Mpad, const MathTables T)
 {
   if (wait_target) wait_arrivals(arrivals, wait_target, xflag, xstat);
@@ -574,15 +591,16 @@ __device__ __noinline__ bool stage_pool(const double *pool_cur, int pool_m, cons
   if (s_scal[3] != 0.0f) return false;
   float mumax = 0.0f, isig = 0.0f;
   for (int i = threadIdx.x; i < Mpad * D; i += blockDim.x) {
+    float *pf = reinterpret_cast<float *>(sPf + (i / D >> 1) * D + i % D) + (i / D & 1);   // slot pairs (pool_pair)
     if (i < pool_m * D) {
       const double m = pool_cur[i * 2], s2 = pool_cur[i * 2 + 1];
       const double h = -0.5 / s2, sd = sqrt(s2);       // sigma = sqrt(sig^2), mcpar.cc:346
       sPmh[i] = make_double2(m, h); sPs[i] = sd;
       const double g = sqrt(-h * 1.4426950408889634);   // sqrt(log2(e) / (2 sigma^2)): a_s log2(e) = -sum_i (g mu - g x)^2
-      sPf[i] = make_float2((float)(g * m), (float)g); sSf[i] = make_float2((float)sd, (float)m);
+      pf[0] = (float)(g * m); pf[2] = (float)g; sSf[i] = make_float2((float)sd, (float)m);
       mumax = fmaxf(mumax, __double2float_ru(fabs(m))); isig = fmaxf(isig, __double2float_ru(1.0 / sd));
     } else {                                           // padding: (mu - x)^2 overflows / is huge, a = -inf, Q = 0
-      sPmh[i] = make_double2(1.0e300, -1.0); sPf[i] = make_float2(1.0e18f, 0.0f); sSf[i] = make_float2(0.0f, 0.0f);
+      sPmh[i] = make_double2(1.0e300, -1.0); pf[0] = 1.0e18f; pf[2] = 0.0f; sSf[i] = make_float2(0.0f, 0.0f);
     }
   }
   // normalisation of the components (remote mode 1): n_s = -1/2 sum_i log sig2_si, and nb_s = n_s log2(e) in fp32
@@ -623,8 +641,8 @@ mh_steps_kernel(const StepParams p)
   double2 *sPmh = reinterpret_cast<double2*>(sW + ((p.nsteps + 1) & ~1));     // (mu, -1/(2 sig^2)) pairs, 16-byte aligned
   const int Mpad = (p.pool_m + 7) & ~7;
   double *sPs = reinterpret_cast<double*>(sPmh + Mpad * D);
-  float2 *sPf = reinterpret_cast<float2*>(sPs + Mpad * D);                    // fp32 copy: (g mu, g), g = sqrt(log2(e)/(2 sig^2))
-  float2 *sSf = sPf + Mpad * D;                                               //            (sigma, mu)
+  float4 *sPf = reinterpret_cast<float4*>(sPs + Mpad * D);                    // fp32 copy: (g mu, g), g = sqrt(log2(e)/(2 sig^2)), slot pairs
+  float2 *sSf = reinterpret_cast<float2*>(sPf + Mpad / 2 * D);                //            (sigma, mu)
   double *sPn = reinterpret_cast<double*>(sSf + Mpad * D);                    // n_s = -1/2 sum_i log sig2_si (remote mode 1)
   float *sNb = reinterpret_cast<float*>(sPn + Mpad);                          // n_s log2(e)
   __shared__ float s_scal[4];                           // pool-wide max |mu|, max 1/sigma, max |nb| (error bounds of the fp32 pool tests)
@@ -722,35 +740,38 @@ mh_steps_kernel(const StepParams p)
       const unsigned rm0 = rm;                          // the chains of this warp that take a remote step
       if constexpr (CAN_REMOTE && !SUMMIX) {
         bool pending = remote && live;
-        uint32_t it_next = 0;
-        if (rm) s_itacc[threadIdx.x] = 0u;
+        uint32_t it_next = 0;                           // this chain's next candidate; once it is done, its accepted one
+        // launch-uniform inputs of remote_candidate, read once per remote step instead of once per candidate
+        const float mu_max = s_scal[0], isig_max = s_scal[1], eps0 = remote_eps0<D>(p.pool_m);
+        const bool bounded = !p.exact_tests;
+        // A lane only ever serves a pending chain, and pending lanes are live, so the chain of lane tgt is
+        // chain0 + (j - lane) + tgt: its Philox counter needs no shuffle.
+        const unsigned long long gwarp = (unsigned long long)(p.chain0 + (j - lane));
+        unsigned char *const rank = s_rank[threadIdx.x >> 5];
         while (rm) {
           // schedule 32 candidates over the unfinished chains
           const int n = __popc(rm);
           const int kk = (int)(((unsigned)lane * c_recip[n]) >> 16), r = lane - kk * n;   // lane / n, lane % n
           const int my_r = __popc(rm & ((1u << lane) - 1u));      // rank of this lane's chain among the unfinished
-          if (pending) s_rank[threadIdx.x >> 5][my_r] = (unsigned char)lane;
+          if (pending) rank[my_r] = (unsigned char)lane;
           __syncwarp();
-          const int tgt = s_rank[threadIdx.x >> 5][r];  // lane owning the r-th unfinished chain
+          const int tgt = rank[r];                      // lane owning the r-th unfinished chain
           __syncwarp();
           const uint32_t it = __shfl_sync(0xffffffffu, it_next, tgt) + (uint32_t)kk;
-          const uint32_t tlo = __shfl_sync(0xffffffffu, glo, tgt), thi = __shfl_sync(0xffffffffu, ghi, tgt);
-          const bool acc = remote_candidate<D, true>(tlo, thi, step, MCGPU_SLOT_REMOTE | (it << 6), p, sPf, sSf, sPmh, sPs,
-                                                           s_scal[0], s_scal[1], T, &s_stat[2]);
+          const unsigned long long gt = gwarp + (unsigned)tgt;
+          const bool acc = remote_candidate<D, true>((uint32_t)gt, (uint32_t)(gt >> 32), step, MCGPU_SLOT_REMOTE | (it << 6), p,
+                                                     sPf, sSf, sPmh, sPs, mu_max, isig_max, eps0, Mpad, bounded, T, &s_stat[2]);
           const unsigned accmask = __ballot_sync(0xffffffffu, acc);
           if (pending) {
-            const unsigned cm = c_stride_mask[n] << my_r;             // lanes my_r, my_r+n, ... served this chain
-            const unsigned hit = accmask & cm;
-            if (hit) {                                                // lowest lane = lowest iteration index
-              s_itacc[threadIdx.x] = it_next + (uint32_t)__popc(cm & ((1u << (__ffs(hit) - 1)) - 1u));
-              pending = false;
-            } else {
-              it_next += (uint32_t)__popc(cm);
-              if (it_next >= (1u << 24) - 64u) { s_itacc[threadIdx.x] = it_next; pending = false; }   // slot space exhausted (never in practice)
-            }
+            // lanes my_r, my_r+n, ... served this chain, in iteration order; the lowest accepting lane (if any)
+            // holds the first accepted candidate: advance past the candidates before it, or past all of them
+            const unsigned cm = c_stride_mask[n] << my_r, hit = accmask & cm;
+            it_next += (uint32_t)__popc(cm & ((hit & (0u - hit)) - 1u));
+            pending = !hit && it_next < (1u << 24) - 64u;              // or the slot space is exhausted (never in practice)
           }
           rm = __ballot_sync(0xffffffffu, pending);
         }
+        if (rm0) s_itacc[threadIdx.x] = it_next;
       }
       // Materialise the proposal in fp64, once per step and with one copy of the Philox + Box-Muller
       // code for both kinds: a local step draws its normals from the chain's local stream and
