@@ -25,7 +25,7 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-ccbin", "/u
 # engine loads only plugins whose stamp equals its own.
 STAMPED = ["include/mcgpu.h", "mcpar_b200/csrc/mcgpu_device.cuh", "mcpar_b200/csrc/mh_kernels.cuh",
            "mcpar_b200/csrc/mcgpu_math.cuh", "mcpar_b200/csrc/mcgpu_tables.h", "mcpar_b200/csrc/mh_plugin.cu",
-           "mcpar_b200/csrc/mh_wide.cuh"]
+           "mcpar_b200/csrc/mh_wide.cuh", "mcpar_b200/csrc/mcgpu_cellbound.cuh"]
 
 
 def kernel_stamp(root=ROOT):

@@ -67,6 +67,7 @@ struct mcgpu_engine {
   bool wide = false;
   double *factor_cm = nullptr; int *diag_d = nullptr;
   double *pprep = nullptr; int mpad = 0;
+  float4 *cell_tab = nullptr;              // d = 2, reference remote mode: the window's table of acceptance-ratio bounds
   double *gm_t = nullptr; int kpad = 0;
 
   // VERIFY extras
@@ -714,7 +715,7 @@ int mcgpu_destroy(mcgpu_engine *e)
   void *ptrs[] = {e->x, e->ly, e->mu, e->ps, e->factor, e->counts, e->xchg, e->xflag_d, e->peers_d, e->hist, e->overrun,
                   e->Zd, e->Ud, e->Id, e->ptrial, e->sig, e->mutrial, e->sigtrial, e->musig, e->snap[0], e->snap[1],
                   e->soff, e->cursors, e->irate_d, e->rstats, e->tr_accept, e->tr_remote, e->tr_trial_ly,
-                  e->tr_trial_p, e->tr_cfac, e->tr_iters, e->lik_dev, e->factor_cm, e->diag_d, e->pprep, e->gm_t, e->hist_f32,
+                  e->tr_trial_p, e->tr_cfac, e->tr_iters, e->lik_dev, e->factor_cm, e->diag_d, e->pprep, e->gm_t, e->hist_f32, e->cell_tab,
                   e->aux, e->lytrial_d, e->flags_d};
   for (void *p : ptrs) if (p) cudaFree(p);
   for (void *q : e->peer_opened) cudaIpcCloseMemHandle(q);
@@ -1107,9 +1108,20 @@ int mcgpu_sample(mcgpu_engine *e, int nsteps)
       p.hist = e->hist; p.hist_ring0 = e->hist ? (int)((e->t_main / e->cfg.thin) % e->hist_cap) : 0;
       // publish (mu, sigma^2) into the next pool only from the launch that ends the window
       double *const publish = ((e->t_main + n) % sync == 0) ? pool_next(e) : nullptr;
+      // reference remote mode at d = 2: the table of acceptance-ratio bounds over this window's pool, built right
+      // before the window's first launch that can take a remote step (it does not depend on the likelihood)
+      const bool use_tab = e->d == 2 && !e->wide && e->remote_mode == 0 && !p.exact_tests && !e->replay_local && e->cfg.pl < 1.0;
+      auto cell_table = [&]() -> int {
+        if (!e->cell_tab) CK(cudaMalloc((void**)&e->cell_tab, fast::cell_table_bytes()));
+        ++e->launches;
+        CK(fast::launch_cell_table(pool_cur(e), e->M, e->cell_tab, p.arrivals, p.wait_target, p.xflag, p.xstat, e->stream));
+        p.cell_tab = e->cell_tab;
+        return MCGPU_OK;
+      };
       if (e->cfg.coin_group > 0 || e->replay_local) {       // per-group coins: one mixed launch per window
         p.step0 = (uint32_t)(e->nburn_total + e->t_main); p.nsteps = n; p.t0 = (int)e->t_main;
         p.pool_next = publish;
+        if (use_tab && p.t0 + n > p.first_remote_t) { int rc = cell_table(); if (rc) return rc; }
         CK(launch_steps_any(e, PH_MIXED, p));
       } else {                                               // job-wide coin: the host cuts the window into segments
         // wide kernels read the pool as (mu, -1/2sig^2, sig), slot-fastest: prepared right before the window's
@@ -1146,6 +1158,7 @@ int mcgpu_sample(mcgpu_engine *e, int nsteps)
             for (int i = 0; i < len; ++i) if (is_remote(t + i)) mask |= 1u << i;
             p.plan_mask = mask; p.plan_valid = 1;
             phase = mask ? PH_MIXED : PH_LOCAL;
+            if (mask && use_tab && !p.cell_tab) { int rc = cell_table(); if (rc) return rc; }
           }
           p.step0 = (uint32_t)(e->nburn_total + t); p.nsteps = len; p.t0 = (int)t;
           p.hist_ring0 = e->hist ? (int)((t / e->cfg.thin) % e->hist_cap) : 0;

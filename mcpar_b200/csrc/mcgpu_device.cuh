@@ -12,6 +12,9 @@
 #define MCGPU_SLOT_REMOTE 0x40000000u
 #define MCGPU_MAX_D_REG 16           // thread-per-chain kernels keep the state in registers up to this d
 #define MCGPU_MAX_D 64
+#ifndef MCGPU_CELL_G
+#define MCGPU_CELL_G 64              // cells per axis of the d = 2 acceptance-ratio table (mcgpu_cellbound.cuh)
+#endif
 
 namespace mcgpu {
 
@@ -114,6 +117,10 @@ struct StepParams {
   const double *Z, *U; long long nz, nu; int *overrun;
   // likelihood parameters
   double lp[8]; const double *lik_dev; int lik_k;
+  // (last, so that the offsets of the fields above stay as they were)
+  // reference remote mode, d = 2: this window's table of acceptance-ratio bounds, or null.  cell_tab[0] = (origin x,
+  // origin y, 1 / cell width x, 1 / cell width y), then MCGPU_CELL_G^2 cells (R_lo, R_hi) as float2, row y major
+  const float4 *cell_tab;
 };
 
 // One launch worth of arguments for the wide (d >= 8, D/2 lanes per chain) kernels.

@@ -5,6 +5,7 @@
 #include "mh_kernels.cuh"
 #include "mh_wide.cuh"
 #include "mh_coop.cuh"
+#include "mcgpu_cellbound.cuh"
 namespace mcgpu { namespace fast {
 #include "mh_dispatch.inl"
 
@@ -98,9 +99,75 @@ cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, double2
   return cudaGetLastError();
 }
 
+// ---- reference remote mode, d = 2: the window's table of acceptance-ratio bounds (mcgpu_cellbound.cuh) ----------
+struct CellRedWarp {
+  __device__ double max(double v) const { for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o)); return v; }
+  __device__ double sum(double v) const { for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o); return v; }
+  __device__ int min(int v) const { for (int o = 16; o > 0; o >>= 1) v = ::min(v, __shfl_xor_sync(0xffffffffu, v, o)); return v; }
+};
+
+// One warp per cell.  The grid spans, per axis, min_s (mu_s - 5 sigma_s) .. max_s (mu_s + 5 sigma_s): the fp32 Box-Muller
+// normals stay below 6.66, so the few candidates beyond it fall back to the pool loop.  Every warp derives the grid
+// from the pool itself (exact min / max reductions: all warps agree); a pool with a non-finite or non-positive entry
+// gets a NaN header, which no candidate passes.  With a peer-to-peer exchange the CTAs first wait for the arrivals,
+// as pool_prep_kernel does.
+static __global__ void __launch_bounds__(128) cell_table_kernel(const double *pool, int M, float4 *tab,
+                                                                 const unsigned long long *arrivals, unsigned long long wait_target,
+                                                                 int *xflag, unsigned long long *xstat)
+{
+  if (wait_target) { wait_arrivals(arrivals, wait_target, xflag, xstat); __syncthreads(); }
+  constexpr int G = MCGPU_CELL_G;
+  const int lane = threadIdx.x & 31, cell = blockIdx.x * 4 + (threadIdx.x >> 5);
+  const CellRedWarp red;
+  double lo[2] = {INFINITY, INFINITY}, hi[2] = {-INFINITY, -INFINITY}, bad = 0.0;
+  for (int s = lane; s < M; s += 32)
+    for (int i = 0; i < 2; ++i) {
+      const double m = pool[(s * 2 + i) * 2], sd = sqrt(pool[(s * 2 + i) * 2 + 1]);
+      if (!(sd > 0.0 && fabs(m) + 5.0 * sd <= 1.0e30)) bad = 1.0;
+      else { lo[i] = fmin(lo[i], m - 5.0 * sd); hi[i] = fmax(hi[i], m + 5.0 * sd); }
+    }
+  float o[2], inv[2];
+  bool ok = red.max(bad) == 0.0;
+  for (int i = 0; i < 2; ++i) {
+    const double l = -red.max(-lo[i]), h = red.max(hi[i]);
+    o[i] = __double2float_rd(l);
+    inv[i] = __double2float_rn((double)G / (h - (double)o[i]));
+    ok = ok && inv[i] > 0.0f && inv[i] < 1.0e30f;
+  }
+  if (!ok) { o[0] = o[1] = inv[0] = inv[1] = NAN; }
+  if (blockIdx.x == 0 && threadIdx.x == 0) tab[0] = make_float4(o[0], o[1], inv[0], inv[1]);
+  if (!ok || cell >= G * G) return;
+  const int gx = cell % G, gy = cell / G;
+  const double ix = 1.0 / (double)inv[0], iy = 1.0 / (double)inv[1];
+  double rlo, rhi;
+  cell_bounds2(pool, M, (double)o[0] + (gx + 0.5) * ix, (double)o[1] + (gy + 0.5) * iy,
+               (0.5 + 1.0 / 64.0) * ix * (1.0 + 1.0e-12), (0.5 + 1.0 / 64.0) * iy * (1.0 + 1.0e-12), lane, 32, red, rlo, rhi);
+  float flo, fhi;
+  cell_store_bounds(rlo, rhi, flo, fhi);
+  if (lane == 0) reinterpret_cast<float2 *>(tab + 1)[cell] = make_float2(flo, fhi);
+}
+
+size_t cell_table_bytes() { return sizeof(float4) + sizeof(float2) * MCGPU_CELL_G * MCGPU_CELL_G; }
+
+cudaError_t launch_cell_table(const double *pool, int M, float4 *tab, const unsigned long long *arrivals,
+                              unsigned long long wait_target, int *xflag, unsigned long long *xstat, cudaStream_t st)
+{
+  cell_table_kernel<<<MCGPU_CELL_G * MCGPU_CELL_G / 4, 128, 0, st>>>(pool, M, tab, arrivals, wait_target, xflag, xstat);
+  return cudaGetLastError();
+}
+
 cudaError_t launch_factor_prep(const double *rm, double *cm, int D, int *diag, cudaStream_t st)
 {
   factor_prep_kernel<<<1, 256, 0, st>>>(rm, cm, D, diag);
   return cudaGetLastError();
 }
 }}
+#ifdef MCGPU_CELL_COUNT
+// counting build: read and clear the table's counters (tools/cell_hits.py)
+extern "C" int mcgpu_cell_counts(unsigned long long out[4])
+{
+  if (cudaMemcpyFromSymbol(out, mcgpu::fast::mcgpu_cell_count, 4 * sizeof(unsigned long long)) != cudaSuccess) return 1;
+  const unsigned long long z[4] = {0, 0, 0, 0};
+  return cudaMemcpyToSymbol(mcgpu::fast::mcgpu_cell_count, z, sizeof z) != cudaSuccess;
+}
+#endif

@@ -355,6 +355,10 @@ __device__ __forceinline__ float2 pool_slot(const float4 *sPf, int D, int c, int
 // tests/test_gpu_audit.py checks the decisions against an all-fp64 run of the same kernels.
 // The launch-uniform inputs come from the caller, once per remote step: mu_max, isig_max (s_scal), eps0 =
 // (1.01e-4 + 1e-5 D) + 2e-5 M (remote_eps0), Mpad, and bounded = !p.exact_tests.
+#ifdef MCGPU_CELL_COUNT
+// counting build (tools/build_variant.py): table-decided candidates, rounds with a table miss, rounds
+__device__ unsigned long long mcgpu_cell_count[4];
+#endif
 template <int D>
 __device__ __forceinline__ float remote_eps0(int M) { return fmaf(2.0e-5f, (float)M, 1.01e-4f + 1.0e-5f * (float)D); }
 
@@ -392,7 +396,8 @@ __device__ __forceinline__ bool remote_candidate(uint32_t tlo, uint32_t thi, uin
   float2 xx[D];
 #pragma unroll
   for (int i = 0; i < D; ++i) xx[i] = make_float2(xf[i], xf[i]);
-  const float theta = fmaf(1.9e-7f, mu_max + xabs, zerr * sgmax) * isig_max;
+  const float dx = fmaf(1.9e-7f, mu_max + xabs, zerr * sgmax);    // bounds |x'_f32 - x'_fp64| per parameter
+  const float theta = dx * isig_max;
   // the comparison itself runs in fp32 as well: u rounded to fp32 and three fp32 roundings add < 3e-7 to eps
   const float epsf = fmaf(theta, 21.3f * sqrtf((float)D), eps0);
   if constexpr (D <= 4) {
@@ -406,6 +411,32 @@ __device__ __forceinline__ bool remote_candidate(uint32_t tlo, uint32_t thi, uin
     const bool fastok = theta < 2.0e-3f && bounded;
     const float uf = u32_mid_f32(uw);                                // (float)u
     const float uf_lo = uf * (1.0f - epsf) * (1.0f - 2.0e-7f), ebound = ex2_approx(-ref) * (1.0f + 1.0e-6f);
+    if constexpr (D == 2) {
+      // The window's table of rigorous bounds on R (mcgpu_cellbound.cuh): each cell was dilated by 1/64 of its width,
+      // which covers |x'_f32 - x'_fp64| < 1/128 of a width and the fp32 rounding of the cell index.  The fp64
+      // candidate that remote_exact would evaluate lies in the dilated cell, so the stored bounds settle u as that
+      // evaluation would; a candidate outside the grid or between the bounds runs the pool loop below.
+      const float4 *const tab = p.cell_tab;
+      if (tab != nullptr) {
+        const float4 hd = __ldg(tab);                  // (origin x, origin y, 1/width x, 1/width y); NaN: no valid table
+        const int gx = __float2int_rd((xf[0] - hd.x) * hd.z), gy = __float2int_rd((xf[1] - hd.y) * hd.w);
+        bool hit = false, dec = false;
+        if (dx * fmaxf(hd.z, hd.w) < 0.0078125f && (unsigned)gx < (unsigned)MCGPU_CELL_G && (unsigned)gy < (unsigned)MCGPU_CELL_G) {
+          const float2 b = __ldg(reinterpret_cast<const float2 *>(tab + 1) + gy * MCGPU_CELL_G + gx);
+          dec = uf < b.x;                              // u < R_lo
+          hit = dec || uf >= b.y;                      // or u >= R_hi
+        }
+#ifdef MCGPU_CELL_COUNT
+        const unsigned miss = __ballot_sync(0xffffffffu, !hit);
+        if ((threadIdx.x & 31) == 0) {
+          atomicAdd(&mcgpu_cell_count[0], (unsigned long long)(32 - __popc(miss)));
+          atomicAdd(&mcgpu_cell_count[1], miss ? 1ull : 0ull);
+          atomicAdd(&mcgpu_cell_count[2], 1ull);
+        }
+#endif
+        if (hit) return dec;
+      }
+    }
     const float2 acc0 = make_float2(-ref, -ref);
     float mr = -INFINITY, S = 0.0f;                    // max_s and sum_s of 2^(a_s - a_c)
     for (int s0 = 0; s0 < Mpad;) {                     // (before the first chunk S = 0 and ebound >= 1: no test)

@@ -12,6 +12,9 @@ cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, double2
                              const unsigned long long *arrivals, unsigned long long wait_target, int *xflag,
                              unsigned long long *xstat, cudaStream_t st);
 cudaError_t launch_factor_prep(const double *rm, double *cm, int D, int *diag, cudaStream_t st);
+size_t cell_table_bytes();       // the d = 2 table of acceptance-ratio bounds (StepParams::cell_tab)
+cudaError_t launch_cell_table(const double *pool, int M, float4 *tab, const unsigned long long *arrivals,
+                              unsigned long long wait_target, int *xflag, unsigned long long *xstat, cudaStream_t st);
 bool steps_supported(int lik, int d);
 size_t steps_smem_bytes(int d, int nsteps, int pool_m, bool with_pool);
 StepLaunch steps_launch(int d, long long C, int nsteps, int pool_m, int phase);   // the step kernels' launch rule (built-in likelihoods and plugins)
