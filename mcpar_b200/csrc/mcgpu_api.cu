@@ -182,17 +182,34 @@ double *pool_newest(const mcgpu_engine *e) { return e->pool[e->npub % pool_nbuf(
 double *pool_next(const mcgpu_engine *e) { return e->pool[(e->npub + 1) % pool_nbuf(e)]; }
 int arrivals_per_slot(const mcgpu_engine *e) { return e->wide ? e->d / 2 : 1; }   // the wide kernel's lanes arrive one by one
 
-// peer-to-peer exchange: where this launch publishes and what it waits for
-void fill_p2p(const mcgpu_engine *e, StepParams &p)
+// The exchange block of a main-phase launch: it publishes into `publish` (null: it does not publish); with a
+// peer-to-peer exchange also where those stores go and what the launch waits for
+void fill_exchange(const mcgpu_engine *e, ExchangeParams &x, double *publish)
 {
+  x.pool_next = publish; x.pool_stride = e->stride;
+  x.xstat = e->counts + 8;
   if (!e->p2p) return;
-  p.peers = e->peers_d; p.npeers = e->p2p_world;
-  p.next_off = (long long)(((e->npub + 1) % pool_nbuf(e)) * e->pool_bytes); p.arr_off = (long long)(NPOOL * e->pool_bytes);
-  p.arrivals = reinterpret_cast<const unsigned long long*>(e->xchg + NPOOL * e->pool_bytes);
+  x.peers = e->peers_d; x.npeers = e->p2p_world;
+  x.next_off = (long long)(((e->npub + 1) % pool_nbuf(e)) * e->pool_bytes); x.arr_off = (long long)(NPOOL * e->pool_bytes);
+  x.arrivals = reinterpret_cast<const unsigned long long*>(e->xchg + NPOOL * e->pool_bytes);
   const unsigned long long per_pub = (unsigned long long)e->M * arrivals_per_slot(e);
-  p.wait_target = per_pub * (unsigned long long)pool_read_index(e);     // readers: the publication this window reads
-  p.pub_wait_target = per_pub * (unsigned long long)e->npub;            // publishers: never more than one publication ahead
-  p.xflag = e->xflag_d;
+  x.wait_target = per_pub * (unsigned long long)pool_read_index(e);     // readers: the publication this window reads
+  x.pub_wait_target = per_pub * (unsigned long long)e->npub;            // publishers: never more than one publication ahead
+  x.xflag = e->xflag_d;
+}
+
+// The wide kernels' prepared pool, one allocation: (mu, -1/(2 sigma^2)) pairs [d][mpad], sigma [d][mpad] and n_s [mpad]
+// in fp64, then the fp32 copy: (g mu, g) pairs [d][mpad], n_s log2 e [mpad] and 4 scalars.  Returns the bytes to
+// allocate and, in *v, the views into e->pprep.
+size_t wide_pool(const mcgpu_engine *e, WidePool *v = nullptr)
+{
+  const size_t n = (size_t)e->d * e->mpad, m = (size_t)e->mpad;
+  if (v) {
+    float *f = reinterpret_cast<float *>(e->pprep + 3 * n + m);
+    v->pmh = reinterpret_cast<double2 *>(e->pprep); v->psd = e->pprep + 2 * n; v->pnb = e->pprep + 3 * n;
+    v->pf = reinterpret_cast<float2 *>(f); v->pnbf = f + 2 * n; v->pscal = v->pnbf + m;
+  }
+  return (3 * n + m) * 8 + (2 * n + m) * 4 + 16;
 }
 
 void fill_step_params(mcgpu_engine *e, StepParams &p)
@@ -206,7 +223,7 @@ void fill_step_params(mcgpu_engine *e, StepParams &p)
   p.sync = e->cfg.sync; p.coin_group = e->cfg.coin_group; p.pl = e->cfg.pl;
   p.first_remote_t = e->cfg.sync * (1 + e->lag);
   p.hist_cap = (int)std::max<long long>(e->hist_cap, 1);
-  p.pool_m = e->M; p.pool_stride = e->stride;
+  p.pool_m = e->M;
   p.thin = e->cfg.thin;
   static const int exact_tests = getenv("MCGPU_EXACT_TESTS") ? atoi(getenv("MCGPU_EXACT_TESTS")) : 0;
   p.exact_tests = exact_tests;
@@ -344,15 +361,11 @@ cudaError_t launch_steps_any(mcgpu_engine *e, int phase, const StepParams &p)
     w.x = p.x; w.ly = p.ly; w.mu = p.mu; w.ps = p.ps; w.C = p.C; w.chain0 = p.chain0;
     w.factor_cm = e->factor_cm; w.factor_rm = e->factor; w.diagonal = e->diag_d; w.counts = p.counts;
     w.key0 = p.key0; w.key1 = p.key1; memcpy(w.rk, p.rk, sizeof w.rk); w.step0 = p.step0; w.nsteps = p.nsteps; w.t0 = p.t0;
-    w.pmh = reinterpret_cast<const double2*>(e->pprep); w.psd = e->pprep + (size_t)2 * e->d * e->mpad;
-    w.pool_m = e->M; w.mpad = e->mpad; w.pool_next = p.pool_next; w.pool_stride = p.pool_stride;
-    w.peers = p.peers; w.npeers = p.npeers; w.next_off = p.next_off; w.arr_off = p.arr_off;
-    w.arrivals = p.arrivals; w.wait_target = p.wait_target; w.pub_wait_target = p.pub_wait_target; w.xflag = p.xflag;   // readers wait in pool_prep, publishers in the kernel
-    w.xstat = p.xstat;
+    WidePool v; wide_pool(e, &v);
+    w.pmh = v.pmh; w.psd = v.psd; w.pnb = v.pnb; w.pf = v.pf; w.pnbf = v.pnbf; w.pscal = v.pscal;
+    w.pool_m = e->M; w.mpad = e->mpad; w.xc = p.xc;
     w.hist = p.hist; w.thin = p.thin; w.hist_cap = p.hist_cap; w.hist_ring0 = p.hist_ring0;
-    w.pnb = e->pprep + (size_t)3 * e->d * e->mpad; w.summix = e->remote_mode; w.exact_tests = p.exact_tests;
-    w.pf = reinterpret_cast<const float2*>(e->pprep + ((size_t)3 * e->d + 1) * e->mpad);        // fp32 copy behind the fp64 arrays
-    w.pnbf = reinterpret_cast<const float*>(w.pf + (size_t)e->d * e->mpad); w.pscal = w.pnbf + e->mpad;
+    w.summix = e->remote_mode; w.exact_tests = p.exact_tests;
     w.gm2 = reinterpret_cast<const double2*>(e->gm_t);
     w.gm_lw = e->gm_t ? e->gm_t + (size_t)2 * e->d * e->kpad : nullptr; w.kpad = e->kpad;
     w.lik_dev = e->lik_dev; w.lik_k = e->lik_k;
@@ -747,8 +760,7 @@ static int wide_buffers(mcgpu_engine *e)
   const int d = e->d, L = d / 2;
   if (!e->factor_cm) { CK(cudaMalloc((void**)&e->factor_cm, (size_t)d * d * 8)); CK(cudaMalloc((void**)&e->diag_d, sizeof(int))); }
   e->mpad = (e->M + L - 1) / L * L;
-  // (mu, h) pairs, sigma, n_s in fp64; then the fp32 copy: (g mu, g) pairs, n_s log2 e, 4 scalars
-  if (!e->pprep) CK(cudaMalloc((void**)&e->pprep, ((size_t)3 * d + 1) * e->mpad * 8 + ((size_t)2 * d + 1) * e->mpad * 4 + 16));
+  if (!e->pprep) CK(cudaMalloc((void**)&e->pprep, wide_pool(e)));
   return MCGPU_OK;
 }
 
@@ -1102,25 +1114,24 @@ int mcgpu_sample(mcgpu_engine *e, int nsteps)
       CK(exact::launch_verify(p, e->Rl, e->stream));
     } else {
       StepParams p; fill_step_params(e, p);
-      p.counts = e->counts + 4; p.xstat = e->counts + 8;
+      p.counts = e->counts + 4;
       p.pool_cur = pool_cur(e);
-      fill_p2p(e, p);
       p.hist = e->hist; p.hist_ring0 = e->hist ? (int)((e->t_main / e->cfg.thin) % e->hist_cap) : 0;
       // publish (mu, sigma^2) into the next pool only from the launch that ends the window
       double *const publish = ((e->t_main + n) % sync == 0) ? pool_next(e) : nullptr;
+      fill_exchange(e, p.xc, publish);
       // reference remote mode at d = 2: the table of acceptance-ratio bounds over this window's pool, built right
       // before the window's first launch that can take a remote step (it does not depend on the likelihood)
       const bool use_tab = e->d == 2 && !e->wide && e->remote_mode == 0 && !p.exact_tests && !e->replay_local && e->cfg.pl < 1.0;
       auto cell_table = [&]() -> int {
         if (!e->cell_tab) CK(cudaMalloc((void**)&e->cell_tab, fast::cell_table_bytes()));
         ++e->launches;
-        CK(fast::launch_cell_table(pool_cur(e), e->M, e->cell_tab, p.arrivals, p.wait_target, p.xflag, p.xstat, e->stream));
+        CK(fast::launch_cell_table(pool_cur(e), e->M, e->cell_tab, p.xc, e->stream));
         p.cell_tab = e->cell_tab;
         return MCGPU_OK;
       };
       if (e->cfg.coin_group > 0 || e->replay_local) {       // per-group coins: one mixed launch per window
         p.step0 = (uint32_t)(e->nburn_total + e->t_main); p.nsteps = n; p.t0 = (int)e->t_main;
-        p.pool_next = publish;
         if (use_tab && p.t0 + n > p.first_remote_t) { int rc = cell_table(); if (rc) return rc; }
         CK(launch_steps_any(e, PH_MIXED, p));
       } else {                                               // job-wide coin: the host cuts the window into segments
@@ -1130,12 +1141,8 @@ int mcgpu_sample(mcgpu_engine *e, int nsteps)
         bool prepped = !e->wide;
         auto pool_prep = [&]() -> cudaError_t {
           prepped = true; ++e->launches;
-          return fast::launch_pool_prep(pool_cur(e), e->M, e->mpad, e->d, reinterpret_cast<double2*>(e->pprep),
-                                        e->pprep + (size_t)2 * e->d * e->mpad, e->pprep + (size_t)3 * e->d * e->mpad,
-                                        reinterpret_cast<float2*>(e->pprep + ((size_t)3 * e->d + 1) * e->mpad),
-                                        reinterpret_cast<float*>(e->pprep + ((size_t)3 * e->d + 1) * e->mpad) + (size_t)2 * e->d * e->mpad,
-                                        reinterpret_cast<float*>(e->pprep + ((size_t)3 * e->d + 1) * e->mpad) + ((size_t)2 * e->d + 1) * e->mpad,
-                                        p.arrivals, p.wait_target, p.xflag, p.xstat, e->stream);
+          WidePool v; wide_pool(e, &v);
+          return fast::launch_pool_prep(pool_cur(e), e->M, e->mpad, e->d, v, p.xc, e->stream);
         };
         auto is_remote = [&](long long tt) {
           return tt >= (long long)sync * (1 + e->lag) && !(host_coin(e, (uint32_t)(e->nburn_total + tt)) <= e->cfg.pl);   // mcpar.cc:142-152
@@ -1162,7 +1169,7 @@ int mcgpu_sample(mcgpu_engine *e, int nsteps)
           }
           p.step0 = (uint32_t)(e->nburn_total + t); p.nsteps = len; p.t0 = (int)t;
           p.hist_ring0 = e->hist ? (int)((t / e->cfg.thin) % e->hist_cap) : 0;
-          p.pool_next = (k + len == n) ? publish : nullptr;
+          p.xc.pool_next = (k + len == n) ? publish : nullptr;
           CK(launch_steps_any(e, phase, p));
           k += len;
         }

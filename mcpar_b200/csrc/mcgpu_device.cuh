@@ -80,6 +80,21 @@ __device__ __forceinline__ void normal_pair(uint32_t wa, uint32_t wb, double &z0
   z0 = r * s; z1 = r * c;
 }
 
+// The exchange of the remote pool between windows: where a launch publishes its pool slots and, with a peer-to-peer
+// exchange, what it waits for.  The protocol itself is wait_pool, publish_slot and exchange_failed below.
+struct ExchangeParams {
+  double *pool_next;               // publication target [pool_m][d][2], or null: this launch does not publish
+  long long pool_stride;           // slot s is global chain s*pool_stride
+  // peer-to-peer exchange (chains sharded over GPUs, one process each): publication stores go
+  // straight into every peer's next pool buffer over NVLink, then bump the peer's arrival counter
+  char *const *peers; int npeers; long long next_off, arr_off;
+  // consumer side: wait until `arrivals` (this GPU's counter) reaches wait_target before reading the pool
+  // (wait_target: all slots of the publication this launch READS; pub_wait_target: all slots of the
+  // publication before the one it WRITES -- equal without pool lag)
+  const unsigned long long *arrivals; unsigned long long wait_target, pub_wait_target; int *xflag;
+  unsigned long long *xstat;       // {ns CTA 0 spent waiting for arrivals, launches that waited}
+};
+
 // One launch worth of arguments for the fused step kernels.
 struct StepParams {
   // chain state, structure-of-arrays over the hosted chains: x[i*ld + j] etc.
@@ -98,17 +113,9 @@ struct StepParams {
   int first_remote_t;              // main steps before this one are local: sync * (1 + pool_lag)  (mcpar.cc:142-146 with lag 0)
   double pl;
   uint32_t plan_mask; int plan_valid;   // PH_MIXED with a job-wide coin: bit k = step k of this launch is remote
-  // remote-proposal pool: [pool_m][d][2] (mu, sigma^2); slot s is global chain s*pool_stride
-  const double *pool_cur; double *pool_next;
-  // peer-to-peer exchange (chains sharded over GPUs, one process each): publication stores go
-  // straight into every peer's next pool buffer over NVLink, then bump the peer's arrival counter
-  char *const *peers; int npeers; long long next_off, arr_off;
-  // consumer side: wait until `arrivals` (this GPU's counter) reaches wait_target before reading the pool
-  // (wait_target: all slots of the publication this launch READS; pub_wait_target: all slots of the
-  // publication before the one it WRITES -- equal without pool lag)
-  const unsigned long long *arrivals; unsigned long long wait_target, pub_wait_target; int *xflag;
-  unsigned long long *xstat;       // {ns CTA 0 spent waiting for arrivals, launches that waited}
-  int pool_m; long long pool_stride;
+  // remote-proposal pool: [pool_m][d][2] (mu, sigma^2), and where this launch publishes
+  const double *pool_cur; int pool_m;
+  ExchangeParams xc;
   int exact_tests;                 // audit mode: accept / rejection tests always in fp64 (MCGPU_EXACT_TESTS=1)
   // sample history: rows (p..., logL), kept step major, then hosted chain
   // (a ring of hist_cap kept steps; the first kept step of this launch goes to ring row hist_ring0)
@@ -117,7 +124,6 @@ struct StepParams {
   const double *Z, *U; long long nz, nu; int *overrun;
   // likelihood parameters
   double lp[8]; const double *lik_dev; int lik_k;
-  // (last, so that the offsets of the fields above stay as they were)
   // reference remote mode, d = 2: this window's table of acceptance-ratio bounds, or null.  cell_tab[0] = (origin x,
   // origin y, 1 / cell width x, 1 / cell width y), then MCGPU_CELL_G^2 cells (R_lo, R_hi) as float2, row y major
   const float4 *cell_tab;
@@ -137,13 +143,7 @@ struct WideParams {
   int nsteps, t0;
   // remote pool, prepared, slot fastest: pmh [D][Mpad] = (mu, -1/(2 sig^2)) pairs, psd [D][Mpad] = sigma
   const double2 *pmh; const double *psd; int pool_m, mpad;
-  double *pool_next; long long pool_stride;      // publication target [M][D][2]
-  // peer-to-peer exchange (chains sharded over GPUs, one process each): publication stores go
-  // straight into every peer's next pool buffer over NVLink, then bump the peer's arrival counter
-  char *const *peers; int npeers; long long next_off, arr_off;
-  // consumer side: wait until `arrivals` (this GPU's counter) reaches wait_target before reading the pool
-  const unsigned long long *arrivals; unsigned long long wait_target, pub_wait_target; int *xflag;
-  unsigned long long *xstat;
+  ExchangeParams xc;               // readers wait in pool_prep_kernel, publishers here
   double *hist; int thin; int hist_cap, hist_ring0;
   const double *pnb;               // [Mpad] n_s = -1/2 sum_i log sig2_si (remote mode 1: normalised components)
   const float2 *pf; const float *pnbf; const float *pscal;   // fp32 copy [D][Mpad] (g mu, g), [Mpad] n_s log2 e, {max |mu|, max 1/sigma, max |nb|}
@@ -154,6 +154,10 @@ struct WideParams {
   // device likelihood plugin: its par[] (lik_k reals) on the device
   const double *lik_dev; int lik_k;
 };
+
+// The wide kernels' prepared pool, written by pool_prep_kernel and read through the same fields of WideParams (one
+// allocation: wide_pool in mcgpu_api.cu)
+struct WidePool { double2 *pmh; double *psd, *pnb; float2 *pf; float *pnbf, *pscal; };
 
 // Grid, block, dynamic shared memory and chains per lane group of a wide-kernel launch (wide_launch, mh_wide.cuh)
 struct WideLaunch { unsigned grid, block; size_t smem; int nch; };
@@ -234,6 +238,40 @@ __device__ __forceinline__ void wait_arrivals(const unsigned long long *arrivals
   const unsigned long long t0 = global_ns();
   wait_arrivals_thread(arrivals, target, xflag);
   if (xstat && blockIdx.x == 0) { atomicAdd(xstat, global_ns() - t0); atomicAdd(xstat + 1, 1ull); }
+}
+// A peer-to-peer wait timed out (in this launch or an earlier one): the kernel stops stepping instead of sampling from
+// an incomplete pool, and the host reports MCGPU_EPEER at the next synchronize.
+__device__ __forceinline__ bool exchange_failed(const ExchangeParams &x)
+{
+  return x.npeers > 0 && *reinterpret_cast<volatile int *>(x.xflag);
+}
+// The pool-side kernels (pool_prep_kernel, cell_table_kernel): the CTA waits until the publication it reads has arrived.
+__device__ __forceinline__ void wait_pool(const ExchangeParams &x)
+{
+  if (x.wait_target) { wait_arrivals(x.arrivals, x.wait_target, x.xflag, x.xstat); __syncthreads(); }
+}
+// Publish parameters i0 .. i0+N-1 of pool slot s, (mu, ps * winv), into the next pool [pool_m][D][2].  With a
+// peer-to-peer exchange they go into every GPU's next pool over NVLink, and the calling thread then bumps each
+// peer's arrival counter once.  A GPU may not publish P+1 before all of P has reached it: its peers' last CTAs of
+// the previous window may still read pool P-1, which P+2 will overwrite (three buffers).
+template <int N>
+__device__ __forceinline__ void publish_slot(const ExchangeParams &x, long long s, int D, int i0, const double (&mu)[N],
+                                             const double (&ps)[N], double winv)
+{
+  if (x.npeers > 0) {
+    wait_arrivals_thread(x.arrivals, x.pub_wait_target, x.xflag);
+    for (int q = 0; q < x.npeers; ++q) {
+      double *dst = reinterpret_cast<double *>(x.peers[q] + x.next_off);
+#pragma unroll
+      for (int i = 0; i < N; ++i) { dst[(s * D + i0) * 2 + 2 * i] = mu[i]; dst[(s * D + i0) * 2 + 2 * i + 1] = ps[i] * winv; }
+    }
+    __threadfence_system();                              // the stores are visible before the arrivals
+    for (int q = 0; q < x.npeers; ++q)
+      atomicAdd_system(reinterpret_cast<unsigned long long *>(x.peers[q] + x.arr_off), 1ull);
+  } else {
+#pragma unroll
+    for (int i = 0; i < N; ++i) { x.pool_next[(s * D + i0) * 2 + 2 * i] = mu[i]; x.pool_next[(s * D + i0) * 2 + 2 * i + 1] = ps[i] * winv; }
+  }
 }
 
 }  // namespace mcgpu

@@ -79,7 +79,7 @@ mh_coop_kernel(const WideParams p, const int nbatch, const int SL, const int lsl
   float *part = sxf + 2 * D * CP;                       // [DC][CP][SL] partial pool exponents, DC * SL = 256; [0] ends up holding the totals
   float *snb = part + kCoopHalf * CP;                   // [SL]         n_s log2 e
   float2 *spool = reinterpret_cast<float2 *>(snb + SL); // [D][SL]      (g mu, g)
-  if (p.npeers > 0 && *reinterpret_cast<volatile int *>(p.xflag)) return;   // a peer-to-peer wait timed out earlier: stop stepping
+  if (exchange_failed(p.xc)) return;
 
   const int tid = threadIdx.x, warp = tid >> 5, r = tid & 31;
   if (REMOTE && POOLSM) {
@@ -224,8 +224,8 @@ mh_coop_kernel(const WideParams p, const int nbatch, const int SL, const int lsl
       // the one chain of this warp's batch (if any) that owns a pool slot: smallest multiple of the stride at or above
       // the warp's first chain (one division per warp and batch, 32-bit when the operands fit)
       long long pub_j = -1, pub_s = 0;
-      if (MAIN && p.pool_next && k == p.nsteps - 1 && p.pool_stride >= NCW) {
-        const unsigned long long g0 = (unsigned long long)(p.chain0 + jb), st = (unsigned long long)p.pool_stride;
+      if (MAIN && p.xc.pool_next && k == p.nsteps - 1 && p.xc.pool_stride >= NCW) {
+        const unsigned long long g0 = (unsigned long long)(p.chain0 + jb), st = (unsigned long long)p.xc.pool_stride;
         const unsigned long long qd = ((g0 | st) >> 32) == 0 ? (unsigned long long)(((unsigned)g0 + (unsigned)st - 1u) / (unsigned)st) : (g0 + st - 1) / st;
         const unsigned long long first = qd * st;
         if (first < g0 + NCW && qd < (unsigned long long)p.pool_m) { pub_j = (long long)(first - (unsigned long long)p.chain0); pub_s = (long long)qd; }
@@ -263,24 +263,15 @@ mh_coop_kernel(const WideParams p, const int nbatch, const int SL, const int lsl
         }
         bool a;
         if (REMOTE) {
-          // u < exp(lyt - ly) q(x)/q(x') from fp32 bounds on the Hastings factor (summix_bounds of mh_kernels.cuh;
+          // u < exp(lyt - ly) q(x)/q(x') from fp32 bounds on the Hastings factor (summix_cfac_bounds of mh_kernels.cuh;
           // here the exponents are summed chunk by chunk and taken relative to the picked component afterwards:
-          // D + 256/SL + 2 roundings instead of D, covered by the larger rounding term cu)
+          // D + 256/SL + 2 roundings instead of D, covered by the larger rounding terms cu = (24 + D) u24, cn = 4.8e-7 ...)
           const float snc = group_sumf<L>(sn[c]), soc = group_sumf<L>(so[c]);
           const float xabs_n = group_maxf<L>(fmaxf(fabsf((float)xt0), fabsf((float)xt1)));
           const float xabs_o = group_maxf<L>(fmaxf(fabsf((float)x0[c]), fabsf((float)x1[c])));
-          const float mumax = __ldg(p.pscal), isig = __ldg(p.pscal + 1), nbmax = __ldg(p.pscal + 2);
-          const float l2m = lg2_approx((float)p.pool_m), cD = (float)D, cu = (24.0f + cD) * 6.0e-8f;
-          const float cn = 4.8e-7f * nbmax + 1.0e-5f + 1.0e-8f * (float)p.pool_m;
-          bool ok = (snc < 1.0e30f) && (soc < 1.0e30f) && (snc > 0.5f);
-          const float th_n = 1.6e-7f * (mumax + xabs_n) * isig, th_o = 1.6e-7f * (mumax + xabs_o) * isig;
-          const float lvl = nbmax - ref[c] + l2m + 30.0f;
-          const float Een = fmaxf(lvl - lg2_approx(snc), 30.0f), Eeo = fmaxf(lvl - lg2_approx(fmaxf(soc, 1.0e-37f)), 30.0f);
-          const float eps_n = 0.75f * (2.0f * th_n * sqrtf(cD * Een) + cu * Een + cD * th_n * th_n) + cn;
-          const float eps_o = 0.75f * (2.0f * th_o * sqrtf(cD * Eeo) + cu * Eeo + cD * th_o * th_o) + cn;
-          ok = ok && !p.exact_tests && th_n < 1.0e-3f && th_o < 1.0e-3f && eps_n < 0.02f && eps_o < 0.02f;   // (audit mode: always the fp64 route)
-          const float cf_lo = __fdividef(soc * (1.0f - eps_o), snc * (1.0f + eps_n)) * (1.0f - 1.0e-6f);
-          const float cf_hi = __fdividef(fmaf(soc, 1.0f + eps_o, 2.0e-38f * (float)p.pool_m), snc * (1.0f - eps_n)) * (1.0f + 1.0e-6f);
+          float cf_lo, cf_hi;
+          const bool ok = summix_cfac_bounds(snc, soc, ref[c], xabs_n, xabs_o, __ldg(p.pscal), __ldg(p.pscal + 1), __ldg(p.pscal + 2),
+                                             p.pool_m, D, 24.0f, 4.8e-7f, cf_lo, cf_hi) && !p.exact_tests;   // (audit mode: always the fp64 route)
           int dec = ok ? accept_test_bounded(u_acc, lyt - ly[c], cf_lo, cf_hi) : -1;
           if (dec < 0) {                                // rare, warp-uniform: exact log q(x) - log q(x') in fp64
             nfb += live ? 1u : 0u;
@@ -326,28 +317,13 @@ mh_coop_kernel(const WideParams p, const int nbatch, const int SL, const int lsl
           if (r == 0) p.ly[j] = ly[c];
           long long sidx = pub_s;
           bool is_pub = jb + c == pub_j;
-          if (MAIN && p.pool_next && p.pool_stride < NCW) {              // several pool chains in one warp's batch: test each
+          if (MAIN && p.xc.pool_next && p.xc.pool_stride < NCW) {        // several pool chains in one warp's batch: test each
             const long long gg = p.chain0 + j;
-            sidx = gg / p.pool_stride; is_pub = gg - sidx * p.pool_stride == 0 && sidx < p.pool_m;
+            sidx = gg / p.xc.pool_stride; is_pub = gg - sidx * p.xc.pool_stride == 0 && sidx < p.pool_m;
           }
-          if (MAIN && p.pool_next) {                                     // musigall slot rule, mcpar.cc:205-208: chain s * stride is slot s
-            if (is_pub) {
-              const double wi = 1.0 / (double)(p.t0 + p.nsteps);
-              if (p.npeers > 0) {                        // sharded: store into every GPU's next pool over NVLink
-                wait_arrivals_thread(p.arrivals, p.pub_wait_target, p.xflag);   // never more than one publication ahead (mh_kernels.cuh)
-                for (int q = 0; q < p.npeers; ++q) {
-                  double *dst = reinterpret_cast<double *>(p.peers[q] + p.next_off);
-                  dst[(sidx * D + i0) * 2] = mu0;     dst[(sidx * D + i0) * 2 + 1] = ps0 * wi;
-                  dst[(sidx * D + i0 + 1) * 2] = mu1; dst[(sidx * D + i0 + 1) * 2 + 1] = ps1 * wi;
-                }
-                __threadfence_system();                  // each lane's stores are visible before its arrival
-                for (int q = 0; q < p.npeers; ++q)
-                  atomicAdd_system(reinterpret_cast<unsigned long long *>(p.peers[q] + p.arr_off), 1ull);
-              } else {
-                p.pool_next[(sidx * D + i0) * 2] = mu0;     p.pool_next[(sidx * D + i0) * 2 + 1] = ps0 * wi;
-                p.pool_next[(sidx * D + i0 + 1) * 2] = mu1; p.pool_next[(sidx * D + i0 + 1) * 2 + 1] = ps1 * wi;
-              }
-            }
+          if (MAIN && p.xc.pool_next && is_pub) {                        // musigall slot rule, mcpar.cc:205-208: chain s * stride is slot s
+            const double m[2] = {mu0, mu1}, v[2] = {ps0, ps1};
+            publish_slot<2>(p.xc, sidx, D, i0, m, v, 1.0 / (double)(p.t0 + p.nsteps));
           }
         }
       }

@@ -89,13 +89,10 @@ cudaError_t launch_wide(int lik, int d, int phase, const WideParams &p, cudaStre
   return cudaErrorInvalidValue;
 }
 
-cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, double2 *pmh, double *psd, double *pnb,
-                             float2 *pf, float *pnbf, float *pscal,
-                             const unsigned long long *arrivals, unsigned long long wait_target, int *xflag,
-                             unsigned long long *xstat, cudaStream_t st)
+cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, const WidePool &w, const ExchangeParams &xc, cudaStream_t st)
 {
-  cudaMemsetAsync(pscal, 0, 4 * sizeof(float), st);
-  pool_prep_kernel<<<(D * mpad + 127) / 128, 128, 0, st>>>(pool, M, mpad, D, pmh, psd, pnb, pf, pnbf, pscal, arrivals, wait_target, xflag, xstat);
+  cudaMemsetAsync(w.pscal, 0, 4 * sizeof(float), st);
+  pool_prep_kernel<<<(D * mpad + 127) / 128, 128, 0, st>>>(pool, M, mpad, D, w, xc);
   return cudaGetLastError();
 }
 
@@ -111,11 +108,9 @@ struct CellRedWarp {
 // from the pool itself (exact min / max reductions: all warps agree); a pool with a non-finite or non-positive entry
 // gets a NaN header, which no candidate passes.  With a peer-to-peer exchange the CTAs first wait for the arrivals,
 // as pool_prep_kernel does.
-static __global__ void __launch_bounds__(128) cell_table_kernel(const double *pool, int M, float4 *tab,
-                                                                 const unsigned long long *arrivals, unsigned long long wait_target,
-                                                                 int *xflag, unsigned long long *xstat)
+static __global__ void __launch_bounds__(128) cell_table_kernel(const double *pool, int M, float4 *tab, const ExchangeParams xc)
 {
-  if (wait_target) { wait_arrivals(arrivals, wait_target, xflag, xstat); __syncthreads(); }
+  wait_pool(xc);
   constexpr int G = MCGPU_CELL_G;
   const int lane = threadIdx.x & 31, cell = blockIdx.x * 4 + (threadIdx.x >> 5);
   const CellRedWarp red;
@@ -149,10 +144,9 @@ static __global__ void __launch_bounds__(128) cell_table_kernel(const double *po
 
 size_t cell_table_bytes() { return sizeof(float4) + sizeof(float2) * MCGPU_CELL_G * MCGPU_CELL_G; }
 
-cudaError_t launch_cell_table(const double *pool, int M, float4 *tab, const unsigned long long *arrivals,
-                              unsigned long long wait_target, int *xflag, unsigned long long *xstat, cudaStream_t st)
+cudaError_t launch_cell_table(const double *pool, int M, float4 *tab, const ExchangeParams &xc, cudaStream_t st)
 {
-  cell_table_kernel<<<MCGPU_CELL_G * MCGPU_CELL_G / 4, 128, 0, st>>>(pool, M, tab, arrivals, wait_target, xflag, xstat);
+  cell_table_kernel<<<MCGPU_CELL_G * MCGPU_CELL_G / 4, 128, 0, st>>>(pool, M, tab, xc);
   return cudaGetLastError();
 }
 

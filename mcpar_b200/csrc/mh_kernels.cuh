@@ -547,6 +547,26 @@ __device__ __noinline__ double summix_lse_exact(const PointD<D> x, const double2
   return m + mc_log(s, T);                             // no finite term: -inf + log 0 = -inf
 }
 
+// The finish of the bound above, shared by every kernel family: from the two sums sn = Sn and so = So, the level ref,
+// max |x'| and max |x| over the parameters and the pool scalars (max |mu|, max 1/sigma, max |nb|) to cfac in [cf_lo,
+// cf_hi]; false when the bound cannot settle the step.  ru and rn are the rounding terms cu = (ru + D) u24 and cn = rn
+// |nb|max + ...: 4 and 2.4e-7 for sums taken relative to ref slot by slot, more where they are not (mh_coop.cuh).
+__device__ __forceinline__ bool summix_cfac_bounds(float sn, float so, float ref, float xabs_n, float xabs_o, float mumax,
+                                                   float isig, float nbmax, int M, int D, float ru, float rn,
+                                                   float &cf_lo, float &cf_hi)
+{
+  const float th_n = 1.6e-7f * (mumax + xabs_n) * isig, th_o = 1.6e-7f * (mumax + xabs_o) * isig;
+  const float lvl = nbmax - ref + lg2_approx((float)M) + 30.0f;
+  const float En = fmaxf(lvl - lg2_approx(sn), 30.0f), Eo = fmaxf(lvl - lg2_approx(fmaxf(so, 1.0e-37f)), 30.0f);
+  const float cD = (float)D, cu = (ru + cD) * 6.0e-8f, cn = rn * nbmax + 1.0e-5f + 1.0e-8f * (float)M;
+  const float eps_n = 0.75f * (2.0f * th_n * sqrtf(cD * En) + cu * En + cD * th_n * th_n) + cn;
+  const float eps_o = 0.75f * (2.0f * th_o * sqrtf(cD * Eo) + cu * Eo + cD * th_o * th_o) + cn;
+  cf_lo = __fdividef(so * (1.0f - eps_o), sn * (1.0f + eps_n)) * (1.0f - 1.0e-6f);
+  cf_hi = __fdividef(fmaf(so, 1.0f + eps_o, 2.0e-38f * (float)M), sn * (1.0f - eps_n)) * (1.0f + 1.0e-6f);
+  return sn < 1.0e30f && so < 1.0e30f && sn > 0.5f &&          // overflow / NaN: exact path
+         th_n < 1.0e-3f && th_o < 1.0e-3f && eps_n < 0.02f && eps_o < 0.02f;
+}
+
 template <int D>
 __device__ __forceinline__ bool summix_bounds(const double (&xo)[D], const double (&xn)[D], int c, int M,
                                               const float4 *sPf, const float *sNb, const float *s_scal,
@@ -576,18 +596,9 @@ __device__ __forceinline__ bool summix_bounds(const double (&xo)[D], const doubl
     }
   }
   const float sn = (Sn[0] + Sn[1]) + (Sn[2] + Sn[3]), so = (So[0] + So[1]) + (So[2] + So[3]);
-  if (!(sn < 1.0e30f) || !(so < 1.0e30f) || !(sn > 0.5f)) return false;      // overflow / NaN: exact path
-  const float mumax = s_scal[0], isig = s_scal[1], nbmax = s_scal[2];
-  const float th_n = 1.6e-7f * (mumax + xabs_n) * isig, th_o = 1.6e-7f * (mumax + xabs_o) * isig;
-  const float lvl = nbmax - ref + lg2_approx((float)M) + 30.0f;
-  const float En = fmaxf(lvl - lg2_approx(sn), 30.0f), Eo = fmaxf(lvl - lg2_approx(fmaxf(so, 1.0e-37f)), 30.0f);
-  const float cD = (float)D, cu = (4.0f + cD) * 6.0e-8f, cn = 2.4e-7f * nbmax + 1.0e-5f + 1.0e-8f * (float)M;
-  const float eps_n = 0.75f * (2.0f * th_n * sqrtf(cD * En) + cu * En + cD * th_n * th_n) + cn;
-  const float eps_o = 0.75f * (2.0f * th_o * sqrtf(cD * Eo) + cu * Eo + cD * th_o * th_o) + cn;
-  if (!(th_n < 1.0e-3f && th_o < 1.0e-3f && eps_n < 0.02f && eps_o < 0.02f)) return false;
-  cf_lo = __fdividef(so * (1.0f - eps_o), sn * (1.0f + eps_n)) * (1.0f - 1.0e-6f);
-  cf_hi = __fdividef(fmaf(so, 1.0f + eps_o, 2.0e-38f * (float)M), sn * (1.0f - eps_n)) * (1.0f + 1.0e-6f);
-  return true;
+  // (the overflow test once more, ahead of the arithmetic: it keeps the step loop of this kernel two instructions shorter)
+  if (!(sn < 1.0e30f) || !(so < 1.0e30f) || !(sn > 0.5f)) return false;
+  return summix_cfac_bounds(sn, so, ref, xabs_n, xabs_o, s_scal[0], s_scal[1], s_scal[2], M, D, 4.0f, 2.4e-7f, cf_lo, cf_hi);
 }
 
 // u < exp(delta) cfac with cfac in [cf_lo, cf_hi]:  1 accept, 0 reject, -1 the bounds straddle u.
@@ -685,7 +696,7 @@ mh_steps_kernel(const StepParams p)
   T.exp_tab = T.log_tab = T.trig_tab = nullptr;
 #endif
 
-  if (MAIN && p.npeers > 0 && *reinterpret_cast<volatile int *>(p.xflag)) return;   // a peer-to-peer wait timed out earlier: stop stepping
+  if (MAIN && exchange_failed(p.xc)) return;
   const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const bool live = j < p.C;
   const long long jc = live ? j : p.C - 1;           // idle lanes shadow the last chain, never store
@@ -718,7 +729,7 @@ mh_steps_kernel(const StepParams p)
   // 3-9 % of the kernel's throughput on every GPU and bought 3 % at 8 GPUs: profiles/r01_history.md.
   if constexpr (CAN_REMOTE) {
     if (p.t0 + p.nsteps > p.first_remote_t)
-      if (!stage_pool<D>(p.pool_cur, p.pool_m, p.arrivals, p.wait_target, p.xflag, p.xstat, sPmh, sPs, sPf, sSf, sPn, sNb, s_scal, Mpad, T)) return;
+      if (!stage_pool<D>(p.pool_cur, p.pool_m, p.xc.arrivals, p.xc.wait_target, p.xc.xflag, p.xc.xstat, sPmh, sPs, sPf, sSf, sPn, sNb, s_scal, Mpad, T)) return;
   }
   for (int k = 0; k < p.nsteps; ++k) {
     const uint32_t step = p.step0 + (uint32_t)k;
@@ -954,29 +965,8 @@ mh_steps_kernel(const StepParams p)
       for (int i = 0; i < D; ++i) { p.mu[i * p.ld + j] = mu[i]; p.ps[i * p.ld + j] = ps[i]; }
       // publish to the next exchange pool (musigall slot rule, mcpar.cc:205-208)
       const long long gg = p.chain0 + j;
-      if (p.pool_next && gg % p.pool_stride == 0 && gg / p.pool_stride < p.pool_m) {
-        const long long s = gg / p.pool_stride;
-        const double winv = 1.0 / (double)(p.t0 + p.nsteps);
-        if (p.npeers > 0) {                            // sharded: store into every GPU's next pool over NVLink
-          // A GPU may not publish P+1 before all of P has reached it: its peers' last CTAs of the
-          // previous window may still read pool P-1, which P+2 will overwrite (three buffers).
-          wait_arrivals_thread(p.arrivals, p.pub_wait_target, p.xflag);
-          for (int r = 0; r < p.npeers; ++r) {
-            double *dst = reinterpret_cast<double *>(p.peers[r] + p.next_off);
-#pragma unroll
-            for (int i = 0; i < D; ++i) { dst[(s * D + i) * 2] = mu[i]; dst[(s * D + i) * 2 + 1] = ps[i] * winv; }
-          }
-          __threadfence_system();
-          for (int r = 0; r < p.npeers; ++r)
-            atomicAdd_system(reinterpret_cast<unsigned long long *>(p.peers[r] + p.arr_off), 1ull);
-        } else {
-#pragma unroll
-          for (int i = 0; i < D; ++i) {
-            p.pool_next[(s * D + i) * 2] = mu[i];
-            p.pool_next[(s * D + i) * 2 + 1] = ps[i] * winv;
-          }
-        }
-      }
+      if (p.xc.pool_next && gg % p.xc.pool_stride == 0 && gg / p.xc.pool_stride < p.pool_m)
+        publish_slot<D>(p.xc, gg / p.xc.pool_stride, D, 0, mu, ps, 1.0 / (double)(p.t0 + p.nsteps));
     }
   }
   // acceptance counters of this window

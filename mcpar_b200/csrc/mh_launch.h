@@ -7,14 +7,10 @@ namespace fast {
 bool wide_supported(int lik, int d);
 cudaError_t launch_wide(int lik, int d, int phase, const WideParams &p, cudaStream_t st);
 WideLaunch wide_launch(int d, long long C);   // the wide kernels' launch rule (built-in likelihoods and plugins)
-cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, double2 *pmh, double *psd, double *pnb,
-                             float2 *pf, float *pnbf, float *pscal,
-                             const unsigned long long *arrivals, unsigned long long wait_target, int *xflag,
-                             unsigned long long *xstat, cudaStream_t st);
+cudaError_t launch_pool_prep(const double *pool, int M, int mpad, int D, const WidePool &w, const ExchangeParams &xc, cudaStream_t st);
 cudaError_t launch_factor_prep(const double *rm, double *cm, int D, int *diag, cudaStream_t st);
 size_t cell_table_bytes();       // the d = 2 table of acceptance-ratio bounds (StepParams::cell_tab)
-cudaError_t launch_cell_table(const double *pool, int M, float4 *tab, const unsigned long long *arrivals,
-                              unsigned long long wait_target, int *xflag, unsigned long long *xstat, cudaStream_t st);
+cudaError_t launch_cell_table(const double *pool, int M, float4 *tab, const ExchangeParams &xc, cudaStream_t st);
 bool steps_supported(int lik, int d);
 size_t steps_smem_bytes(int d, int nsteps, int pool_m, bool with_pool);
 StepLaunch steps_launch(int d, long long C, int nsteps, int pool_m, int phase);   // the step kernels' launch rule (built-in likelihoods and plugins)

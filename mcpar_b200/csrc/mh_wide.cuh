@@ -244,21 +244,10 @@ __device__ __forceinline__ void wide_summix_bounds(const float *sf, int r, const
     for (int c = 0; c < NCH; ++c) { Sn[c] += ex2_approx(an[c]); So[c] += ex2_approx(ao[c]); }
   }
   const float mumax = __ldg(p.pscal), isig = __ldg(p.pscal + 1), nbmax = __ldg(p.pscal + 2);
-  const float l2m = lg2_approx((float)p.pool_m), cD = (float)D, cu = (4.0f + cD) * 6.0e-8f;
-  const float cn = 2.4e-7f * nbmax + 1.0e-5f + 1.0e-8f * (float)p.pool_m;
 #pragma unroll
-  for (int c = 0; c < NCH; ++c) {
-    const float sn_ = group_sumf<L>(Sn[c]), so_ = group_sumf<L>(So[c]);
-    ok[c] = (sn_ < 1.0e30f) && (so_ < 1.0e30f) && (sn_ > 0.5f);
-    const float th_n = 1.6e-7f * (mumax + xabs_n[c]) * isig, th_o = 1.6e-7f * (mumax + xabs_o[c]) * isig;
-    const float lvl = nbmax - ref[c] + l2m + 30.0f;
-    const float En = fmaxf(lvl - lg2_approx(sn_), 30.0f), Eo = fmaxf(lvl - lg2_approx(fmaxf(so_, 1.0e-37f)), 30.0f);
-    const float eps_n = 0.75f * (2.0f * th_n * sqrtf(cD * En) + cu * En + cD * th_n * th_n) + cn;
-    const float eps_o = 0.75f * (2.0f * th_o * sqrtf(cD * Eo) + cu * Eo + cD * th_o * th_o) + cn;
-    ok[c] = ok[c] && th_n < 1.0e-3f && th_o < 1.0e-3f && eps_n < 0.02f && eps_o < 0.02f;
-    cf_lo[c] = __fdividef(so_ * (1.0f - eps_o), sn_ * (1.0f + eps_n)) * (1.0f - 1.0e-6f);
-    cf_hi[c] = __fdividef(fmaf(so_, 1.0f + eps_o, 2.0e-38f * (float)p.pool_m), sn_ * (1.0f - eps_n)) * (1.0f + 1.0e-6f);
-  }
+  for (int c = 0; c < NCH; ++c)
+    ok[c] = summix_cfac_bounds(group_sumf<L>(Sn[c]), group_sumf<L>(So[c]), ref[c], xabs_n[c], xabs_o[c], mumax, isig, nbmax,
+                               p.pool_m, D, 4.0f, 2.4e-7f, cf_lo[c], cf_hi[c]);
 }
 
 // exact log of the normalised sum-mixture at chain c's staged point (remote mode 1, rare path)
@@ -348,7 +337,7 @@ mh_wide_kernel(const WideParams p)
   MathTables T;
   T.exp_tab = smem; T.log_tab = smem + MCGPU_EXP_TAB; T.trig_tab = T.log_tab + 2 * MCGPU_LOG_TAB;
   stage_math_tables(smem);
-  if (p.npeers > 0 && *reinterpret_cast<volatile int *>(p.xflag)) return;   // a peer-to-peer wait timed out earlier: stop stepping (MCGPU_EPEER at the next synchronize)
+  if (exchange_failed(p.xc)) return;
   const int gib = threadIdx.x / L;              // group within the CTA
   double *sx = smem + MCGPU_MATH_SMEM + (size_t)gib * 2 * D * NCH;
   double *sz = sx + D * NCH;
@@ -602,23 +591,9 @@ mh_wide_kernel(const WideParams p)
       if (MAIN) {
         p.mu[j * D + i0] = mu0[c]; p.mu[j * D + i0 + 1] = mu1[c]; p.ps[j * D + i0] = ps0[c]; p.ps[j * D + i0 + 1] = ps1[c];
         const long long gg = p.chain0 + j;
-        if (p.pool_next && gg % p.pool_stride == 0 && gg / p.pool_stride < p.pool_m) {
-          const long long s = gg / p.pool_stride;
-          const double wi = 1.0 / (double)(p.t0 + p.nsteps);
-          if (p.npeers > 0) {                          // sharded: store into every GPU's next pool over NVLink
-            wait_arrivals_thread(p.arrivals, p.pub_wait_target, p.xflag);   // never more than one publication ahead (mh_kernels.cuh)
-            for (int q = 0; q < p.npeers; ++q) {
-              double *dst = reinterpret_cast<double *>(p.peers[q] + p.next_off);
-              dst[(s * D + i0) * 2] = mu0[c];     dst[(s * D + i0) * 2 + 1] = ps0[c] * wi;
-              dst[(s * D + i0 + 1) * 2] = mu1[c]; dst[(s * D + i0 + 1) * 2 + 1] = ps1[c] * wi;
-            }
-            __threadfence_system();                    // each lane's stores are visible before its arrival
-            for (int q = 0; q < p.npeers; ++q)
-              atomicAdd_system(reinterpret_cast<unsigned long long *>(p.peers[q] + p.arr_off), 1ull);
-          } else {
-            p.pool_next[(s * D + i0) * 2] = mu0[c];     p.pool_next[(s * D + i0) * 2 + 1] = ps0[c] * wi;
-            p.pool_next[(s * D + i0 + 1) * 2] = mu1[c]; p.pool_next[(s * D + i0 + 1) * 2 + 1] = ps1[c] * wi;
-          }
+        if (p.xc.pool_next && gg % p.xc.pool_stride == 0 && gg / p.xc.pool_stride < p.pool_m) {   // each lane its two parameters
+          const double m[2] = {mu0[c], mu1[c]}, v[2] = {ps0[c], ps1[c]};
+          publish_slot<2>(p.xc, gg / p.xc.pool_stride, D, i0, m, v, 1.0 / (double)(p.t0 + p.nsteps));
         }
       }
       if (r == 0) { wacc += nacc[c]; ++nlive; }
@@ -643,31 +618,28 @@ mh_wide_kernel(const WideParams p)
   }
 }
 
-// pool [M][D][2] (mu, sigma^2) -> pmh [D][Mpad] (mu, -1/(2 sigma^2)), psd [D][Mpad] sigma; padding slots get Q = 0
-static __global__ void pool_prep_kernel(const double *pool, int M, int mpad, int D, double2 *pmh, double *psd, double *pnb,
-                                        float2 *pf, float *pnbf, float *pscal,
-                                        const unsigned long long *arrivals, unsigned long long wait_target, int *xflag,
-                                        unsigned long long *xstat)
+// pool [M][D][2] (mu, sigma^2) -> the prepared pool w (WidePool); padding slots get Q = 0
+static __global__ void pool_prep_kernel(const double *pool, int M, int mpad, int D, const WidePool w, const ExchangeParams xc)
 {
-  if (wait_target) { wait_arrivals(arrivals, wait_target, xflag, xstat); __syncthreads(); }   // peer-to-peer exchange: all slots in?
+  wait_pool(xc);
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx < mpad) {                                   // n_s = -1/2 sum_i log sig2_si (remote mode 1); padding 0
     double n = 0.0;
     if (idx < M) for (int i = 0; i < D; ++i) n -= 0.5 * log(pool[((size_t)idx * D + i) * 2 + 1]);
-    pnb[idx] = n; pnbf[idx] = (float)(n * 1.4426950408889634);
-    atomicMax(reinterpret_cast<int *>(pscal + 2), __float_as_int(__double2float_ru(fabs(n * 1.4426950408889634))));
+    w.pnb[idx] = n; w.pnbf[idx] = (float)(n * 1.4426950408889634);
+    atomicMax(reinterpret_cast<int *>(w.pscal + 2), __float_as_int(__double2float_ru(fabs(n * 1.4426950408889634))));
   }
   if (idx >= D * mpad) return;
   const int i = idx / mpad, s = idx % mpad;
   if (s < M) {
     const double m = pool[((size_t)s * D + i) * 2], s2 = pool[((size_t)s * D + i) * 2 + 1];
     const double sd = sqrt(s2), g = sqrt(0.5 * 1.4426950408889634 / s2);     // g = sqrt(log2(e) / (2 sig^2)), as stage_pool
-    pmh[idx] = make_double2(m, -0.5 / s2); psd[idx] = sd;
-    pf[idx] = make_float2((float)(g * m), (float)g);
+    w.pmh[idx] = make_double2(m, -0.5 / s2); w.psd[idx] = sd;
+    w.pf[idx] = make_float2((float)(g * m), (float)g);
     // pool-wide max |mu| and max 1/sigma for the fp32 error bound (non-negative floats order like their bit patterns)
-    atomicMax(reinterpret_cast<int *>(pscal), __float_as_int(__double2float_ru(fabs(m))));
-    atomicMax(reinterpret_cast<int *>(pscal + 1), __float_as_int(__double2float_ru(1.0 / sd)));
-  } else { pmh[idx] = make_double2(1.0e300, -1.0); psd[idx] = 0.0; pf[idx] = make_float2(1.0e18f, 0.0f); }
+    atomicMax(reinterpret_cast<int *>(w.pscal), __float_as_int(__double2float_ru(fabs(m))));
+    atomicMax(reinterpret_cast<int *>(w.pscal + 1), __float_as_int(__double2float_ru(1.0 / sd)));
+  } else { w.pmh[idx] = make_double2(1.0e300, -1.0); w.psd[idx] = 0.0; w.pf[idx] = make_float2(1.0e18f, 0.0f); }
 }
 
 // row-major lower factor -> column-major copy + "is diagonal" flag

@@ -98,7 +98,8 @@ def test_accept_test_interval_contains_exp_delta():
 def _summix_model(rng, M, D, npts, mu_scale, sig_lo, sig_hi, far, chunks=None):
     """summix_bounds (mh_kernels.cuh; wide_summix_bounds of mh_wide.cuh is the same arithmetic spread over lanes) in numpy
     float32 against the exact fp64 q(x)/q(x'); returns the true ratio, the kernel's interval and which points the fast
-    path decides.  chunks = DC models the cooperative kernel (mh_coop.cuh): the exponent of a slot is summed in DC
+    path decides.  The step from the two sums to the interval is summix_cfac_bounds (mh_kernels.cuh), which every kernel
+    family calls.  chunks = DC models the cooperative kernel (mh_coop.cuh): the exponent of a slot is summed in DC
     parameter chunks (from 0, or from nb when DC = 1), the chunk totals are added to nb, and the picked component's total
     is subtracted afterwards; its bound uses the larger rounding terms cu = (24 + D) u, cn = 4.8e-7 nbmax + ..."""
     mu = rng.uniform(-mu_scale, mu_scale, (M, D))
