@@ -267,6 +267,52 @@ int  mcgpu_history_maxlike(mcgpu_engine *e, double *out);
  * mean[d], cov[d][d] over all rows (for checks that cannot afford the D2H). */
 int  mcgpu_history_moments(mcgpu_engine *e, double *mean, double *cov);
 
+/* Convergence diagnostics of the stored history, reduced on the device (INTEGRATION.md, "Convergence diagnostics").
+ * The rows are those mcgpu_history_read returns over the valid history: n kept steps x C hosted chains, ncol = nparam + 1
+ * columns (the parameters, then logL).  Chain c's series x_{c,0..n-1} has mean xbar_c and ddof-1 variance s2_c.
+ * Split chains (ArviZ _split_chains): N = floor(n/2); chain c gives draws [0, N) and [n-N, n), M' = 2C split chains
+ * with means ybar_m, ddof-1 variances v_m and biased autocovariances
+ * gamma_{m,t} = (1/N) sum_{s<N-t} (y_s - ybar_m)(y_{s+t} - ybar_m), t = 0..L.  Superchains (nested R-hat, Margossian
+ * et al.): hosted chains [kG, (k+1)G), K = C/G; xbar_k = mean of its xbar_c, Btilde_k = sum (xbar_c - xbar_k)^2/(G-1)
+ * (0 when G = 1), Wtilde_k = mean of its s2_c.
+ *
+ * mcgpu_history_diag_partials writes one engine's partial block, MCGPU_DIAG_BLOCK(ncol, max_lag) doubles: the header
+ * (n, G, L, ncol), then per column the fields
+ *    0 non-finite count, 1 min, 2 max,
+ *    3..6   C,  mean of xbar_c, M2 of xbar_c (sum of squared deviations), sum of s2_c
+ *    7..10  K,  mean of xbar_k, M2 of xbar_k, sum of (Btilde_k + Wtilde_k)
+ *   11..14  M', mean of ybar_m, M2 of ybar_m, sum of v_m
+ *   15..15+L  sum over m of gamma_{m,t}
+ * Means and M2 come from pairwise (Chan) merges in a fixed order: no cancellation when |mean| >> sd, and a repeated
+ * call returns the same bits.  superchain = G must divide the hosted chain count and chain0 (then superchain k is the
+ * global chains [chain0 + kG, chain0 + (k+1)G) however the job is sharded); 1 <= max_lag <= N - 1.
+ * MCGPU_ESTATE: no history or an empty one; MCGPU_EINVAL: n < 4, a bad superchain or max_lag, a NULL block.  A
+ * refusal launches nothing.
+ *
+ * mcgpu_diag_finalize merges nblock blocks (one per sharded engine, rank order; headers must be equal, else
+ * MCGPU_EINVAL) -- counts and sums add, (count, mean, M2) merge by Chan's formula, min / max combine -- and writes
+ * report[ncol][MCGPU_DIAG_NFIELD].  Host arithmetic only (it needs no device); per column:
+ *   mean = f4;  sd = sqrt(((n-1) f6 + n f5) / (C n - 1)), the ddof-1 sd of all C n draws;
+ *   rhat_split = ArviZ _rhat on the split chains = sqrt((B/W + N - 1)/N), W = f14/M', B = N f13/(M'-1);
+ *   rhat_nested = sqrt(1 + Bhat/What), Bhat = f9/(K-1), What = f10/K (NaN when K < 2);
+ *   ess_mean = ArviZ _ess on the split chains (Geyer's initial positive then monotone sequence) with
+ *     mean_j acov[j,t] = f[15+t]/M', mean_var = (f15/M') N/(N-1), var_plus = mean_var (N-1)/N + f13/(M'-1);
+ *     ess_truncated = 1 when that loop needed a lag beyond L (t < N-3 and the pair sum still > 0);
+ *   mcse_mean = sd / sqrt(ess_mean).
+ * A column with max - min < 1e-15 has ess = M'N, NaN R-hats and mcse 0; a column holding a non-finite value reports
+ * only its count (every statistic NaN).
+ *
+ * mcgpu_history_quantiles: numpy's quantile(method="linear") of each column over this engine's S = C n draws (for a
+ * sharded job: this engine's chains only), q[ncol][nprob]; h = (S-1) p, the order statistics x_(floor h) and
+ * x_(floor h + 1) are exact (radix select on the device) and combined as numpy's _lerp.  1 <= nprob <= 16, p in
+ * [0, 1]; +-inf are ordered values; a column holding NaN gives NaN. */
+#define MCGPU_DIAG_BLOCK(ncol, max_lag) (4 + (ncol) * (16 + (max_lag)))
+enum { MCGPU_DIAG_MEAN, MCGPU_DIAG_SD, MCGPU_DIAG_MCSE_MEAN, MCGPU_DIAG_RHAT_SPLIT, MCGPU_DIAG_RHAT_NESTED,
+       MCGPU_DIAG_ESS_MEAN, MCGPU_DIAG_ESS_TRUNCATED, MCGPU_DIAG_NONFINITE, MCGPU_DIAG_NFIELD };
+int  mcgpu_history_diag_partials(mcgpu_engine *e, int superchain, int max_lag, double *block);
+int  mcgpu_diag_finalize(const double *blocks, int nblock, double *report);
+int  mcgpu_history_quantiles(mcgpu_engine *e, const double *probs, int nprob, double *q);
+
 /* Checkpoint / restart (NORMAL mode; the reference has none).  The blob holds the chain state, the
  * running moments, the tuned proposal factor, the counters, the exchange pools and the schedule;
  * an engine created with the same configuration and likelihood continues the run bit for bit after

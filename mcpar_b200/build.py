@@ -46,6 +46,7 @@ UNITS = {                       # translation unit -> extra flags
     "mh_fast.cu": [],
     "mh_exact.cu": ["-fmad=false"],        # operation-by-operation IEEE arithmetic (verification)
     "mcgpu_api.cu": [stamp_define(kernel_stamp())],
+    "mcgpu_diag.cu": [],                   # history diagnostics: a device module of their own (mcgpu_diag.cuh)
 }
 
 

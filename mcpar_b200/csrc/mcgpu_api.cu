@@ -8,6 +8,8 @@
 #include "../../include/mcgpu.h"
 #include "mh_launch.h"
 #include "mcgpu_sobol.h"
+#include "mcgpu_diag.cuh"
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdio.h>
@@ -826,6 +828,8 @@ int mcgpu_set_likelihood(mcgpu_engine *e, int lik, const double *par, int npar)
   return MCGPU_OK;
 }
 
+static int p2p_load_kernels(mcgpu_engine *e);
+
 int mcgpu_set_likelihood_plugin(mcgpu_engine *e, const char *cubin_path, const double *par, int npar)
 {
   if (!e) return MCGPU_EINVAL;
@@ -855,6 +859,7 @@ int mcgpu_set_likelihood_plugin(mcgpu_engine *e, const char *cubin_path, const d
   memset(e->lp, 0, sizeof e->lp);
   for (int i = 0; i < npar && i < 8; ++i) e->lp[i] = par[i];
   e->lik = MCGPU_DEVICE_PLUGIN; e->lik_k = npar; e->wide = wide;
+  if (e->p2p) return p2p_load_kernels(e);                 // a plugin set after the peers attached
   return MCGPU_OK;
 }
 
@@ -1233,8 +1238,47 @@ static int p2p_check(mcgpu_engine *e, int world, int rank)
   return MCGPU_OK;
 }
 
+// Load every function of the device module holding `kernel` into the current context (cuFuncLoad through the
+// runtime's driver entry points, CUDA >= 12.4).
+static cudaError_t load_module_of(const void *kernel)
+{
+  static const char *const names[4] = {"cuFuncGetModule", "cuModuleGetFunctionCount", "cuModuleEnumerateFunctions", "cuFuncLoad"};
+  void *fn[4] = {};
+  for (int i = 0; i < 4; ++i) {
+    cudaDriverEntryPointQueryResult q;
+    const cudaError_t s = cudaGetDriverEntryPointByVersion(names[i], &fn[i], 12040, cudaEnableDefault, &q);
+    if (s != cudaSuccess) return s;
+    if (q != cudaDriverEntryPointSuccess || !fn[i]) return cudaErrorSymbolNotFound;
+  }
+  cudaFunction_t f = nullptr; CUmodule m = nullptr; unsigned n = 0;
+  cudaError_t s = cudaGetFuncBySymbol(&f, kernel);
+  if (s != cudaSuccess) return s;
+  if (((CUresult (*)(CUmodule *, CUfunction))fn[0])(&m, (CUfunction)f) != CUDA_SUCCESS ||
+      ((CUresult (*)(unsigned *, CUmodule))fn[1])(&n, m) != CUDA_SUCCESS) return cudaErrorUnknown;
+  std::vector<CUfunction> fs(n);
+  if (n && ((CUresult (*)(CUfunction *, unsigned, CUmodule))fn[2])(fs.data(), n, m) != CUDA_SUCCESS) return cudaErrorUnknown;
+  for (CUfunction h : fs)
+    if (((CUresult (*)(CUfunction))fn[3])(h) != CUDA_SUCCESS) return cudaErrorUnknown;
+  return cudaSuccess;
+}
+
+// A peer-to-peer engine's kernels spin until their peers publish, and peers may share the device.  With lazy module
+// loading (the CUDA default) the first launch of a kernel can need a context synchronisation, which then waits for a
+// peer's spinning kernel while that kernel waits for the launch: a deadlock until the exchange times out.  So every
+// kernel such an engine can launch is loaded before it samples: the step-kernel module, this file's module and the
+// plugin's kernels.
+static int p2p_load_kernels(mcgpu_engine *e)
+{
+  CK(load_module_of(fast::module_kernel()));
+  CK(load_module_of(reinterpret_cast<const void *>(fill_kernel)));
+  for (int w = 0; w < 8; ++w)
+    if (e->pk[w]) { cudaFuncAttributes a; CK(cudaFuncGetAttributes(&a, reinterpret_cast<const void *>(e->pk[w]))); }
+  return MCGPU_OK;
+}
+
 static int p2p_finish(mcgpu_engine *e, int world, const std::vector<char*> &bases)
 {
+  if (int rc = p2p_load_kernels(e)) return rc;
   CK(cudaMalloc((void**)&e->peers_d, sizeof(char*) * world));
   CK(cudaMemcpyAsync(e->peers_d, bases.data(), sizeof(char*) * world, cudaMemcpyHostToDevice, e->stream));
   CK(cudaStreamSynchronize(e->stream));
@@ -1708,6 +1752,269 @@ int mcgpu_history_moments(mcgpu_engine *e, double *mean, double *cov)
   int q = d;
   for (int i = 0; i < d; ++i)
     for (int j = i; j < d; ++j, ++q) { const double c = h[q] / n - mean[i] * mean[j]; cov[i * d + j] = c; cov[j * d + i] = c; }
+  return MCGPU_OK;
+}
+
+// ---- convergence diagnostics and quantiles of the history (kernels: mcgpu_diag.cuh) -------------------------------
+namespace {
+using mcgpu_diag::Part;
+
+// the rows the diagnostics see (the same as mcgpu_history_read over the valid history): their count n and the ring
+// addresses of the logical rows
+int diag_rows(mcgpu_engine *e, long long *n, mcgpu_diag::DiagRows *rows, HistSeg seg[2], int *nseg)
+{
+  if (!e->hist) return fail(e, MCGPU_ESTATE, "engine was created with history_steps = 0");
+  *nseg = hist_segments(e, seg);
+  if (*nseg == 0) return fail(e, MCGPU_ESTATE, "history is empty");
+  const long long row = e->C * (e->d + 1);
+  *n = seg[0].count + (*nseg > 1 ? seg[1].count : 0);
+  if (*n < 4) return fail(e, MCGPU_EINVAL, "diagnostics need at least 4 kept steps in the history");
+  if (*n > (1ll << 30)) return fail(e, MCGPU_EINVAL, "history too long for the diagnostics (more than 2^30 kept steps)");
+  if (rows) *rows = {e->hist + seg[0].ring0 * row, e->hist, seg[0].count, row};
+  return 0;
+}
+
+// fixed-order merge of in[ncol][nin] in groups of gs entries into out[ncol][nin / gs]: one level when a group is at
+// most 1024 entries, else chunks of 1024 into tmp, then the chunks of each group
+int diag_reduce(mcgpu_engine *e, const Part *in, long long nin, long long gs, int to_item, Part *tmp, Part *out)
+{
+  const int ncol = e->d + 1;
+  auto launch = [&](const Part *src, long long nsrc, long long g, long long ch, int item, Part *dst) -> int {
+    ++e->launches;
+    CK(mcgpu_diag::diag_group(src, nsrc, ncol, g, ch, item, dst, e->stream));
+    return 0;
+  };
+  const long long ch = 1024;
+  if (gs <= ch) return launch(in, nin, gs, gs, to_item, out);
+  const long long nchunk = (gs + ch - 1) / ch;
+  if (int rc = launch(in, nin, gs, ch, 0, tmp)) return rc;
+  return launch(tmp, nin / gs * nchunk, nchunk, nchunk, to_item, out);
+}
+}  // namespace
+
+int mcgpu_history_diag_partials(mcgpu_engine *e, int superchain, int max_lag, double *block)
+{
+  if (!e) return MCGPU_EINVAL;
+  if (!block) return fail(e, MCGPU_EINVAL, "block is NULL");
+  DeviceGuard g(e->dev);
+  long long n = 0; mcgpu_diag::DiagRows rows; HistSeg seg[2]; int nseg = 0;
+  if (int rc = diag_rows(e, &n, &rows, seg, &nseg)) return rc;
+  const long long C = e->C, G = superchain;
+  if (G < 1 || C % G || e->cfg.chain0 % G)
+    return fail(e, MCGPU_EINVAL, "superchain must be >= 1 and divide both the hosted chain count and chain0");
+  const int N = (int)(n / 2), L = max_lag, ncol = e->d + 1;
+  if (L < 1 || L > N - 1) return fail(e, MCGPU_EINVAL, "max_lag must be in 1 .. floor(n/2) - 1");
+  const long long K = C / G, cpb = mcgpu_diag::DIAG_THREADS / ncol, nblk = (C + cpb - 1) / cpb;   // diag_chain's CTAs
+  const long long n_chain = ncol * C, n_split = ncol * 2 * C, n_tmp = ncol * (2 * C / 512 + 4), n_sup = ncol * K;
+  const long long n_lagp = nblk * ncol * (L + 1), n_lag = (long long)ncol * (L + 1);
+  const size_t bytes = (size_t)(n_chain + n_split + n_tmp + n_sup + 3 * ncol) * sizeof(Part) + (size_t)(n_lagp + n_lag) * 8;
+  char *scratch = nullptr;
+  CK(cudaMallocAsync((void**)&scratch, bytes, e->stream));
+  Part *chain = (Part*)scratch, *split = chain + n_chain, *tmp = split + n_split, *sup = tmp + n_tmp;
+  Part *all = sup + n_sup, *kst = all + ncol, *spl = kst + ncol;
+  double *lagp = (double*)(spl + ncol), *lags = lagp + n_lagp;
+  int rc = 0;
+  ++e->launches;
+  if (mcgpu_diag::diag_chain(rows, C, ncol, (int)n, L, chain, split, lagp, e->stream) != cudaSuccess)
+    rc = fail(e, MCGPU_ECUDA, "diag_chain_kernel launch failed");
+  if (!rc) rc = diag_reduce(e, chain, C, C, 0, tmp, all);                 // all hosted chains: fields 0..6
+  if (!rc) rc = diag_reduce(e, chain, C, G, 1, tmp, sup);                 // superchain items (xbar_k, Btilde_k + Wtilde_k)
+  if (!rc) rc = diag_reduce(e, sup, K, K, 0, tmp, kst);                   // fields 7..10
+  if (!rc) rc = diag_reduce(e, split, 2 * C, 2 * C, 0, tmp, spl);         // fields 11..14
+  if (!rc) {
+    ++e->launches;
+    if (mcgpu_diag::diag_sum_rows(lagp, nblk, n_lag, lags, e->stream) != cudaSuccess)
+      rc = fail(e, MCGPU_ECUDA, "diag_sum_rows_kernel launch failed");
+  }
+  std::vector<Part> h(3 * ncol); std::vector<double> hl(n_lag);
+  if (!rc) {
+    CK(cudaMemcpyAsync(h.data(), all, 3 * ncol * sizeof(Part), cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaMemcpyAsync(hl.data(), lags, n_lag * 8, cudaMemcpyDeviceToHost, e->stream));
+  }
+  CK(cudaFreeAsync(scratch, e->stream));
+  CK(cudaStreamSynchronize(e->stream));
+  if (rc) return rc;
+  block[0] = (double)n; block[1] = (double)G; block[2] = L; block[3] = ncol;
+  for (int j = 0; j < ncol; ++j) {
+    double *f = block + 4 + (size_t)j * (16 + L);
+    const Part &a = h[j], &k = h[ncol + j], &s = h[2 * ncol + j];
+    f[0] = a.nf; f[1] = a.mn; f[2] = a.mx;
+    f[3] = a.cnt; f[4] = a.mean; f[5] = a.m2; f[6] = a.sx;
+    f[7] = k.cnt; f[8] = k.mean; f[9] = k.m2; f[10] = k.sx;
+    f[11] = s.cnt; f[12] = s.mean; f[13] = s.m2; f[14] = s.sx;
+    for (int t = 0; t <= L; ++t) f[15 + t] = hl[(size_t)j * (L + 1) + t];
+  }
+  return MCGPU_OK;
+}
+
+namespace {
+// ArviZ's _ess (arviz/stats/diagnostics.py) on the split chains, from the merged column fields f (see mcgpu.h);
+// *truncated is set when Geyer's positive-sequence loop needed a lag beyond L
+double diag_ess(const double *f, int N, int L, double *truncated)
+{
+  const double Mp = f[11];
+  auto acov = [&](int t) { return f[15 + t] / Mp; };
+  const double mean_var = acov(0) * N / (N - 1.0);
+  double var_plus = mean_var * (N - 1.0) / N;
+  if (Mp > 1) var_plus += f[13] / (Mp - 1);
+  std::vector<double> rho(N, 0.0);
+  double rho_even = 1.0, rho_odd = 1.0 - (mean_var - acov(1)) / var_plus;
+  rho[0] = rho_even; rho[1] = rho_odd;
+  int t = 1;
+  *truncated = 0.0;
+  while (t < N - 3 && rho_even + rho_odd > 0.0) {
+    if (t + 2 > L) { *truncated = 1.0; break; }
+    rho_even = 1.0 - (mean_var - acov(t + 1)) / var_plus;
+    rho_odd = 1.0 - (mean_var - acov(t + 2)) / var_plus;
+    if (rho_even + rho_odd >= 0) { rho[t + 1] = rho_even; rho[t + 2] = rho_odd; }
+    t += 2;
+  }
+  const int max_t = t - 2;
+  if (rho_even > 0) rho[max_t + 1] = rho_even;
+  for (t = 1; t <= max_t - 2; t += 2)
+    if (rho[t + 1] + rho[t + 2] > rho[t - 1] + rho[t]) { rho[t + 1] = (rho[t - 1] + rho[t]) / 2.0; rho[t + 2] = rho[t + 1]; }
+  const double ess = Mp * N;
+  double s1 = 0.0, s2 = 0.0;
+  for (int k = 0; k <= max_t; ++k) s1 += rho[k];
+  if (max_t + 1 < N) s2 = rho[max_t + 1];
+  double tau = -1.0 + 2.0 * s1 + s2;
+  tau = std::max(tau, 1.0 / log10(ess));
+  for (int k = 0; k < N; ++k) if (isnan(rho[k])) return NAN;
+  return ess / tau;
+}
+}  // namespace
+
+int mcgpu_diag_finalize(const double *blocks, int nblock, double *report)
+{
+  if (!blocks || !report || nblock < 1) return fail(nullptr, MCGPU_EINVAL, "mcgpu_diag_finalize: NULL pointer or nblock < 1");
+  const double n = blocks[0], G = blocks[1], Ld = blocks[2], nc = blocks[3];
+  if (!(n >= 4 && n < 2e9 && n == floor(n)) || !(G >= 1 && G == floor(G)) || !(nc >= 1 && nc <= 1e6 && nc == floor(nc)) ||
+      !(Ld >= 1 && Ld <= floor(n / 2) - 1 && Ld == floor(Ld)))
+    return fail(nullptr, MCGPU_EINVAL, "mcgpu_diag_finalize: malformed block header");
+  const int L = (int)Ld, ncol = (int)nc, N = (int)(n / 2);
+  const size_t bs = 4 + (size_t)ncol * (16 + L);
+  for (int b = 1; b < nblock; ++b)
+    if (memcmp(blocks, blocks + b * bs, 4 * sizeof(double)))
+      return fail(nullptr, MCGPU_EINVAL, "mcgpu_diag_finalize: block headers differ (n, superchain, max_lag or ncol)");
+  std::vector<double> f(16 + L);
+  for (int j = 0; j < ncol; ++j) {
+    const double *f0 = blocks + 4 + (size_t)j * (16 + L);
+    std::copy(f0, f0 + 16 + L, f.begin());
+    for (int b = 1; b < nblock; ++b) {
+      const double *g = f0 + b * bs;
+      f[0] += g[0]; f[1] = fmin(f[1], g[1]); f[2] = fmax(f[2], g[2]);
+      mcgpu_diag::chan_merge(f[3], f[4], f[5], g[3], g[4], g[5]); f[6] += g[6];
+      mcgpu_diag::chan_merge(f[7], f[8], f[9], g[7], g[8], g[9]); f[10] += g[10];
+      mcgpu_diag::chan_merge(f[11], f[12], f[13], g[11], g[12], g[13]); f[14] += g[14];
+      for (int t = 0; t <= L; ++t) f[15 + t] += g[15 + t];
+    }
+    double *r = report + (size_t)j * MCGPU_DIAG_NFIELD;
+    for (int k = 0; k < MCGPU_DIAG_NFIELD; ++k) r[k] = NAN;
+    r[MCGPU_DIAG_NONFINITE] = f[0];
+    if (f[0] > 0) continue;
+    const double Cn = f[3], Mp = f[11], K = f[7];
+    r[MCGPU_DIAG_MEAN] = f[4];
+    r[MCGPU_DIAG_SD] = sqrt(((n - 1) * f[6] + n * f[5]) / (Cn * n - 1));
+    if (f[2] - f[1] < 1e-15) {                             // ArviZ's constant test (np.finfo(float).resolution)
+      r[MCGPU_DIAG_ESS_MEAN] = Mp * N; r[MCGPU_DIAG_ESS_TRUNCATED] = 0; r[MCGPU_DIAG_MCSE_MEAN] = 0;
+      continue;
+    }
+    const double W = f[14] / Mp, B = N * (f[13] / (Mp - 1));
+    r[MCGPU_DIAG_RHAT_SPLIT] = sqrt((B / W + N - 1) / N);
+    if (K >= 2) r[MCGPU_DIAG_RHAT_NESTED] = sqrt(1.0 + (f[9] / (K - 1)) / (f[10] / K));
+    r[MCGPU_DIAG_ESS_MEAN] = diag_ess(f.data(), N, L, &r[MCGPU_DIAG_ESS_TRUNCATED]);
+    r[MCGPU_DIAG_MCSE_MEAN] = r[MCGPU_DIAG_SD] / sqrt(r[MCGPU_DIAG_ESS_MEAN]);
+  }
+  return MCGPU_OK;
+}
+
+int mcgpu_history_quantiles(mcgpu_engine *e, const double *probs, int nprob, double *q)
+{
+  if (!e) return MCGPU_EINVAL;
+  if (!probs || !q) return fail(e, MCGPU_EINVAL, "probs or q is NULL");
+  if (nprob < 1 || nprob > 16) return fail(e, MCGPU_EINVAL, "nprob must be in 1 .. 16");
+  for (int k = 0; k < nprob; ++k)
+    if (!(probs[k] >= 0.0 && probs[k] <= 1.0)) return fail(e, MCGPU_EINVAL, "probabilities must lie in [0, 1]");
+  DeviceGuard g(e->dev);
+  long long n = 0; HistSeg seg[2]; int nseg = 0;
+  if (int rc = diag_rows(e, &n, nullptr, seg, &nseg)) return rc;
+  const int ncol = e->d + 1, nt = 2 * nprob, B = mcgpu_diag::QSEL_BINS;
+  const long long S = n * e->C, row = e->C * ncol;
+  // numpy's method="linear": h = (S - 1) p, order statistics floor(h) and floor(h) + 1 (clipped to S - 1)
+  std::vector<double> hh(nprob); std::vector<long long> rank(nt);
+  for (int k = 0; k < nprob; ++k) {
+    hh[k] = (double)(S - 1) * probs[k];
+    const long long i = std::min<long long>((long long)floor(hh[k]), S - 1);
+    rank[2 * k] = i; rank[2 * k + 1] = std::min(i + 1, S - 1);
+  }
+  std::vector<uint64_t> pref((size_t)ncol * nt, 0); std::vector<unsigned long long> rem((size_t)ncol * nt);
+  for (int j = 0; j < ncol; ++j) for (int t = 0; t < nt; ++t) rem[(size_t)j * nt + t] = rank[t];
+  int optin = 0;
+  CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, e->dev));
+  const size_t budget = std::min<size_t>((size_t)optin, 200 << 10);
+  const size_t nslot_max = (size_t)ncol * nt;
+  char *scratch = nullptr;
+  const size_t bytes = nslot_max * B * 8 + nslot_max * 8 + (ncol + 1) * 4 + ncol * 8 + 64;
+  CK(cudaMallocAsync((void**)&scratch, bytes, e->stream));
+  unsigned long long *hist = (unsigned long long*)scratch, *nanc = hist + nslot_max * B;
+  uint64_t *dpref = (uint64_t*)(nanc + ncol); int *dsoff = (int*)(dpref + nslot_max);
+  CK(cudaMemsetAsync(nanc, 0, ncol * 8, e->stream));
+  std::vector<unsigned long long> hh_hist; std::vector<uint64_t> spref; std::vector<int> soff, tslot((size_t)ncol * nt);
+  int rc = 0;
+  for (int pass = 0; pass < 8 && !rc; ++pass) {
+    for (int j0 = 0; j0 < ncol && !rc;) {
+      // slots: the distinct prefixes of each column's targets, columns [j0, j1) as many as the shared memory holds
+      spref.clear(); soff.assign(1, 0);
+      int j1 = j0;
+      while (j1 < ncol) {
+        std::vector<uint64_t> u;
+        for (int t = 0; t < nt; ++t) u.push_back(pass ? pref[(size_t)j1 * nt + t] : 0);
+        std::sort(u.begin(), u.end()); u.erase(std::unique(u.begin(), u.end()), u.end());
+        if (j1 > j0 && ((spref.size() + u.size()) * B + (j1 - j0 + 1)) * 4 > budget) break;
+        for (int t = 0; t < nt; ++t)
+          tslot[(size_t)j1 * nt + t] = (int)spref.size() + (int)(std::lower_bound(u.begin(), u.end(), pass ? pref[(size_t)j1 * nt + t] : 0) - u.begin());
+        spref.insert(spref.end(), u.begin(), u.end()); soff.push_back((int)spref.size());
+        ++j1;
+      }
+      const int nslot = (int)spref.size();
+      const size_t smem = ((size_t)nslot * B + (j1 - j0)) * 4;
+      CK(cudaMemcpyAsync(dpref, spref.data(), nslot * 8, cudaMemcpyHostToDevice, e->stream));
+      CK(cudaMemcpyAsync(dsoff, soff.data(), soff.size() * 4, cudaMemcpyHostToDevice, e->stream));
+      CK(cudaMemsetAsync(hist, 0, (size_t)nslot * B * 8, e->stream));
+      for (int sg = 0; sg < nseg && !rc; ++sg) {
+        ++e->launches;
+        if (mcgpu_diag::diag_radix(e->hist + seg[sg].ring0 * row, seg[sg].count * e->C, ncol, j0, j1, pass, dpref, dsoff,
+                                   hist, nanc, smem, e->stream) != cudaSuccess)
+          rc = fail(e, MCGPU_ECUDA, "diag_radix_kernel launch failed");
+      }
+      if (rc) break;
+      hh_hist.resize((size_t)nslot * B);
+      CK(cudaMemcpyAsync(hh_hist.data(), hist, (size_t)nslot * B * 8, cudaMemcpyDeviceToHost, e->stream));
+      CK(cudaStreamSynchronize(e->stream));                // spref / soff are host temporaries
+      for (int j = j0; j < j1; ++j)
+        for (int t = 0; t < nt; ++t) {
+          const size_t jt = (size_t)j * nt + t;
+          const unsigned long long *h = hh_hist.data() + (size_t)tslot[jt] * B;
+          int dg = 0;
+          while (dg < B - 1 && rem[jt] >= h[dg]) rem[jt] -= h[dg++];
+          pref[jt] = (pref[jt] << 8) | (uint64_t)dg;
+        }
+      j0 = j1;
+    }
+  }
+  std::vector<unsigned long long> hn(ncol);
+  if (!rc) CK(cudaMemcpyAsync(hn.data(), nanc, ncol * 8, cudaMemcpyDeviceToHost, e->stream));
+  CK(cudaFreeAsync(scratch, e->stream));
+  CK(cudaStreamSynchronize(e->stream));
+  if (rc) return rc;
+  for (int j = 0; j < ncol; ++j)
+    for (int k = 0; k < nprob; ++k) {
+      if (hn[j]) { q[(size_t)j * nprob + k] = NAN; continue; }
+      uint64_t ua = mcgpu_diag::diag_unkey(pref[(size_t)j * nt + 2 * k]), ub = mcgpu_diag::diag_unkey(pref[(size_t)j * nt + 2 * k + 1]);
+      double a, b; memcpy(&a, &ua, 8); memcpy(&b, &ub, 8);
+      const double gam = hh[k] - floor(hh[k]), diff = b - a;   // numpy's _lerp, operation for operation
+      q[(size_t)j * nprob + k] = gam >= 0.5 ? b - diff * (1 - gam) : a + diff * gam;
+    }
   return MCGPU_OK;
 }
 

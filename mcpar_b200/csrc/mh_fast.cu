@@ -150,6 +150,8 @@ cudaError_t launch_cell_table(const double *pool, int M, float4 *tab, const Exch
   return cudaGetLastError();
 }
 
+const void *module_kernel() { return reinterpret_cast<const void *>(cell_table_kernel); }
+
 cudaError_t launch_factor_prep(const double *rm, double *cm, int D, int *diag, cudaStream_t st)
 {
   factor_prep_kernel<<<1, 256, 0, st>>>(rm, cm, D, diag);

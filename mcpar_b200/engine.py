@@ -28,6 +28,7 @@ EXPORTS = [
     "mcgpu_tune", "mcgpu_synchronize", "mcgpu_get_state", "mcgpu_get_factor", "mcgpu_get_musig",
     "mcgpu_get_trace", "mcgpu_history_read", "mcgpu_history_attach_host", "mcgpu_history_attach_host_f32",
     "mcgpu_history_maxlike", "mcgpu_history_moments",
+    "mcgpu_history_diag_partials", "mcgpu_diag_finalize", "mcgpu_history_quantiles",
     "mcgpu_checkpoint_size", "mcgpu_checkpoint_save", "mcgpu_checkpoint_load",
     "mcgpu_get_stats", "mcgpu_device_ptr", "mcgpu_loglik", "mcgpu_qriguess",
     "mcgpu_set_likelihood_plugin", "mcgpu_loglik_plugin",
@@ -37,6 +38,9 @@ EXPORTS = [
 
 class McgpuError(RuntimeError):
     pass
+
+
+DIAG_FIELDS = ["mean", "sd", "mcse_mean", "rhat_split", "rhat_nested", "ess_mean", "ess_truncated", "nonfinite"]
 
 
 class Config(C.Structure):
@@ -129,6 +133,21 @@ def measure_fp64_peak(device=0):
     return v.value
 
 
+def diag_finalize(blocks):
+    """Convergence diagnostics from the partial blocks of Engine.diag_partials (one per sharded engine, rank order):
+    a dict of per-column arrays (the parameters, then logL) named by DIAG_FIELDS.  Host arithmetic; needs no GPU."""
+    blocks = [np.ascontiguousarray(b, dtype=np.float64).ravel() for b in blocks]
+    if not blocks or blocks[0].size < 4:
+        raise ValueError("diag_finalize: no block, or a block without its header")
+    ncol, L = int(blocks[0][3]), int(blocks[0][2])
+    if any(b.size != 4 + ncol * (16 + L) for b in blocks):
+        raise ValueError("diag_finalize: a block's size does not match the header's ncol and max_lag")
+    flat = np.concatenate(blocks)
+    rep = np.empty((ncol, len(DIAG_FIELDS)))
+    _check(load().mcgpu_diag_finalize(_p(flat), len(blocks), _p(rep)))
+    return {k: rep[:, i].copy() for i, k in enumerate(DIAG_FIELDS)}
+
+
 class DevicePtr:
     """A raw device range exposing __cuda_array_interface__ so torch can alias it
     (torch.as_tensor(ptr, device='cuda')) for the NCCL exchange."""
@@ -185,6 +204,7 @@ class Engine:
         self.cfg = cfg
         self.d, self.C, self.mode = nparam, nchain, mode
         self.p2p = False
+        self._hist_from = 0                  # first kept step still valid on the device (a checkpoint load moves it)
         self.h = C.c_void_p()
         _check(self.lib.mcgpu_create(C.byref(cfg), C.byref(self.h)))
 
@@ -297,6 +317,7 @@ class Engine:
 
     def sample_begin(self, nsamp):
         self._ck(self.lib.mcgpu_sample_begin(self.h, nsamp))
+        self._hist_from = 0
 
     def sample(self, nsteps):
         self._ck(self.lib.mcgpu_sample(self.h, nsteps))
@@ -402,6 +423,35 @@ class Engine:
         self._ck(self.lib.mcgpu_history_moments(self.h, _p(mean), _p(cov)))
         return mean, cov
 
+    # -- convergence diagnostics and quantiles of the history (include/mcgpu.h) ----
+    def _valid_rows(self):
+        """n: the kept steps the device history still holds, [max(valid_from, kept - history_steps), kept)."""
+        kept = self.stats()["history_rows"] // self.C
+        return kept - max(self._hist_from, kept - self.cfg.history_steps)
+
+    def diag_partials(self, superchain=1, max_lag=None):
+        """This engine's partial block (MCGPU_DIAG_BLOCK(d + 1, max_lag) doubles) for diag_finalize.  max_lag defaults
+        to max(1, N - 2), N = floor(n/2): the largest lag ArviZ's ESS loop can reach, so the ESS is never truncated.
+        """
+        if max_lag is None:
+            max_lag = max(1, self._valid_rows() // 2 - 2)
+        blk = np.empty(4 + (self.d + 1) * (16 + max_lag))
+        self._ck(self.lib.mcgpu_history_diag_partials(self.h, int(superchain), int(max_lag), _p(blk)))
+        return blk
+
+    def quantiles(self, probs=(0.05, 0.5, 0.95)):
+        """numpy.quantile(method="linear") of every column over this engine's draws: [d + 1][len(probs)]."""
+        p = np.ascontiguousarray(probs, dtype=np.float64).ravel()
+        q = np.empty((self.d + 1, p.size))
+        self._ck(self.lib.mcgpu_history_quantiles(self.h, _p(p), int(p.size), _p(q)))
+        return q
+
+    def diagnostics(self, superchain=1, max_lag=None, probs=(0.05, 0.5, 0.95)):
+        """diag_finalize([diag_partials(...)]) plus "quantiles" [d + 1][len(probs)]: one engine's whole report."""
+        rep = diag_finalize([self.diag_partials(superchain, max_lag)])
+        rep["quantiles"] = self.quantiles(probs)
+        return rep
+
     # -- checkpoint / restart -------------------------------------------------
     def checkpoint(self):
         """Opaque blob (numpy uint8) from which an engine of the same configuration continues bit for bit."""
@@ -414,6 +464,7 @@ class Engine:
     def restore(self, blob):
         blob = np.ascontiguousarray(blob, dtype=np.uint8)
         self._ck(self.lib.mcgpu_checkpoint_load(self.h, _p(blob), C.c_size_t(blob.size)))
+        self._hist_from = self.stats()["history_rows"] // self.C
 
     def stats(self):
         s = Stats()

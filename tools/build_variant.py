@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Build an A/B variant of libmcgpu.so here (no GPU needed): mh_fast.cu recompiled with extra nvcc flags and linked
-with the current mh_exact.o / mcgpu_api.o into mcpar_b200/variants/libmcgpu_<tag>.so (git-ignored; travels to the GPU
+with the current mh_exact.o / mcgpu_api.o / mcgpu_diag.o into mcpar_b200/variants/libmcgpu_<tag>.so (git-ignored; travels to the GPU
 box).  Select it at run time with MCGPU_LIB=<path>.    python tools/build_variant.py mb9 -DMCGPU_MINB_LOCAL=9"""
 import os
 import subprocess
@@ -19,6 +19,7 @@ cmd = [b.NVCC] + b.ARCH + b.COMMON + flags + ["-c", os.path.join(b.CSRC, "mh_fas
 subprocess.check_call(cmd)
 lib = os.path.join(vdir, "libmcgpu_%s.so" % tag)
 subprocess.check_call([b.NVCC] + b.ARCH + ["-shared", "-Xcompiler", "-fPIC", "-ccbin", "/usr/bin/g++", "-o", lib, obj,
-                       os.path.join(b.OBJ, "mh_exact.o"), os.path.join(b.OBJ, "mcgpu_api.o")])
+                       os.path.join(b.OBJ, "mh_exact.o"), os.path.join(b.OBJ, "mcgpu_api.o"),
+                       os.path.join(b.OBJ, "mcgpu_diag.o")])
 os.remove(obj)
 print(lib)
