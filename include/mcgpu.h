@@ -305,13 +305,37 @@ int  mcgpu_history_moments(mcgpu_engine *e, double *mean, double *cov);
  * mcgpu_history_quantiles: numpy's quantile(method="linear") of each column over this engine's S = C n draws (for a
  * sharded job: this engine's chains only), q[ncol][nprob]; h = (S-1) p, the order statistics x_(floor h) and
  * x_(floor h + 1) are exact (radix select on the device) and combined as numpy's _lerp.  1 <= nprob <= 16, p in
- * [0, 1]; +-inf are ordered values; a column holding NaN gives NaN. */
+ * [0, 1]; +-inf are ordered values; a column holding NaN gives NaN.
+ *
+ * mcgpu_history_rank_diag: ArviZ's rank-normalised diagnostics (rhat(method="rank"), ess(method="bulk"),
+ * ess(method="tail")) of each column over this engine's chains, report[ncol][MCGPU_RANK_NFIELD].  For a sharded job
+ * each engine reports over its own chains only: ranks do not merge from partial blocks.  With the split draws y
+ * (S' = 2CN of them; the middle draw of odd n is dropped):
+ *   z(v) = Phi^-1((rank(v) - 3/8) / (S' + 1/4)), rank = the average rank of v among the S' values (ties share the
+ *     mean of their ranks; -0.0 ties with +0.0);
+ *   rhat_bulk = split R-hat of z(y); rhat_tail = split R-hat of z(|y - median(y)|), the median being the mean of the
+ *     two middle split draws; rhat = rhat_tail if rhat_tail > rhat_bulk, else rhat_bulk (Python's max());
+ *   ess_bulk = the split-chain ESS of z(y);
+ *   ess_tail = min over p = 0.05, 0.95 of the split-chain ESS of I(y <= q_p), q_p being scipy's
+ *     mquantiles(alphap=1, betap=1) over all S = Cn draws: aleph = S p + (1 - p), k = floor(clip(aleph, 1, S-1)),
+ *     g = clip(aleph - k, 0, 1), q_p = (1-g) x_(k-1) + g x_(k) (0-based order statistics, exact by radix select);
+ *   ess_truncated = 1 when any of the three ESS loops needed a lag beyond max_lag.
+ * Each transformed series is reduced as mcgpu_history_diag_partials (superchain 1) and finalized as
+ * mcgpu_diag_finalize, so the constant-column rules are theirs (all ranks tie: z = 0, ess = M'N, NaN R-hats) and
+ * C < 2 gives NaN R-hats.  A column holding a non-finite value reports only its count (ArviZ checks for NaN only).
+ * 1 <= max_lag <= N - 1.  MCGPU_ESTATE: no history or an empty one; MCGPU_EINVAL: n < 4, a bad max_lag, a NULL
+ * report, or 2CN >= 2^32; MCGPU_ENOMEM: the scratch (about 56 bytes per split draw, independent of nparam) cannot be
+ * allocated.  A refusal launches nothing.  The columns are worked one at a time; kernel_launches counts each kernel
+ * and each CUB sort or scan call (one launch each). */
 #define MCGPU_DIAG_BLOCK(ncol, max_lag) (4 + (ncol) * (16 + (max_lag)))
 enum { MCGPU_DIAG_MEAN, MCGPU_DIAG_SD, MCGPU_DIAG_MCSE_MEAN, MCGPU_DIAG_RHAT_SPLIT, MCGPU_DIAG_RHAT_NESTED,
        MCGPU_DIAG_ESS_MEAN, MCGPU_DIAG_ESS_TRUNCATED, MCGPU_DIAG_NONFINITE, MCGPU_DIAG_NFIELD };
+enum { MCGPU_RANK_RHAT, MCGPU_RANK_RHAT_BULK, MCGPU_RANK_RHAT_TAIL, MCGPU_RANK_ESS_BULK, MCGPU_RANK_ESS_TAIL,
+       MCGPU_RANK_ESS_TRUNCATED, MCGPU_RANK_NONFINITE, MCGPU_RANK_NFIELD };
 int  mcgpu_history_diag_partials(mcgpu_engine *e, int superchain, int max_lag, double *block);
 int  mcgpu_diag_finalize(const double *blocks, int nblock, double *report);
 int  mcgpu_history_quantiles(mcgpu_engine *e, const double *probs, int nprob, double *q);
+int  mcgpu_history_rank_diag(mcgpu_engine *e, int max_lag, double *report);
 
 /* Checkpoint / restart (NORMAL mode; the reference has none).  The blob holds the chain state, the
  * running moments, the tuned proposal factor, the counters, the exchange pools and the schedule;

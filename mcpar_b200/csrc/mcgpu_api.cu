@@ -1776,9 +1776,8 @@ int diag_rows(mcgpu_engine *e, long long *n, mcgpu_diag::DiagRows *rows, HistSeg
 
 // fixed-order merge of in[ncol][nin] in groups of gs entries into out[ncol][nin / gs]: one level when a group is at
 // most 1024 entries, else chunks of 1024 into tmp, then the chunks of each group
-int diag_reduce(mcgpu_engine *e, const Part *in, long long nin, long long gs, int to_item, Part *tmp, Part *out)
+int diag_reduce(mcgpu_engine *e, int ncol, const Part *in, long long nin, long long gs, int to_item, Part *tmp, Part *out)
 {
-  const int ncol = e->d + 1;
   auto launch = [&](const Part *src, long long nsrc, long long g, long long ch, int item, Part *dst) -> int {
     ++e->launches;
     CK(mcgpu_diag::diag_group(src, nsrc, ncol, g, ch, item, dst, e->stream));
@@ -1790,20 +1789,11 @@ int diag_reduce(mcgpu_engine *e, const Part *in, long long nin, long long gs, in
   if (int rc = launch(in, nin, gs, ch, 0, tmp)) return rc;
   return launch(tmp, nin / gs * nchunk, nchunk, nchunk, to_item, out);
 }
-}  // namespace
 
-int mcgpu_history_diag_partials(mcgpu_engine *e, int superchain, int max_lag, double *block)
+// the partial block (mcgpu.h) of the rows [n][C][ncol] that `rows` addresses; n, G and L already checked
+int diag_partials_rows(mcgpu_engine *e, const mcgpu_diag::DiagRows &rows, long long C, int ncol, int n, long long G, int L,
+                       double *block)
 {
-  if (!e) return MCGPU_EINVAL;
-  if (!block) return fail(e, MCGPU_EINVAL, "block is NULL");
-  DeviceGuard g(e->dev);
-  long long n = 0; mcgpu_diag::DiagRows rows; HistSeg seg[2]; int nseg = 0;
-  if (int rc = diag_rows(e, &n, &rows, seg, &nseg)) return rc;
-  const long long C = e->C, G = superchain;
-  if (G < 1 || C % G || e->cfg.chain0 % G)
-    return fail(e, MCGPU_EINVAL, "superchain must be >= 1 and divide both the hosted chain count and chain0");
-  const int N = (int)(n / 2), L = max_lag, ncol = e->d + 1;
-  if (L < 1 || L > N - 1) return fail(e, MCGPU_EINVAL, "max_lag must be in 1 .. floor(n/2) - 1");
   const long long K = C / G, cpb = mcgpu_diag::DIAG_THREADS / ncol, nblk = (C + cpb - 1) / cpb;   // diag_chain's CTAs
   const long long n_chain = ncol * C, n_split = ncol * 2 * C, n_tmp = ncol * (2 * C / 512 + 4), n_sup = ncol * K;
   const long long n_lagp = nblk * ncol * (L + 1), n_lag = (long long)ncol * (L + 1);
@@ -1815,12 +1805,12 @@ int mcgpu_history_diag_partials(mcgpu_engine *e, int superchain, int max_lag, do
   double *lagp = (double*)(spl + ncol), *lags = lagp + n_lagp;
   int rc = 0;
   ++e->launches;
-  if (mcgpu_diag::diag_chain(rows, C, ncol, (int)n, L, chain, split, lagp, e->stream) != cudaSuccess)
+  if (mcgpu_diag::diag_chain(rows, C, ncol, n, L, chain, split, lagp, e->stream) != cudaSuccess)
     rc = fail(e, MCGPU_ECUDA, "diag_chain_kernel launch failed");
-  if (!rc) rc = diag_reduce(e, chain, C, C, 0, tmp, all);                 // all hosted chains: fields 0..6
-  if (!rc) rc = diag_reduce(e, chain, C, G, 1, tmp, sup);                 // superchain items (xbar_k, Btilde_k + Wtilde_k)
-  if (!rc) rc = diag_reduce(e, sup, K, K, 0, tmp, kst);                   // fields 7..10
-  if (!rc) rc = diag_reduce(e, split, 2 * C, 2 * C, 0, tmp, spl);         // fields 11..14
+  if (!rc) rc = diag_reduce(e, ncol, chain, C, C, 0, tmp, all);           // all hosted chains: fields 0..6
+  if (!rc) rc = diag_reduce(e, ncol, chain, C, G, 1, tmp, sup);           // superchain items (xbar_k, Btilde_k + Wtilde_k)
+  if (!rc) rc = diag_reduce(e, ncol, sup, K, K, 0, tmp, kst);             // fields 7..10
+  if (!rc) rc = diag_reduce(e, ncol, split, 2 * C, 2 * C, 0, tmp, spl);   // fields 11..14
   if (!rc) {
     ++e->launches;
     if (mcgpu_diag::diag_sum_rows(lagp, nblk, n_lag, lags, e->stream) != cudaSuccess)
@@ -1845,6 +1835,22 @@ int mcgpu_history_diag_partials(mcgpu_engine *e, int superchain, int max_lag, do
     for (int t = 0; t <= L; ++t) f[15 + t] = hl[(size_t)j * (L + 1) + t];
   }
   return MCGPU_OK;
+}
+}  // namespace
+
+int mcgpu_history_diag_partials(mcgpu_engine *e, int superchain, int max_lag, double *block)
+{
+  if (!e) return MCGPU_EINVAL;
+  if (!block) return fail(e, MCGPU_EINVAL, "block is NULL");
+  DeviceGuard g(e->dev);
+  long long n = 0; mcgpu_diag::DiagRows rows; HistSeg seg[2]; int nseg = 0;
+  if (int rc = diag_rows(e, &n, &rows, seg, &nseg)) return rc;
+  const long long C = e->C, G = superchain;
+  if (G < 1 || C % G || e->cfg.chain0 % G)
+    return fail(e, MCGPU_EINVAL, "superchain must be >= 1 and divide both the hosted chain count and chain0");
+  const int N = (int)(n / 2), L = max_lag;
+  if (L < 1 || L > N - 1) return fail(e, MCGPU_EINVAL, "max_lag must be in 1 .. floor(n/2) - 1");
+  return diag_partials_rows(e, rows, C, e->d + 1, (int)n, G, L, block);
 }
 
 namespace {
@@ -1928,26 +1934,15 @@ int mcgpu_diag_finalize(const double *blocks, int nblock, double *report)
   return MCGPU_OK;
 }
 
-int mcgpu_history_quantiles(mcgpu_engine *e, const double *probs, int nprob, double *q)
+namespace {
+// exact order statistics of every column over the S = C n draws of the valid history, by radix select on diag_key:
+// pref[j][t] = the key of x_(rank[t]) of column j (0-based ranks), nan[j] = column j's NaN count
+int diag_select(mcgpu_engine *e, const HistSeg *seg, int nseg, const std::vector<long long> &rank,
+                std::vector<uint64_t> &pref, std::vector<unsigned long long> &nan)
 {
-  if (!e) return MCGPU_EINVAL;
-  if (!probs || !q) return fail(e, MCGPU_EINVAL, "probs or q is NULL");
-  if (nprob < 1 || nprob > 16) return fail(e, MCGPU_EINVAL, "nprob must be in 1 .. 16");
-  for (int k = 0; k < nprob; ++k)
-    if (!(probs[k] >= 0.0 && probs[k] <= 1.0)) return fail(e, MCGPU_EINVAL, "probabilities must lie in [0, 1]");
-  DeviceGuard g(e->dev);
-  long long n = 0; HistSeg seg[2]; int nseg = 0;
-  if (int rc = diag_rows(e, &n, nullptr, seg, &nseg)) return rc;
-  const int ncol = e->d + 1, nt = 2 * nprob, B = mcgpu_diag::QSEL_BINS;
-  const long long S = n * e->C, row = e->C * ncol;
-  // numpy's method="linear": h = (S - 1) p, order statistics floor(h) and floor(h) + 1 (clipped to S - 1)
-  std::vector<double> hh(nprob); std::vector<long long> rank(nt);
-  for (int k = 0; k < nprob; ++k) {
-    hh[k] = (double)(S - 1) * probs[k];
-    const long long i = std::min<long long>((long long)floor(hh[k]), S - 1);
-    rank[2 * k] = i; rank[2 * k + 1] = std::min(i + 1, S - 1);
-  }
-  std::vector<uint64_t> pref((size_t)ncol * nt, 0); std::vector<unsigned long long> rem((size_t)ncol * nt);
+  const int ncol = e->d + 1, nt = (int)rank.size(), B = mcgpu_diag::QSEL_BINS;
+  const long long row = e->C * ncol;
+  pref.assign((size_t)ncol * nt, 0); std::vector<unsigned long long> rem((size_t)ncol * nt);
   for (int j = 0; j < ncol; ++j) for (int t = 0; t < nt; ++t) rem[(size_t)j * nt + t] = rank[t];
   int optin = 0;
   CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, e->dev));
@@ -2002,11 +1997,35 @@ int mcgpu_history_quantiles(mcgpu_engine *e, const double *probs, int nprob, dou
       j0 = j1;
     }
   }
-  std::vector<unsigned long long> hn(ncol);
-  if (!rc) CK(cudaMemcpyAsync(hn.data(), nanc, ncol * 8, cudaMemcpyDeviceToHost, e->stream));
+  nan.assign(ncol, 0);
+  if (!rc) CK(cudaMemcpyAsync(nan.data(), nanc, ncol * 8, cudaMemcpyDeviceToHost, e->stream));
   CK(cudaFreeAsync(scratch, e->stream));
   CK(cudaStreamSynchronize(e->stream));
-  if (rc) return rc;
+  return rc;
+}
+}  // namespace
+
+int mcgpu_history_quantiles(mcgpu_engine *e, const double *probs, int nprob, double *q)
+{
+  if (!e) return MCGPU_EINVAL;
+  if (!probs || !q) return fail(e, MCGPU_EINVAL, "probs or q is NULL");
+  if (nprob < 1 || nprob > 16) return fail(e, MCGPU_EINVAL, "nprob must be in 1 .. 16");
+  for (int k = 0; k < nprob; ++k)
+    if (!(probs[k] >= 0.0 && probs[k] <= 1.0)) return fail(e, MCGPU_EINVAL, "probabilities must lie in [0, 1]");
+  DeviceGuard g(e->dev);
+  long long n = 0; HistSeg seg[2]; int nseg = 0;
+  if (int rc = diag_rows(e, &n, nullptr, seg, &nseg)) return rc;
+  const int ncol = e->d + 1, nt = 2 * nprob;
+  const long long S = n * e->C;
+  // numpy's method="linear": h = (S - 1) p, order statistics floor(h) and floor(h) + 1 (clipped to S - 1)
+  std::vector<double> hh(nprob); std::vector<long long> rank(nt);
+  for (int k = 0; k < nprob; ++k) {
+    hh[k] = (double)(S - 1) * probs[k];
+    const long long i = std::min<long long>((long long)floor(hh[k]), S - 1);
+    rank[2 * k] = i; rank[2 * k + 1] = std::min(i + 1, S - 1);
+  }
+  std::vector<uint64_t> pref; std::vector<unsigned long long> hn;
+  if (int rc = diag_select(e, seg, nseg, rank, pref, hn)) return rc;
   for (int j = 0; j < ncol; ++j)
     for (int k = 0; k < nprob; ++k) {
       if (hn[j]) { q[(size_t)j * nprob + k] = NAN; continue; }
@@ -2016,6 +2035,99 @@ int mcgpu_history_quantiles(mcgpu_engine *e, const double *probs, int nprob, dou
       q[(size_t)j * nprob + k] = gam >= 0.5 ? b - diff * (1 - gam) : a + diff * gam;
     }
   return MCGPU_OK;
+}
+
+int mcgpu_history_rank_diag(mcgpu_engine *e, int max_lag, double *report)
+{
+  if (!e) return MCGPU_EINVAL;
+  if (!report) return fail(e, MCGPU_EINVAL, "report is NULL");
+  DeviceGuard g(e->dev);
+  long long n = 0; mcgpu_diag::DiagRows rows; HistSeg seg[2]; int nseg = 0;
+  if (int rc = diag_rows(e, &n, &rows, seg, &nseg)) return rc;
+  const long long C = e->C, N = n / 2, S2 = 2 * C * N, S = C * n;
+  const int L = max_lag, ncol = e->d + 1, RC = mcgpu_diag::RANK_COLS, NF = MCGPU_DIAG_NFIELD;
+  if (L < 1 || L > N - 1) return fail(e, MCGPU_EINVAL, "max_lag must be in 1 .. floor(n/2) - 1");
+  if (S2 >= (1ll << 32)) return fail(e, MCGPU_EINVAL, "rank diagnostics need 2 C floor(n/2) < 2^32 split draws");
+  size_t tb = 0;
+  CK(mcgpu_diag::rank_temp_bytes(S2, &tb));
+  tb = (tb + 255) & ~(size_t)255;
+  // scratch: CUB's temp storage, the series [2N][C][RC], the sort's two key and two position buffers, a counter
+  const size_t bytes = tb + (size_t)S2 * (RC * 8 + 2 * 8 + 2 * 4) + 8;
+  char *scratch = nullptr;
+  if (cudaMallocAsync((void**)&scratch, bytes, e->stream) != cudaSuccess) {
+    cudaGetLastError();
+    return fail(e, MCGPU_ENOMEM, "cannot allocate the rank diagnostics' scratch (about 56 bytes per split draw)");
+  }
+  double *series = (double*)(scratch + tb);
+  uint64_t *kbuf = (uint64_t*)(series + S2 * RC);
+  unsigned long long *nfc = (unsigned long long*)(kbuf + 2 * S2);
+  uint32_t *pbuf = (uint32_t*)(nfc + 1);
+  // tail thresholds: scipy's mquantiles(alphap=1, betap=1) over all S draws, operation for operation; m = alphap +
+  // p (1 - alphap - betap) = 1 - p.  Each product is rounded on its own (no fused multiply-add on the host).
+  const double pt[2] = {0.05, 0.95};
+  double gam[2]; std::vector<long long> rank(4);
+  for (int t = 0; t < 2; ++t) {
+    const double aleph = (double)S * pt[t] + (1.0 - pt[t]);
+    const double k = floor(std::min(std::max(aleph, 1.0), (double)(S - 1)));
+    gam[t] = std::min(std::max(aleph - k, 0.0), 1.0);
+    rank[2 * t] = (long long)k - 1; rank[2 * t + 1] = (long long)k;
+  }
+  std::vector<uint64_t> pref; std::vector<unsigned long long> nan;
+  int rc = diag_select(e, seg, nseg, rank, pref, nan);
+  std::vector<double> block(MCGPU_DIAG_BLOCK(RC, L)), rep((size_t)RC * NF);
+  const mcgpu_diag::DiagRows srows{series, series, 2 * N, C * RC};
+  for (int j = 0; j < ncol && !rc; ++j) {
+    double *r = report + (size_t)j * MCGPU_RANK_NFIELD, q[2];
+    for (int t = 0; t < 2; ++t) {
+      uint64_t ua = mcgpu_diag::diag_unkey(pref[(size_t)j * 4 + 2 * t]), ub = mcgpu_diag::diag_unkey(pref[(size_t)j * 4 + 2 * t + 1]);
+      double a, b; memcpy(&a, &ua, 8); memcpy(&b, &ub, 8);
+      const double lo = (1.0 - gam[t]) * a, hi = gam[t] * b;
+      q[t] = lo + hi;
+    }
+    uint64_t *keys[2] = {kbuf, kbuf + S2}; uint32_t *pos[2] = {pbuf, pbuf + S2};
+    unsigned long long nf = 0;
+    CK(cudaMemsetAsync(nfc, 0, 8, e->stream));
+    ++e->launches;
+    if (mcgpu_diag::rank_keys(rows, C, ncol, j, (int)n, nullptr, q[0], q[1], keys[0], pos[0], series, nfc, e->stream) != cudaSuccess) {
+      rc = fail(e, MCGPU_ECUDA, "rank_keys_kernel launch failed");
+      break;
+    }
+    CK(cudaMemcpyAsync(&nf, nfc, 8, cudaMemcpyDeviceToHost, e->stream));
+    CK(cudaStreamSynchronize(e->stream));
+    for (int k = 0; k < MCGPU_RANK_NFIELD; ++k) r[k] = NAN;
+    r[MCGPU_RANK_NONFINITE] = (double)nf;
+    if (nf) continue;
+    e->launches += mcgpu_diag::RANK_SCORE_LAUNCHES;
+    if (mcgpu_diag::rank_scores(keys, pos, S2, scratch, tb, series, 0, e->stream) != cudaSuccess) {
+      rc = fail(e, MCGPU_ECUDA, "rank normal scores (sort, scan or kernel) failed");
+      break;
+    }
+    ++e->launches;                                         // the folded draws; keys[0] holds the sorted draws
+    if (mcgpu_diag::rank_keys(rows, C, ncol, j, (int)n, keys[0], 0.0, 0.0, keys[1], pos[1], series, nfc, e->stream) != cudaSuccess) {
+      rc = fail(e, MCGPU_ECUDA, "rank_keys_kernel launch failed");
+      break;
+    }
+    std::swap(keys[0], keys[1]); std::swap(pos[0], pos[1]);
+    e->launches += mcgpu_diag::RANK_SCORE_LAUNCHES;
+    if (mcgpu_diag::rank_scores(keys, pos, S2, scratch, tb, series, 1, e->stream) != cudaSuccess) {
+      rc = fail(e, MCGPU_ECUDA, "rank normal scores (sort, scan or kernel) failed");
+      break;
+    }
+    if ((rc = diag_partials_rows(e, srows, C, RC, (int)(2 * N), 1, L, block.data()))) break;
+    if ((rc = mcgpu_diag_finalize(block.data(), 1, rep.data()))) break;
+    const double *z = &rep[0], *fold = &rep[NF], *i05 = &rep[2 * NF], *i95 = &rep[3 * NF];
+    if (C >= 2) {                                          // ArviZ's _rhat_rank wants two chains
+      r[MCGPU_RANK_RHAT_BULK] = z[MCGPU_DIAG_RHAT_SPLIT];
+      r[MCGPU_RANK_RHAT_TAIL] = fold[MCGPU_DIAG_RHAT_SPLIT];
+      r[MCGPU_RANK_RHAT] = r[MCGPU_RANK_RHAT_TAIL] > r[MCGPU_RANK_RHAT_BULK] ? r[MCGPU_RANK_RHAT_TAIL] : r[MCGPU_RANK_RHAT_BULK];
+    }
+    r[MCGPU_RANK_ESS_BULK] = z[MCGPU_DIAG_ESS_MEAN];
+    r[MCGPU_RANK_ESS_TAIL] = i95[MCGPU_DIAG_ESS_MEAN] < i05[MCGPU_DIAG_ESS_MEAN] ? i95[MCGPU_DIAG_ESS_MEAN] : i05[MCGPU_DIAG_ESS_MEAN];
+    r[MCGPU_RANK_ESS_TRUNCATED] = std::max({z[MCGPU_DIAG_ESS_TRUNCATED], i05[MCGPU_DIAG_ESS_TRUNCATED], i95[MCGPU_DIAG_ESS_TRUNCATED]});
+  }
+  CK(cudaFreeAsync(scratch, e->stream));
+  CK(cudaStreamSynchronize(e->stream));
+  return rc;
 }
 
 // ---- checkpoint / restart ---------------------------------------------------------------------

@@ -1,6 +1,9 @@
 // mcgpu_diag.cu -- the kernels of the history diagnostics and quantiles and their launchers (mcgpu_diag.cuh).
 #include "mcgpu_diag.cuh"
 #include <algorithm>
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
+#include <cuda/functional>
 
 namespace mcgpu_diag {
 
@@ -211,6 +214,111 @@ cudaError_t diag_radix(const double *rows, long long nrows, int ncol, int j0, in
   if (r != cudaSuccess) return r;
   diag_radix_kernel<<<(unsigned)(std::max(occ, 1) * nsm), 256, smem, st>>>(rows, nrows, ncol, j0, j1, pass, prefix, soff,
                                                                           hist, nan_count);
+  return cudaGetLastError();
+}
+
+// ---- rank normalisation -------------------------------------------------------------------------------------------
+__device__ inline double key_value(uint64_t k) { return __longlong_as_double((long long)diag_unkey(k)); }
+
+// One thread per draw (kept step k, hosted chain c) of column j; see rank_keys in mcgpu_diag.cuh.  -0.0 is keyed as
+// +0.0 because rankdata ties them.
+__global__ void rank_keys_kernel(DiagRows rows, long long C, int ncol, int j, int n, const uint64_t *mid, double q05,
+                                 double q95, uint64_t *keys, uint32_t *pos, double *series,
+                                 unsigned long long *nonfinite)
+{
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int N = n / 2;
+  bool bad = false;
+  if (t < (long long)n * C) {
+    const int k = (int)(t / C);
+    const long long c = t - (long long)k * C;
+    double x = rows.at(k)[c * ncol + j];
+    bad = !isfinite(x);
+    if (k < N || k >= n - N) {
+      const long long i = (long long)(k < N ? k : k - (n - 2 * N)) * C + c;
+      if (mid) {
+        const double med = (key_value(mid[(long long)N * C - 1]) + key_value(mid[(long long)N * C])) / 2;
+        x = fabs(x - med);
+      } else {
+        series[i * RANK_COLS + 2] = x <= q05 ? 1.0 : 0.0;
+        series[i * RANK_COLS + 3] = x <= q95 ? 1.0 : 0.0;
+      }
+      keys[i] = diag_key((uint64_t)__double_as_longlong(x == 0.0 ? 0.0 : x));
+      pos[i] = (uint32_t)i;
+    }
+  }
+  if (!mid) {
+    const unsigned int m = __ballot_sync(0xffffffffu, bad);
+    if (m && (threadIdx.x & 31) == 0) atomicAdd(nonfinite, (unsigned long long)__popc(m));
+  }
+}
+
+// head[i] = i where a run of equal sorted keys starts, else 0; a running max then gives each entry its run's start
+__global__ void rank_heads_kernel(const uint64_t *keys, long long S2, uint32_t *head)
+{
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < S2) head[i] = (i == 0 || keys[i] != keys[i - 1]) ? (uint32_t)i : 0u;
+}
+
+// the last entry of each run stores its index at the run's start: end[start] = the run's last sorted index
+__global__ void rank_tails_kernel(const uint64_t *keys, const uint32_t *start, long long S2, uint32_t *end)
+{
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < S2 && (i == S2 - 1 || keys[i] != keys[i + 1])) end[start[i]] = (uint32_t)i;
+}
+
+// a run over sorted indices [a, b] has the average rank (a + b)/2 + 1 (exact in fp64); its normal score
+// Phi^-1((rank - 3/8) / (S2 + 1/4)) goes to series[pos][col]
+__global__ void rank_scores_kernel(const uint32_t *start, const uint32_t *end, const uint32_t *pos, long long S2,
+                                   double *series, int col)
+{
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= S2) return;
+  const uint32_t a = start[i], b = end[a];
+  const double rank = ((double)a + (double)b) / 2 + 1.0;
+  series[(long long)pos[i] * RANK_COLS + col] = normcdfinv((rank - 0.375) / ((double)S2 + 0.25));
+}
+
+cudaError_t rank_temp_bytes(long long S2, size_t *bytes)
+{
+  cub::DoubleBuffer<uint64_t> kb(nullptr, nullptr);
+  cub::DoubleBuffer<uint32_t> pb(nullptr, nullptr);
+  size_t sort = 0, scan = 0;
+  cudaError_t r = cub::DeviceRadixSort::SortPairs(nullptr, sort, kb, pb, S2, 0, 64);
+  if (r == cudaSuccess)
+    r = cub::DeviceScan::InclusiveScan(nullptr, scan, (const uint32_t*)nullptr, (uint32_t*)nullptr,
+                                       cuda::maximum<uint32_t>{}, (uint32_t)S2);
+  *bytes = std::max(sort, scan);
+  return r;
+}
+
+cudaError_t rank_keys(const DiagRows &rows, long long C, int ncol, int j, int n, const uint64_t *mid, double q05,
+                      double q95, uint64_t *keys, uint32_t *pos, double *series, unsigned long long *nonfinite,
+                      cudaStream_t st)
+{
+  rank_keys_kernel<<<(unsigned)((n * C + 255) / 256), 256, 0, st>>>(rows, C, ncol, j, n, mid, q05, q95, keys, pos,
+                                                                     series, nonfinite);
+  return cudaGetLastError();
+}
+
+cudaError_t rank_scores(uint64_t *keys[2], uint32_t *pos[2], long long S2, void *temp, size_t temp_bytes, double *series,
+                        int col, cudaStream_t st)
+{
+  cub::DoubleBuffer<uint64_t> kb(keys[0], keys[1]);
+  cub::DoubleBuffer<uint32_t> pb(pos[0], pos[1]);
+  cudaError_t r = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, kb, pb, S2, 0, 64, st);
+  if (r != cudaSuccess) return r;
+  keys[0] = kb.Current(); keys[1] = kb.Alternate(); pos[0] = pb.Current(); pos[1] = pb.Alternate();
+  uint32_t *start = reinterpret_cast<uint32_t*>(keys[1]), *end = start + S2;   // the spare key buffer, 2 S2 words
+  const unsigned nb = (unsigned)((S2 + 255) / 256);
+  rank_heads_kernel<<<nb, 256, 0, st>>>(keys[0], S2, end);
+  if ((r = cudaGetLastError()) != cudaSuccess) return r;
+  r = cub::DeviceScan::InclusiveScan(temp, temp_bytes, (const uint32_t*)end, start, cuda::maximum<uint32_t>{},
+                                     (uint32_t)S2, st);
+  if (r != cudaSuccess) return r;
+  rank_tails_kernel<<<nb, 256, 0, st>>>(keys[0], start, S2, end);
+  if ((r = cudaGetLastError()) != cudaSuccess) return r;
+  rank_scores_kernel<<<nb, 256, 0, st>>>(start, end, pos[0], S2, series, col);
   return cudaGetLastError();
 }
 

@@ -1,6 +1,7 @@
 // mcgpu_diag.cuh -- device reductions of the sample history for convergence diagnostics (split and nested R-hat,
-// multi-chain ESS, MCSE) and exact posterior quantiles (include/mcgpu.h: mcgpu_history_diag_partials,
-// mcgpu_history_quantiles): the types and launchers mcgpu_api.cu uses; the kernels are in mcgpu_diag.cu.
+// multi-chain ESS, MCSE), exact posterior quantiles and the rank normalisation of ArviZ's rank diagnostics
+// (include/mcgpu.h: mcgpu_history_diag_partials, mcgpu_history_quantiles, mcgpu_history_rank_diag): the types and
+// launchers mcgpu_api.cu uses; the kernels are in mcgpu_diag.cu.
 //
 // The kernels are a translation unit (a device module) of their own: a sampling engine never loads them, and the
 // modules a peer-to-peer engine loads up front (DESIGN.md section 6) do not grow with them.
@@ -10,7 +11,7 @@
 //
 // Every floating-point reduction runs in a fixed order (a per-thread sequence, a fixed shuffle tree, a fixed
 // sequential sum over a CTA's chains): no floating-point atomics, so a repeated call returns the same bits.
-// Integer counters (quantile histograms, NaN counts) use atomics.
+// Integer counters (quantile histograms, NaN counts) use atomics; CUB's radix sort and scan are deterministic.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -58,5 +59,25 @@ cudaError_t diag_sum_rows(const double *in, long long nb, long long nr, double *
 cudaError_t diag_radix(const double *rows, long long nrows, int ncol, int j0, int j1, int pass, const uint64_t *prefix,
                        const int *soff, unsigned long long *hist, unsigned long long *nan_count, size_t smem,
                        cudaStream_t st);
+
+// ---- rank normalisation (mcgpu_history_rank_diag) ----------------------------------------------------------------
+// The split draws of one column (S2 = 2CN of them) become the series [2N][C][RANK_COLS]: column 0 the normal scores
+// of their ranks, column 1 those of the folded draws |y - median|, columns 2 and 3 the tail indicators.  Position
+// i = r C + c is split row r of hosted chain c (rows N..2N-1 are kept steps n-N..n-1).
+constexpr int RANK_COLS = 4;
+constexpr int RANK_SCORE_LAUNCHES = 5;   // rank_scores: the sort, 3 kernels, the scan
+
+// CUB temp storage rank_scores needs for S2 pairs
+cudaError_t rank_temp_bytes(long long S2, size_t *bytes);
+// keys, pos := the sort keys and positions of column j's split draws.  mid == nullptr: of the draws; series
+// columns 2 and 3 := I(x <= q05), I(x <= q95); *nonfinite += the non-finite draws of all n kept steps.  Else: of the
+// folded draws, with mid the sorted keys of the draws (the median is the mean of its middle two).
+cudaError_t rank_keys(const DiagRows &rows, long long C, int ncol, int j, int n, const uint64_t *mid, double q05,
+                      double q95, uint64_t *keys, uint32_t *pos, double *series, unsigned long long *nonfinite,
+                      cudaStream_t st);
+// sorts the pairs (keys[0], pos[0]) through the buffers keys[1], pos[1] (on return keys[0], pos[0] name the sorted
+// pairs, keys[1] the spare buffer of 8 S2 bytes) and writes series[i][col] = the normal score of the average rank
+cudaError_t rank_scores(uint64_t *keys[2], uint32_t *pos[2], long long S2, void *temp, size_t temp_bytes, double *series,
+                        int col, cudaStream_t st);
 
 }  // namespace mcgpu_diag

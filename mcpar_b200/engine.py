@@ -28,7 +28,7 @@ EXPORTS = [
     "mcgpu_tune", "mcgpu_synchronize", "mcgpu_get_state", "mcgpu_get_factor", "mcgpu_get_musig",
     "mcgpu_get_trace", "mcgpu_history_read", "mcgpu_history_attach_host", "mcgpu_history_attach_host_f32",
     "mcgpu_history_maxlike", "mcgpu_history_moments",
-    "mcgpu_history_diag_partials", "mcgpu_diag_finalize", "mcgpu_history_quantiles",
+    "mcgpu_history_diag_partials", "mcgpu_diag_finalize", "mcgpu_history_quantiles", "mcgpu_history_rank_diag",
     "mcgpu_checkpoint_size", "mcgpu_checkpoint_save", "mcgpu_checkpoint_load",
     "mcgpu_get_stats", "mcgpu_device_ptr", "mcgpu_loglik", "mcgpu_qriguess",
     "mcgpu_set_likelihood_plugin", "mcgpu_loglik_plugin",
@@ -41,6 +41,7 @@ class McgpuError(RuntimeError):
 
 
 DIAG_FIELDS = ["mean", "sd", "mcse_mean", "rhat_split", "rhat_nested", "ess_mean", "ess_truncated", "nonfinite"]
+RANK_FIELDS = ["rhat", "rhat_bulk", "rhat_tail", "ess_bulk", "ess_tail", "ess_truncated", "nonfinite"]
 
 
 class Config(C.Structure):
@@ -78,6 +79,7 @@ def load():
         lib.mcgpu_version.restype = C.c_char_p
         lib.mcgpu_last_error.restype = C.c_char_p
         lib.mcgpu_last_error.argtypes = [C.c_void_p]
+        lib.mcgpu_history_rank_diag.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
         _lib = lib
     return _lib
 
@@ -445,6 +447,16 @@ class Engine:
         q = np.empty((self.d + 1, p.size))
         self._ck(self.lib.mcgpu_history_quantiles(self.h, _p(p), int(p.size), _p(q)))
         return q
+
+    def rank_diagnostics(self, max_lag=None):
+        """ArviZ's rank-normalised R-hat (rhat = max of rhat_bulk and rhat_tail), bulk ESS and tail ESS of every column
+        over this engine's chains: a dict of per-column arrays named by RANK_FIELDS.  max_lag defaults as in
+        diag_partials."""
+        if max_lag is None:
+            max_lag = max(1, self._valid_rows() // 2 - 2)
+        rep = np.empty((self.d + 1, len(RANK_FIELDS)))
+        self._ck(self.lib.mcgpu_history_rank_diag(self.h, int(max_lag), _p(rep)))
+        return {k: rep[:, i].copy() for i, k in enumerate(RANK_FIELDS)}
 
     def diagnostics(self, superchain=1, max_lag=None, probs=(0.05, 0.5, 0.95)):
         """diag_finalize([diag_partials(...)]) plus "quantiles" [d + 1][len(probs)]: one engine's whole report."""
